@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the B200-native diffusion-curve ray tracer.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one frame of the hot path: ray generation + closest-hit traversal + shading + normalisation
@@ -70,7 +70,15 @@ def parse_args():
     ap.add_argument("--no-secondary", dest="secondary", action="store_false",
                     help="skip the config-5 block (8192x8192 @512 synthetic scene) that follows the headline measurement")
     ap.add_argument("--secondary-steps", type=int, default=2)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="b200 arm only: after the timed steps, write the finished frame of the last timed step to DIR/frame.npy "
+                         "(float32 RGBA; frames over 64 MB: a seeded sample of rows, their indices in DIR/frame_rows.npy)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the b200 path computed")
+    return args
 
 
 def workload_zoom(spec, height):
@@ -364,7 +372,7 @@ class Workload:
         for s in range(steps):
             flush.zero_()  # evict L2 between timed iterations (untimed)
             starts[s].record()
-            self.frame_step(warmup + s)
+            self.last_frame = self.frame_step(warmup + s)
             ends[s].record()
         self.barrier()
         wall = time.perf_counter() - wall0
@@ -476,6 +484,32 @@ def np_isfinite_or_nan_rows(frame):
     return np.all(np.abs(a - 1.0) < 1e-3)
 
 
+DUMP_BYTES = 64 * 1000 * 1000
+
+
+def dump_outputs(work, out_dir):
+    """--dump-outputs: the frame the last timed step left on (rank 0's) device, as the caller of the timed path receives it.
+    Frames larger than DUMP_BYTES keep a fixed, seeded sample of whole rows, so runs with the same arguments compare."""
+    import numpy as np
+
+    torch = work.torch
+    h, w = work.height, work.width
+
+    class DeviceFrame:  # the frame lives in memory the library owns (peer frames for N > 1): viewed, not copied
+        __cuda_array_interface__ = {"shape": (h, w, 4), "typestr": "<f4", "data": (work.last_frame, False), "strides": None,
+                                    "version": 3}
+
+    frame = torch.as_tensor(DeviceFrame(), device=work.dev)
+    os.makedirs(out_dir, exist_ok=True)
+    row_bytes = w * 4 * 4
+    if h * row_bytes > DUMP_BYTES:
+        n_rows = (DUMP_BYTES - 4096) // (row_bytes + 8)  # 4096: room for the two .npy headers
+        rows = np.sort(np.random.default_rng(0).choice(h, n_rows, replace=False))
+        frame = frame.index_select(0, torch.from_numpy(rows).to(work.dev))
+        np.save(os.path.join(out_dir, "frame_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, "frame.npy"), frame.cpu().numpy())
+
+
 def measure_peaks(api, torch, stream, dev):
     """FP32 (dependent FFMA) and L2-read microbenchmarks on this GPU, now."""
     sink = torch.zeros((4,), dtype=torch.float32, device=dev)
@@ -554,6 +588,8 @@ def main():
     work = Workload(args.workload, api, torch, dist, dev, rank, world)
     sampler = ClockSampler(local_rank)
     ms_per_step, wall = work.time_value(args.steps, args.warmup, flush, sampler)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(work, args.dump_outputs)
     rays_per_frame = float(work.width) * work.height * work.rpp
     value = rays_per_frame / (ms_per_step * 1e-3) / 1e9
 

@@ -1,11 +1,43 @@
 """Shared helpers for the parity tests."""
 import glob
+import hashlib
+import json
 import os
 
 import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 XML_DIR = os.path.join(ROOT, "tests", "golden", "xmls")
+
+# Inputs of the reference-comparison tests; tests/golden/make_golden.py stores the reference's answers to them.
+DIFFERENT_VIEW = ("PortalDemo.xml", (48, 36, 24), dict(zoom_factor=9.0, offset_x=13.0, offset_y=-7.5, frame=3, seed=11))
+# fille.xml at the pixel scale of a 200x150 frame: its real sigmas, up to 8.4 output pixels
+FILLE_BLUR_VIEW = ("DiffusionCurvePack/fille.xml", (64, 48, 8), dict(zoom_factor=512 / 150))
+
+
+def seeded_blur_input():
+    """37x53 image with one all-miss (NaN) pixel; sigmas up to 6, zero below 1.5."""
+    rng = np.random.default_rng(5)
+    image = rng.random((37, 53, 4), dtype=np.float32)
+    sigma = (rng.random((37, 53), dtype=np.float32) * 6.0).astype(np.float32)
+    sigma[sigma < 1.5] = 0.0
+    image[3, 4, :3] = np.nan
+    return image, sigma
+
+
+def sha_bits(a: np.ndarray) -> str:
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+def ingest_digest(scene: dict) -> dict:
+    """Arrays as dtype, shape and sha256 of their bits; counts as they are."""
+    return {k: {"dtype": str(v.dtype), "shape": list(v.shape), "sha256": sha_bits(v)} if isinstance(v, np.ndarray) else int(v)
+            for k, v in scene.items()}
+
+
+def reference_checks() -> dict:
+    with open(os.path.join(ROOT, "tests", "golden", "reference_checks.json")) as fh:
+        return json.load(fh)
 
 
 def all_scene_files():

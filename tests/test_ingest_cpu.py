@@ -9,7 +9,7 @@ import os
 import numpy as np
 import pytest
 
-from helpers import all_scene_files, assert_scene_equal, bits, scene_ids, XML_DIR
+from helpers import all_scene_files, assert_scene_equal, ingest_digest, reference_checks, scene_ids, sha_bits, XML_DIR
 from oracle import pyoracle as po
 from raytracingdiffusioncurves_b200 import api
 
@@ -190,20 +190,21 @@ def test_numbers_are_read_like_atof(tmp_path):
 def test_product_ingest_equals_the_reference_own_loop(path):
     """a2 pinned by the reference's code: optixHello.cpp:108-117,170-515 and its helpers :1302-1386, cut out of the file where
     it lies and compiled for the host (oracle/ref_extract.sh -> oracle/_ref/libref_ingest.so), run on every bundled XML.
-    The product's arrays equal the reference's bit for bit (the product appends +INF sentinels after them)."""
-    from oracle import pyoracle as po
-
-    if not po.ref_extracts_available():
-        pytest.skip("oracle/_ref/libref_ingest.so not built (needs /root/reference at build time)")
-    ref = po.ref_ingest(path)
+    The product's arrays equal the reference's bit for bit (the product appends +INF sentinels after them). The reference's
+    arrays are stored as sha256 of their bits (tests/golden/make_golden.py); where oracle/_ref is built they are also
+    computed live and must match what is stored."""
+    want = reference_checks()["ingest"][os.path.relpath(path, XML_DIR)]
     mine = api.HostScene.from_xml_file(path).to_numpy()
-    assert set(ref) == set(mine)
-    for k, v in ref.items():
-        if isinstance(v, np.ndarray):
-            m = np.ascontiguousarray(mine[k][: len(v)])
-            assert m.shape == v.shape, k
-            assert np.array_equal(bits(m), bits(np.ascontiguousarray(v))), k
+    assert set(want) == set(mine)
+    for k, v in want.items():
+        if isinstance(v, dict):
+            n = v["shape"][0]
+            m = np.ascontiguousarray(mine[k][:n])
+            assert [str(m.dtype), list(m.shape)] == [v["dtype"], v["shape"]], k
+            assert sha_bits(m) == v["sha256"], k
             if k.endswith("_u"):  # what follows the reference's entries is the two sentinels, nothing else
-                assert np.all(np.isinf(mine[k][len(v):])) and len(mine[k]) >= len(v) + 2
+                assert np.all(np.isinf(mine[k][n:])) and len(mine[k]) >= n + 2
         else:
             assert mine[k] == v, k
+    if po.ref_extracts_available():
+        assert ingest_digest(po.ref_ingest(path)) == want

@@ -315,11 +315,27 @@ def test_blur_parity(name, xml_dir, api, port_oracle):
     assert np.max(np.abs(got[m] - full[m]), initial=0) <= 2e-4
 
 
-def test_blur_against_the_reference_own_kernels(xml_dir, api):
+def test_blur_against_the_reference_own_kernels(golden_dir, xml_dir, api):
     """k_blur_* against gaussHorizontal / gaussVertical themselves (helperKernels.cu:48-134 compiled for the host by
-    oracle/ref_extract.sh), on a rendered frame with the scene's real sigmas."""
+    oracle/ref_extract.sh), on a rendered frame with the scene's real sigmas: the stored frame and its reference blur
+    (tests/golden/make_golden.py), and, where oracle/_ref is built, the GPU's own 200x150 render blurred live."""
+    import torch
+
+    z = np.load(os.path.join(golden_dir, "blur_fille.npz"))
+    h, w = z["blur_map"].shape
+    assert float(z["blur_map"].max()) > 4.0
+    src = torch.from_numpy(z["image"]).cuda()
+    sigma = torch.from_numpy(z["blur_map"]).cuda()
+    dest, scratch = torch.empty_like(src), torch.empty_like(src)
+    api.gaussian_blur(dest.data_ptr(), src.data_ptr(), sigma.data_ptr(), scratch.data_ptr(), w, h, 0, h, 0,
+                      torch.cuda.current_stream().cuda_stream)
+    got, want = dest.cpu().numpy()[..., :3], z["blurred_rgb"]
+    assert np.array_equal(np.isnan(got), np.isnan(want))
+    m = ~np.isnan(want)
+    assert np.max(np.abs(got[m] - want[m]), initial=0) <= 1e-5
     if not po.ref_extracts_available():
-        pytest.skip("oracle/_ref/libref_blur.so did not travel with the snapshot")
+        return
+    assert np.array_equal(bits(po.ref_blur(z["image"], z["blur_map"])[..., :3]), bits(want))  # the stored answer is the reference's
     r = GpuRenderer(os.path.join(xml_dir, "DiffusionCurvePack/fille.xml"))
     w, h, n = 200, 150, 8
     out = r.render(api.default_frame_params(w, h, n, zoom_factor=512 / h), blur=True)
