@@ -8,9 +8,7 @@ CSRC      := $(PKG)/csrc
 BUILD     := build
 ARCH      := -gencode arch=compute_100a,code=sm_100a
 # -fmad=false / -ffp-contract=off: see the arithmetic contract at the top of csrc/rdc_math.h
-# per-chord shading records (device_scene.h); `make variantd NAME=norec RECORDS=` builds without them to measure the difference
-RECORDS   ?= -DRDC_SHADE_RECORDS
-NVFLAGS   := $(ARCH) -O3 -std=c++17 -lineinfo -fmad=false -Xcompiler -fPIC,-ffp-contract=off,-Wall -Iinclude $(RECORDS)
+NVFLAGS   := $(ARCH) -O3 -std=c++17 -lineinfo -fmad=false -Xcompiler -fPIC,-ffp-contract=off,-Wall -Iinclude
 CXXFLAGS  := -O2 -std=c++17 -fPIC -ffp-contract=off -Wall -Iinclude
 
 LIB       := $(PKG)/librdc_b200.so
@@ -48,15 +46,3 @@ clean:
 	$(MAKE) -C oracle clean
 
 .PHONY: all oracle sass clean
-
-# kernel-tuning variants (not shipped): make variantd NAME=w4 DEFS=-DRDC_LOCAL_WORDS=4 -> build/librdc_b200_w4.so
-variantd:
-	@mkdir -p $(BUILD)/v$(NAME)
-	for f in $(CU_SRCS); do $(NVCC) $(NVFLAGS) $(DEFS) -c $$f -o $(BUILD)/v$(NAME)/$$(basename $$f).o || exit 1; done
-	$(NVCC) $(ARCH) -shared -o $(BUILD)/librdc_b200_$(NAME).so $(BUILD)/v$(NAME)/*.o $(CPP_OBJS)
-
-# kernel-tuning variants (not shipped): make variant MINB=3 -> build/librdc_b200_mb3.so
-variant:
-	@mkdir -p $(BUILD)/v$(MINB)
-	for f in $(CU_SRCS); do $(NVCC) $(NVFLAGS) -DRDC_MIN_BLOCKS=$(MINB) -c $$f -o $(BUILD)/v$(MINB)/$$(basename $$f).o || exit 1; done
-	$(NVCC) $(ARCH) -shared -o $(BUILD)/librdc_b200_mb$(MINB).so $(BUILD)/v$(MINB)/*.o $(CPP_OBJS)

@@ -675,13 +675,11 @@ int build_scene(const rdc_scene_arrays& a, const rdc_accel_options& o, cudaStrea
     BUILD_CUDA(cudaMemcpyAsync(h_base.data(), base, (nseg + 1) * sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
     BUILD_CUDA(cudaStreamSynchronize(stream));
     std::vector<uint4> hints(2 * (size_t)n_chords);
-#ifdef RDC_SHADE_RECORDS
     // the table only pays while it stays in L2 next to everything else: 32 MB at most (250 k chords)
     const bool with_records = (size_t)n_chords * 128 <= (32u << 20) && o.shading_records >= 0;
     std::vector<float4> records(with_records ? 8 * (size_t)n_chords : 0);
     const float* scalar_v[3] = {a.blur, a.weight, a.weight_degree};
     const float* colour_v[2] = {a.color_left, a.color_right};
-#endif
     for (uint32_t sg = 0; sg < nseg; ++sg) {
       const uint32_t c = a.curve_map[sg];
       const int K = (int)(h_base[sg + 1] - h_base[sg]);
@@ -702,7 +700,6 @@ int build_scene(const rdc_scene_arrays& a, const rdc_accel_options& o, cudaStrea
         }
         hints[2 * (size_t)(h_base[sg] + k)] = make_uint4(f[0], f[1], f[2], f[3]);
         hints[2 * (size_t)(h_base[sg] + k) + 1] = make_uint4(f[4], f[5], 0u, 0u);
-#ifdef RDC_SHADE_RECORDS
         if (with_records) {
           // the largest parameter a hit on this chord can have: s = 1 (rounding is monotone, so every hit lies in between)
           const float cu_max = rdc_hit_u(k, K, 1.0f) + a.curve_index[sg];
@@ -726,13 +723,10 @@ int build_scene(const rdc_scene_arrays& a, const rdc_accel_options& o, cudaStrea
           if (K > 0xFFFF || c > 0x07FFFFFFu) meta.w &= 0x07FFFFFFu;  // does not fit the packing: never simple
           std::memcpy(&rec[7], &meta, sizeof meta);
         }
-#endif
       }
     }
     d.chord_walk = up.upload(hints.data(), hints.size());
-#ifdef RDC_SHADE_RECORDS
     d.chord_records = with_records ? up.upload(records.data(), records.size()) : nullptr;
-#endif
     BUILD_CUDA(cudaStreamSynchronize(stream));  // `hints` leaves scope
     if (up.status) return fail(up.status);
   }

@@ -68,13 +68,11 @@ struct DevScene {
   const uint32_t* seg_chord_count; // [n_segments]   K
   const SegWalk* seg_walk;         // [n_segments]
   const uint4* chord_walk;         // [2*n_chords] per chord: walk start of left, right, blur, weight | degree, portal-left
-#ifdef RDC_SHADE_RECORDS
-  // Shading records (on in the Makefile; build without -DRDC_SHADE_RECORDS to measure the difference): per chord, the two
-  // stops of every family its hits interpolate between — 8 x 16 bytes: blur, weight, exponent {u0,u1,v0,v1}; left colour
-  // {rgb0,u0} {rgb1,u1}; right colour likewise; {segment, ordinal, k | K << 16, curve | flags << 27}. flags 0x1F: every
-  // family stays inside one stop interval over the whole chord, and the record replaces the walks. nullptr: no table.
+  // Shading records: per chord, the two stops of every family its hits interpolate between — 8 x 16 bytes: blur, weight,
+  // exponent {u0,u1,v0,v1}; left colour {rgb0,u0} {rgb1,u1}; right colour likewise; {segment, ordinal, k | K << 16,
+  // curve | flags << 27}. flags 0x1F: every family stays inside one stop interval over the whole chord, and the record
+  // replaces the walks. nullptr: no table (rdc_accel_options::shading_records = -1 turns it off, to measure the difference).
   const float4* chord_records;
-#endif
   // acceleration structure: what rays touch
   const RunRecord* runs;           // [n_runs] Morton order
   const uint4* run_ids;            // [n_runs] Morton order: first chord id, segment, k of the first chord, K
@@ -105,8 +103,8 @@ struct rdc_scene {
   cudaEvent_t launched = nullptr;
   cudaStream_t launched_on = nullptr;
   bool launched_any = false;
-  uint32_t grid_blocks[64] = {};  // SM-filling grid size per kernel variant ...
-  size_t grid_dyn[64] = {};       // ... at this much dynamic shared memory
+  uint32_t grid_blocks[32] = {};  // SM-filling grid size per k_render variant (render.cu, variant_index) ...
+  size_t grid_dyn[32] = {};       // ... at this much dynamic shared memory
   float mean_run_w = 0.0f, mean_run_h = 0.0f;  // mean padded run box (local-table radius estimate)
   // partial sums of k_render's work units (a tile's rays are dealt to several units), grown on demand
   float4* part_rgbw = nullptr;
