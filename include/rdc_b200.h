@@ -119,7 +119,9 @@ void rdc_scene_destroy(rdc_scene* scene);
 #define RDC_STRIP_ROWS 8
 #define RDC_TRAVERSAL_LBVH 0
 #define RDC_TRAVERSAL_BRUTE_FORCE 1 /* every ray against every chord; validates the LBVH at full size */
-/* how primary rays find their closest chord (rdc_frame_params::route); every route gives the same bits */
+/* how primary rays find their closest chord (rdc_frame_params::route). Every route finds the same first hits. With
+ * units_per_tile pinned, the tree, the whole-scene table and the cut table give the same pixel bits; the local run table
+ * adds the samples of the rays it defers to the tree after the others, so its pixels may differ in the last bits. */
 #define RDC_ROUTE_AUTO 0        /* whole-scene run table up to 64 runs; per-tile cut table for every larger scene that
                                    has a surface-area tree (up to 65 536 runs); per-tile local run table beyond,
                                    when the view is close enough; the tree otherwise                           */
@@ -173,6 +175,20 @@ void rdc_default_frame_params(rdc_frame_params* p, uint32_t width, uint32_t heig
  * parameters of at most this size and the same rays per pixel only enqueue; without it the first call at a new
  * size does this work itself (and so synchronises once). */
 int rdc_scene_reserve(rdc_scene* scene, const rdc_frame_params* params, int host_frames, rdc_stream stream);
+/* Test hook: which render kernel rdc_render would launch for `params` on this handle, and how. Validates the parameters
+ * like rdc_render; no device work. */
+typedef struct rdc_launch_plan {
+  int mode;                /* 0 tree, 1 whole-scene run table, 2 local run table, 3 cut table              */
+  int smem;                /* nodes + runs staged in shared memory                                         */
+  int portals;             /* portal-capable kernel (the counting build always is)                         */
+  int stats;               /* counting build (rdc_frame_params::stats set)                                 */
+  int variant;             /* index into the library's kernel table                                        */
+  int built;               /* a kernel exists for that index                                               */
+  uint32_t units_per_tile; /* work units per tile actually used, after the reductions for few rays per pixel */
+  uint32_t group;          /* warps that take a tile's units together, 0 = units combine in global memory  */
+  uint64_t dynamic_smem;   /* bytes of dynamic shared memory per block                                     */
+} rdc_launch_plan;
+int rdc_scene_launch_plan(const rdc_scene* scene, const rdc_frame_params* params, rdc_launch_plan* out);
 /* image = float4[rows*W] (xyz written, w = 1), blur_map = float[rows*W]; both device pointers. */
 int rdc_render(rdc_scene* scene, const rdc_frame_params* params, float* image, float* blur_map, rdc_stream stream);
 

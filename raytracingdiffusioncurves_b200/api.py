@@ -73,10 +73,18 @@ class FrameParams(C.Structure):
     ]
 
 
+class LaunchPlan(C.Structure):
+    _fields_ = [
+        ("mode", C.c_int), ("smem", C.c_int), ("portals", C.c_int), ("stats", C.c_int), ("variant", C.c_int),
+        ("built", C.c_int), ("units_per_tile", C.c_uint32), ("group", C.c_uint32), ("dynamic_smem", C.c_uint64),
+    ]
+
+
 TRAVERSAL_LBVH = 0
 TRAVERSAL_BRUTE_FORCE = 1
 ROUTE_AUTO, ROUTE_TREE, ROUTE_LOCAL_TABLE, ROUTE_CUT_TABLE = 0, 1, 2, 3
 TREE_AUTO, TREE_MORTON, TREE_SAH = 0, 1, 2
+MODE_TREE, MODE_TABLE, MODE_LOCAL, MODE_CUT = 0, 1, 2, 3  # rdc_launch_plan::mode
 
 # every symbol include/rdc_b200.h declares, with its prototype (tests check the library exports them all)
 PROTOTYPES = {
@@ -96,6 +104,7 @@ PROTOTYPES = {
     "rdc_scene_destroy": (None, [C.c_void_p]),
     "rdc_default_frame_params": (None, [C.POINTER(FrameParams), C.c_uint32, C.c_uint32, C.c_float]),
     "rdc_scene_reserve": (C.c_int, [C.c_void_p, C.POINTER(FrameParams), C.c_int, C.c_void_p]),
+    "rdc_scene_launch_plan": (C.c_int, [C.c_void_p, C.POINTER(FrameParams), C.POINTER(LaunchPlan)]),
     "rdc_render": (C.c_int, [C.c_void_p, C.POINTER(FrameParams), C.c_void_p, C.c_void_p, C.c_void_p]),
     "rdc_render_to_frames": (C.c_int, [C.c_void_p, C.POINTER(FrameParams), C.c_uint32, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p),
                                        C.c_void_p]),
@@ -350,6 +359,12 @@ class Scene:
     def reserve(self, params: FrameParams, host_frames: bool = False, stream: int = 0) -> None:
         """rdc_scene_reserve: allocate the handle's scratch for frames like `params` ahead of the first render."""
         _check(_lib.rdc_scene_reserve(self._h, C.byref(params), int(host_frames), C.c_void_p(stream)), "rdc_scene_reserve")
+
+    def launch_plan(self, params: FrameParams) -> LaunchPlan:
+        """rdc_scene_launch_plan: the render kernel variant, units per tile and shared memory rdc_render would use."""
+        out = LaunchPlan()
+        _check(_lib.rdc_scene_launch_plan(self._h, C.byref(params), C.byref(out)), "rdc_scene_launch_plan")
+        return out
 
     def render(self, params: FrameParams, image_ptr: int, blur_map_ptr: int, stream: int = 0) -> None:
         """Enqueue one frame (rows [row_begin,row_end)) on `stream`. Pointers are device addresses."""

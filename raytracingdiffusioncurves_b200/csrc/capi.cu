@@ -423,6 +423,14 @@ int rdc_scene_reserve(rdc_scene* scene, const rdc_frame_params* params, int host
   });
 }
 
+int rdc_scene_launch_plan(const rdc_scene* scene, const rdc_frame_params* params, rdc_launch_plan* out) {
+  if (!scene || !params || !out) {
+    rdc::set_error("launch plan: null argument");
+    return RDC_E_INVALID;
+  }
+  return guarded(RDC_E_INVALID, [&]() { return rdc::launch_plan(scene, *params, out); });
+}
+
 // Enqueue-only frame: render -> [blur] on `stream`, then the copy to host memory on the handle's own copy
 // stream, so that the copy of frame f overlaps the rendering of frame f+1 (two device images, used in turn).
 int rdc_render_frame_to_host_async(rdc_scene* scene, const rdc_frame_params* params, int use_blur, float* host_image,

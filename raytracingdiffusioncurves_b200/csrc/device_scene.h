@@ -132,6 +132,7 @@ int download_chords(const rdc_scene* s, float* geom, uint32_t* ids);
 int render(rdc_scene* s, const rdc_frame_params& p, float4* image, float* blur_map, cudaStream_t stream, uint32_t n_targets = 0,
            float* const* target_images = nullptr, float* const* target_blur_maps = nullptr);
 int reserve(rdc_scene* s, const rdc_frame_params& p, cudaStream_t stream);
+int launch_plan(const rdc_scene* s, const rdc_frame_params& p, rdc_launch_plan* out);
 // blur.cu
 int gaussian_blur(float4* dest, const float4* src, const float* sigma, float4* scratch, int width, int height,
                   int row_begin, int row_end, const float* max_sigma, cudaStream_t stream, int halo_rows = -1);

@@ -1740,6 +1740,25 @@ int reserve(rdc_scene* s, const rdc_frame_params& p, cudaStream_t stream) {
   return ensure_capacity(s, L, stream);
 }
 
+int launch_plan(const rdc_scene* s, const rdc_frame_params& p, rdc_launch_plan* out) {
+  if (!s || !out) {
+    set_error("launch plan: null argument");
+    return RDC_E_INVALID;
+  }
+  if (int rc = check_params(p)) return rc;
+  const LaunchPlan L = plan_launch(s, p);
+  out->mode = L.mode;
+  out->smem = L.smem ? 1 : 0;
+  out->portals = (L.variant >> 1) & 1;
+  out->stats = L.variant & 1;
+  out->variant = L.variant;
+  out->built = kKernels[L.variant] != nullptr ? 1 : 0;
+  out->units_per_tile = L.split;
+  out->group = L.group;
+  out->dynamic_smem = L.dyn;
+  return 0;
+}
+
 int render(rdc_scene* s, const rdc_frame_params& p, float4* image, float* blur_map, cudaStream_t stream, uint32_t n_targets,
            float* const* target_images, float* const* target_blur_maps) {
   if (!s || (n_targets == 0 && (!image || !blur_map))) {
