@@ -111,6 +111,32 @@ int rdc_scene_get_info(const rdc_scene* scene, rdc_scene_info* out);
 /* Test hook: copies the chord list (original order) to host arrays of n_chords entries each.
  * geom = 4 floats per chord (ax,ay,bx,by); ids = 3 uint32 per chord (segment, k, K). Synchronous. */
 int rdc_scene_download_chords(const rdc_scene* scene, float* geom, uint32_t* ids);
+/* Test hook: copies the tables shading derives from the stop lists to host memory: seg_walk = n_segments x 64 bytes (per
+ * segment, where each stop walk starts and ends), chord_walk = n_chords x 32 bytes (per chord, where each walk stands at the
+ * chord's smallest parameter), chord_records = n_chords x 128 bytes of shading records when the handle has them (else pass
+ * NULL). Waits for the handle's last launch or update. Synchronous. */
+int rdc_scene_download_stop_tables(const rdc_scene* scene, void* seg_walk, void* chord_walk, void* chord_records);
+/* Recolours a built scene: replaces the handle's five stop families (the n_* counts, *_index, values and *_u of `arrays`,
+ * with the sentinels and padding of rdc_scene_arrays) and the three tables shading derives from them. Chords, runs, tree,
+ * cut and boxes are kept, so an edit of colours, blur, weight or weight degree costs a copy and one small kernel instead of
+ * a rebuild; edits of control points or curves need rdc_accel_build.
+ *   Equivalence: afterwards every launch on the handle (rdc_render, rdc_render_to_frames, the frame-to-host and peer calls,
+ *     every route) gives the same image, blur map, hit ids and counters, bit for bit, as the same launch on a handle that
+ *     rdc_accel_build built from `arrays` with the same options.
+ *   Geometry: the geometry fields of `arrays` must be those the handle was built from. n_vertices, n_segments and n_curves
+ *     are checked; no other geometry array is read.
+ *   Validation: the stop lists get the checks of rdc_accel_build (no null array; each curve's {start,count} inside its
+ *     list). A rejection returns RDC_E_INVALID with a message and leaves the handle unchanged.
+ *   Stream order: like a launch, the call's device work waits (stream-ordered, no host wait) for the handle's previous
+ *     launch or update, whatever stream that was on, and the handle's next launch waits for it.
+ *   Memory: the handle keeps room for the largest stop lists it has held. An update that fits overwrites them in place
+ *     and only enqueues. The handle's first update also allocates its pinned staging buffer, and an update that needs
+ *     more room waits for the handle's last launch and reallocates: those synchronise once. rdc_scene_info::device_bytes
+ *     follows.
+ *   The caller's arrays: the call packs them into the handle's pinned staging buffer before it returns, so the caller may
+ *     free or change them at once. The buffer is reused: an update first waits on the host until the previous update's
+ *     copy out of it has run, and that copy runs once the launch enqueued before the previous update has finished. */
+int rdc_scene_update_stops(rdc_scene* scene, const rdc_scene_arrays* arrays, rdc_stream stream);
 void rdc_scene_destroy(rdc_scene* scene);
 
 /* ---- per-frame render: replaces optixLaunch(pipeline, stream, d_param, sizeof(Params), &sbt, W, H, 1)

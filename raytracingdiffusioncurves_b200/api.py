@@ -101,6 +101,8 @@ PROTOTYPES = {
     "rdc_accel_build": (C.c_int, [C.POINTER(SceneArrays), C.POINTER(AccelOptions), C.c_void_p, C.POINTER(C.c_void_p)]),
     "rdc_scene_get_info": (C.c_int, [C.c_void_p, C.POINTER(SceneInfo)]),
     "rdc_scene_download_chords": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
+    "rdc_scene_download_stop_tables": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "rdc_scene_update_stops": (C.c_int, [C.c_void_p, C.POINTER(SceneArrays), C.c_void_p]),
     "rdc_scene_destroy": (None, [C.c_void_p]),
     "rdc_default_frame_params": (None, [C.POINTER(FrameParams), C.c_uint32, C.c_uint32, C.c_float]),
     "rdc_scene_reserve": (C.c_int, [C.c_void_p, C.POINTER(FrameParams), C.c_int, C.c_void_p]),
@@ -288,6 +290,36 @@ class HostScene:
         return out
 
 
+def arrays_from_numpy(d: dict) -> SceneArrays:
+    """SceneArrays over a dictionary laid out like HostScene.to_numpy() (its inverse): edit a copy of a scene in numpy
+    and pass it to Scene or Scene.update_stops. The structure keeps its arrays alive."""
+    keep = {}
+
+    def ptr(name, dtype, ctype):
+        arr = np.ascontiguousarray(d[name], dtype)
+        keep[name] = arr
+        return arr.ctypes.data_as(C.POINTER(ctype))
+
+    a = SceneArrays()
+    a.image_width, a.image_height = int(d["image_width"]), int(d["image_height"])
+    a.n_vertices = len(d["vertices"])
+    a.n_segments = len(d["segment_indices"])
+    a.n_curves = len(d["curve_connect"])
+    a.vertices = ptr("vertices", np.float32, C.c_float)
+    a.segment_indices = ptr("segment_indices", np.uint32, C.c_uint32)
+    a.curve_map = ptr("curve_map", np.uint32, C.c_uint32)
+    a.curve_index = ptr("curve_index", np.uint32, C.c_uint32)
+    a.curve_connect = ptr("curve_connect", np.int32, C.c_int32)
+    a.curve_map_inverse = ptr("curve_map_inverse", np.uint32, C.c_uint32)
+    for fam in _FAMILIES:
+        setattr(a, "n_" + fam, int(d["n_" + fam]))
+        setattr(a, fam + "_index", ptr(fam + "_index", np.uint32, C.c_uint32))
+        setattr(a, fam, ptr(fam, np.float32, C.c_float))
+        setattr(a, fam + "_u", ptr(fam + "_u", np.float32, C.c_float))
+    a._keep = keep
+    return a
+
+
 def xml_dump(path: str) -> str:
     p = C.c_void_p()
     _check(_lib.rdc_xml_dump_file(os.fsencode(path), C.byref(p)), "rdc_xml_dump_file")
@@ -329,6 +361,11 @@ class Scene:
         _check(_lib.rdc_accel_build(C.byref(arrays), C.byref(options) if options else None, C.c_void_p(stream), C.byref(h)),
                "rdc_accel_build")
         self._h = h
+        self._refresh_stats()
+        # build_scene's rule for the per-chord shading records: not turned off, and the table fits 32 MB
+        self.has_records = (options.shading_records if options else 0) >= 0 and self.stats.n_chords * 128 <= 32 << 20
+
+    def _refresh_stats(self) -> None:
         info = SceneInfo()
         _check(_lib.rdc_scene_get_info(self._h, C.byref(info)), "rdc_scene_get_info")
         self.stats = SceneStats(info.n_segments, info.n_curves, info.n_chords, info.n_runs, info.n_nodes, info.bvh_depth,
@@ -355,6 +392,23 @@ class Scene:
         ids = np.empty((n, 3), np.uint32)
         _check(_lib.rdc_scene_download_chords(self._h, geom.ctypes.data, ids.ctypes.data), "rdc_scene_download_chords")
         return geom, ids
+
+    def update_stops(self, arrays: SceneArrays, stream: int = 0) -> None:
+        """rdc_scene_update_stops: new colour, blur, weight and exponent stops on the built scene (same geometry)."""
+        _check(_lib.rdc_scene_update_stops(self._h, C.byref(arrays), C.c_void_p(stream)), "rdc_scene_update_stops")
+        self._refresh_stats()
+
+    def stop_tables(self) -> dict:
+        """rdc_scene_download_stop_tables: seg_walk uint32 [n_segments,16], chord_walk uint32 [n_chords,8], chord_records
+        float32 [n_chords,32] or None when the scene has no shading records."""
+        st = self.stats
+        seg_walk = np.empty((st.n_segments, 16), np.uint32)
+        chord_walk = np.empty((st.n_chords, 8), np.uint32)
+        records = np.empty((st.n_chords, 32), np.float32) if self.has_records else None
+        _check(_lib.rdc_scene_download_stop_tables(self._h, seg_walk.ctypes.data, chord_walk.ctypes.data,
+                                                   records.ctypes.data if records is not None else None),
+               "rdc_scene_download_stop_tables")
+        return {"seg_walk": seg_walk, "chord_walk": chord_walk, "chord_records": records}
 
     def reserve(self, params: FrameParams, host_frames: bool = False, stream: int = 0) -> None:
         """rdc_scene_reserve: allocate the handle's scratch for frames like `params` ahead of the first render."""

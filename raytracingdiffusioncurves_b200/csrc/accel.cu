@@ -281,6 +281,179 @@ __global__ void k_fill(float* dest, unsigned int n, float v) {
   for (unsigned int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += blockDim.x * gridDim.x) dest[i] = v;
 }
 
+// ---- stop tables (device_scene.h: SegWalk, chord_walk, chord_records) from the stop lists on the device ------------------
+// Threads [0, n_segments) write one segment's SegWalk each; the next n_chords threads one chord's walk starts and, when
+// `records` is set, its shading record.
+//
+// A walk over a list [start, end) of parameters u stands at W(x) = the first j >= start with j == end || !(u[j+1] < x)
+// once it has consumed every stop below x. A scan that starts anywhere in [start, W(x)] ends at W(x): no j before W(x)
+// stops it. For x <= y, every j that stops the walk at y also stops it at x, so W is non-decreasing in x, whether or not
+// u is sorted. A chord's walks stand at W(cu_min), cu_min = rdc_hit_u(k, K, 0) + ordinal, which is non-decreasing in k
+// (IEEE rounding is monotone) and at least the ordinal, where the segment's hint W(ordinal) stands. So a scan from the
+// list's start, from the segment's hint or from the previous chord's result all end at the same j: each chord scans from
+// the list's start on its own thread and finds what a sequential loop continuing from the previous chord finds.
+constexpr int kWalks = 6;  // chord_walk order: left, right, blur, weight, exponent, portal-left
+
+struct Walks {
+  const uint2* index[kWalks];
+  const float* u[kWalks];
+};
+
+__device__ __forceinline__ Walks walks_of(const DevScene& d) {
+  // the portal-left walk takes the right list's range on the LEFT u array (DeviceCode.cu:297)
+  return Walks{{d.color_left.index, d.color_right.index, d.blur.index, d.weight.index, d.weight_degree.index, d.color_right.index},
+               {d.color_left.u, d.color_right.u, d.blur.u, d.weight.u, d.weight_degree.u, d.color_left.u}};
+}
+
+__global__ void __launch_bounds__(kThreads) k_stop_tables(const DevScene d, uint4* seg_walk, uint4* chord_walk, uint4* records) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  const Walks w = walks_of(d);
+  if (i < d.n_segments) {
+    const uint32_t c = __ldg(d.curve_map + i), ordinal = __ldg(d.curve_index + i);
+    uint32_t first[kWalks], end[kWalks];
+#pragma unroll
+    for (int f = 0; f < kWalks; ++f) {
+      const uint2 r = __ldg(w.index[f] + c);
+      first[f] = rdc_walk_hint(r.x, r.y, (float)ordinal, w.u[f]);
+      end[f] = r.x + r.y;
+    }
+    uint4* out = seg_walk + 4 * (size_t)i;  // SegWalk field order; the pad words are zero
+    out[0] = make_uint4(first[0], end[0], first[1], end[1]);
+    out[1] = make_uint4(first[2], end[2], first[3], end[3]);
+    out[2] = make_uint4(first[4], end[4], c, ordinal);
+    out[3] = make_uint4(first[5], end[5], 0u, 0u);
+    return;
+  }
+  const uint32_t ch = i - d.n_segments;
+  if (ch >= d.n_chords) return;
+  const uint4 id = __ldg(d.chord_ids + ch);  // chord id, segment, k, K
+  const uint32_t sg = id.y, c = __ldg(d.curve_map + sg), ordinal = __ldg(d.curve_index + sg);
+  const int k = (int)id.z, K = (int)id.w;
+  const float cu_min = rdc_hit_u(k, K, 0.0f) + ordinal;
+  uint32_t f[kWalks];
+#pragma unroll
+  for (int fam = 0; fam < kWalks; ++fam) {
+    const uint2 r = __ldg(w.index[fam] + c);
+    f[fam] = rdc_walk_hint(r.x, r.y, cu_min, w.u[fam]);
+  }
+  chord_walk[2 * (size_t)ch] = make_uint4(f[0], f[1], f[2], f[3]);
+  chord_walk[2 * (size_t)ch + 1] = make_uint4(f[4], f[5], 0u, 0u);
+  if (!records) return;
+  // the largest parameter a hit on this chord can have: s = 1 (rounding is monotone, so every hit lies in between)
+  const float cu_max = rdc_hit_u(k, K, 1.0f) + ordinal;
+  uint32_t flags = 0;
+#pragma unroll
+  for (int fam = 0; fam < 5; ++fam) {  // family `fam` is simple when the walk would not step even at cu_max
+    const uint2 r = __ldg(w.index[fam] + c);
+    if (!(f[fam] < r.x + r.y && __ldg(w.u[fam] + f[fam] + 1) < cu_max)) flags |= 1u << fam;
+  }
+  float4* rec = reinterpret_cast<float4*>(records) + 8 * (size_t)ch;
+  const float* scalar_v[3] = {d.blur.value, d.weight.value, d.weight_degree.value};
+#pragma unroll
+  for (int sf = 0; sf < 3; ++sf) {  // blur, weight, exponent: families 2, 3, 4
+    const uint32_t j = f[2 + sf];
+    const float* us = w.u[2 + sf];
+    rec[sf] = make_float4(__ldg(us + j), __ldg(us + j + 1), __ldg(scalar_v[sf] + j), __ldg(scalar_v[sf] + j + 1));
+  }
+  const float4* rgb[2] = {d.color_left.rgb, d.color_right.rgb};
+#pragma unroll
+  for (int side = 0; side < 2; ++side) {  // left, right colour: families 0, 1
+    const uint32_t j = f[side];
+    const float4 c0 = __ldg(rgb[side] + j), c1 = __ldg(rgb[side] + j + 1);
+    rec[3 + 2 * side] = make_float4(c0.x, c0.y, c0.z, __ldg(w.u[side] + j));
+    rec[4 + 2 * side] = make_float4(c1.x, c1.y, c1.z, __ldg(w.u[side] + j + 1));
+  }
+  uint4 meta = make_uint4(sg, ordinal, (uint32_t)k | ((uint32_t)K << 16), (c & 0x07FFFFFFu) | (flags << 27));
+  if (K > 0xFFFF || c > 0x07FFFFFFu) meta.w &= 0x07FFFFFFu;  // does not fit the packing: never simple
+  records[8 * (size_t)ch + 7] = meta;
+}
+
+// Where each stop array sits in the stop block (rdc_scene::stops). Per family: the {start,count} pairs, the parameters
+// and the values (colours widened to float4 with w = 0), each at a 128-byte boundary. Both colour families hold
+// max(n_color_left, n_color_right) + 2 stops, the scalar families n + 2 (the sentinels of rdc_scene_arrays).
+struct StopLayout {
+  size_t index[5], u[5], value[5], len[5];
+  size_t bytes;
+};
+
+StopLayout stop_layout(const rdc_scene_arrays& a) {
+  const uint32_t n[5] = {a.n_color_left, a.n_color_right, a.n_blur, a.n_weight, a.n_weight_degree};
+  StopLayout L{};
+  size_t at = 0;
+  auto place = [&](size_t bytes) {
+    const size_t here = at;
+    at = (at + bytes + 127) & ~(size_t)127;
+    return here;
+  };
+  for (int f = 0; f < 5; ++f) {
+    const bool colour = f < 2;
+    L.len[f] = colour ? (size_t)std::max(a.n_color_left, a.n_color_right) + 2 : (size_t)n[f] + 2;
+    L.index[f] = place((size_t)2 * a.n_curves * sizeof(uint32_t));
+    L.u[f] = place(L.len[f] * sizeof(float));
+    L.value[f] = place(L.len[f] * (colour ? sizeof(float4) : sizeof(float)));
+  }
+  L.bytes = at;
+  return L;
+}
+
+void pack_stops(const rdc_scene_arrays& a, const StopLayout& L, void* dst) {
+  char* base = static_cast<char*>(dst);
+  const uint32_t* index[5] = {a.color_left_index, a.color_right_index, a.blur_index, a.weight_index, a.weight_degree_index};
+  const float* value[5] = {a.color_left, a.color_right, a.blur, a.weight, a.weight_degree};
+  const float* u[5] = {a.color_left_u, a.color_right_u, a.blur_u, a.weight_u, a.weight_degree_u};
+  for (int f = 0; f < 5; ++f) {
+    std::memcpy(base + L.index[f], index[f], (size_t)2 * a.n_curves * sizeof(uint32_t));
+    std::memcpy(base + L.u[f], u[f], L.len[f] * sizeof(float));
+    if (f < 2) {
+      float4* c4 = reinterpret_cast<float4*>(base + L.value[f]);
+      for (size_t i = 0; i < L.len[f]; ++i) c4[i] = make_float4(value[f][3 * i], value[f][3 * i + 1], value[f][3 * i + 2], 0.0f);
+    } else {
+      std::memcpy(base + L.value[f], value[f], L.len[f] * sizeof(float));
+    }
+  }
+}
+
+void point_stops(DevScene& d, void* block, const StopLayout& L) {
+  const char* base = static_cast<const char*>(block);
+  DevStops* st[5] = {&d.color_left, &d.color_right, &d.blur, &d.weight, &d.weight_degree};
+  for (int f = 0; f < 5; ++f) {
+    *st[f] = DevStops{};
+    st[f]->index = reinterpret_cast<const uint2*>(base + L.index[f]);
+    st[f]->u = reinterpret_cast<const float*>(base + L.u[f]);
+    if (f < 2) st[f]->rgb = reinterpret_cast<const float4*>(base + L.value[f]);
+    else st[f]->value = reinterpret_cast<const float*>(base + L.value[f]);
+  }
+}
+
+// The checks every stop list passes before it reaches the device, in rdc_accel_build and rdc_scene_update_stops alike.
+int check_stops(const rdc_scene_arrays& a, const char* who) {
+  const uint32_t* idx[5] = {a.color_left_index, a.color_right_index, a.blur_index, a.weight_index, a.weight_degree_index};
+  const float* value[5] = {a.color_left, a.color_right, a.blur, a.weight, a.weight_degree};
+  const float* u[5] = {a.color_left_u, a.color_right_u, a.blur_u, a.weight_u, a.weight_degree_u};
+  const uint32_t cnt[5] = {a.n_color_left, a.n_color_right, a.n_blur, a.n_weight, a.n_weight_degree};
+  for (int f = 0; f < 5; ++f) {
+    if (!idx[f] || !value[f] || !u[f]) {
+      set_error("%s: stop list %d has a null array", who, f);
+      return RDC_E_INVALID;
+    }
+    for (uint32_t c = 0; c < a.n_curves; ++c)
+      if ((uint64_t)idx[f][2 * c] + idx[f][2 * c + 1] > cnt[f]) {
+        set_error("%s: stop list %d of curve %u runs past its array", who, f, c);
+        return RDC_E_INVALID;
+      }
+  }
+  return 0;
+}
+
+int launch_stop_tables(const rdc_scene* s, cudaStream_t stream) {
+  const DevScene& d = s->dev;
+  k_stop_tables<<<blocks_for((size_t)d.n_segments + d.n_chords), kThreads, 0, stream>>>(
+      d, const_cast<uint4*>(reinterpret_cast<const uint4*>(d.seg_walk)), const_cast<uint4*>(d.chord_walk),
+      const_cast<uint4*>(reinterpret_cast<const uint4*>(d.chord_records)));
+  RDC_CUDA(cudaGetLastError());
+  return 0;
+}
+
 struct Uploader {
   rdc_scene* s;
   cudaStream_t stream;
@@ -337,6 +510,12 @@ void destroy_scene(rdc_scene* s) {
     }
   }
   if (s->launched) cudaEventDestroy(s->launched);
+  cudaFree(s->stops);
+  if (s->staged) {
+    cudaEventSynchronize(s->staged);  // the last update's copy has read the staging buffer
+    cudaEventDestroy(s->staged);
+  }
+  cudaFreeHost(s->staging);
   cudaFree(s->frame_scratch);
   cudaFree(s->frame_sigma);
   cudaFree(s->part_rgbw);
@@ -521,15 +700,8 @@ int build_scene(const rdc_scene_arrays& a, const rdc_accel_options& o, cudaStrea
       set_error("accel: segment %u does not address four aligned control points", i);
       return RDC_E_INVALID;
     }
+  if (int rc = check_stops(a, "accel")) return rc;
   {
-    const uint32_t* idx[5] = {a.color_left_index, a.color_right_index, a.blur_index, a.weight_index, a.weight_degree_index};
-    const uint32_t cnt[5] = {a.n_color_left, a.n_color_right, a.n_blur, a.n_weight, a.n_weight_degree};
-    for (int f = 0; f < 5; ++f)
-      for (uint32_t c = 0; c < a.n_curves; ++c)
-        if ((uint64_t)idx[f][2 * c] + idx[f][2 * c + 1] > cnt[f]) {
-          set_error("accel: stop list %d of curve %u runs past its array", f, c);
-          return RDC_E_INVALID;
-        }
     // segments of a curve are consecutive: curve c owns [curve_map_inverse[c], next curve's first segment)
     std::vector<uint32_t> seg_count(a.n_curves, 0u);
     for (uint32_t sg = 0; sg < a.n_segments; ++sg) {
@@ -576,57 +748,25 @@ int build_scene(const rdc_scene_arrays& a, const rdc_accel_options& o, cudaStrea
   d.curve_index = up.upload(a.curve_index, a.n_segments);
   d.curve_connect = up.upload(a.curve_connect, a.n_curves);
   d.curve_map_inverse = up.upload(a.curve_map_inverse, a.n_curves);
-  const size_t colour_len = (size_t)(a.n_color_left > a.n_color_right ? a.n_color_left : a.n_color_right) + 2;
-  auto colours = [&](const uint32_t* index, const float* rgb, const float* u) {
-    DevStops st{};
-    st.index = reinterpret_cast<const uint2*>(up.upload(index, (size_t)2 * a.n_curves));
-    st.u = up.upload(u, colour_len);
-    std::vector<float4> c4(colour_len);
-    for (size_t i = 0; i < colour_len; ++i) c4[i] = make_float4(rgb[3 * i], rgb[3 * i + 1], rgb[3 * i + 2], 0.0f);
-    st.rgb = up.upload(c4.data(), c4.size());
-    return st;
-  };
-  auto scalars = [&](const uint32_t* index, const float* value, const float* u, uint32_t n) {
-    DevStops st{};
-    st.index = reinterpret_cast<const uint2*>(up.upload(index, (size_t)2 * a.n_curves));
-    st.u = up.upload(u, (size_t)n + 2);
-    st.value = up.upload(value, (size_t)n + 2);
-    return st;
-  };
-  d.color_left = colours(a.color_left_index, a.color_left, a.color_left_u);
-  d.color_right = colours(a.color_right_index, a.color_right, a.color_right_u);
-  d.blur = scalars(a.blur_index, a.blur, a.blur_u, a.n_blur);
-  d.weight = scalars(a.weight_index, a.weight, a.weight_u, a.n_weight);
-  d.weight_degree = scalars(a.weight_degree_index, a.weight_degree, a.weight_degree_u, a.n_weight_degree);
+  s->n_vertices = a.n_vertices;
+  // the stop lists, packed into one block of their own (rdc_scene_update_stops may replace it); the build reads back and
+  // synchronises anyway, so it copies from pageable memory and leaves the pinned staging buffer to the first update
+  const StopLayout stop_at = stop_layout(a);
+  std::vector<char> packed(stop_at.bytes);
+  pack_stops(a, stop_at, packed.data());
+  if (!up.status) {
+    cudaError_t e = cudaMalloc(&s->stops, stop_at.bytes);
+    if (e == cudaSuccess) {
+      s->stops_capacity = stop_at.bytes;
+      s->info.device_bytes += stop_at.bytes;
+      e = cudaMemcpyAsync(s->stops, packed.data(), stop_at.bytes, cudaMemcpyHostToDevice, stream);
+    }
+    if (e != cudaSuccess) up.status = cuda_fail(e, "stop lists");
+  }
+  point_stops(d, s->stops, stop_at);
   d.n_segments = a.n_segments;
   d.n_curves = a.n_curves;
-  {
-    std::vector<SegWalk> walk(a.n_segments);
-    for (uint32_t sg = 0; sg < a.n_segments; ++sg) {
-      const uint32_t c = a.curve_map[sg];
-      if (c >= a.n_curves) {
-        set_error("accel: segment %u maps to a missing curve", sg);
-        destroy_scene(s);
-        return RDC_E_INVALID;
-      }
-      const float u_min = (float)a.curve_index[sg];
-      SegWalk w{};
-      auto range = [&](const uint32_t* index, const float* us, uint32_t& first, uint32_t& end) {
-        first = rdc_walk_hint(index[2 * c], index[2 * c + 1], u_min, us);
-        end = index[2 * c] + index[2 * c + 1];
-      };
-      range(a.color_left_index, a.color_left_u, w.left_first, w.left_end);
-      range(a.color_right_index, a.color_right_u, w.right_first, w.right_end);
-      range(a.blur_index, a.blur_u, w.blur_first, w.blur_end);
-      range(a.weight_index, a.weight_u, w.weight_first, w.weight_end);
-      range(a.weight_degree_index, a.weight_degree_u, w.degree_first, w.degree_end);
-      range(a.color_right_index, a.color_left_u, w.portal_left_first, w.portal_left_end);
-      w.curve = c;
-      w.ordinal = a.curve_index[sg];
-      walk[sg] = w;
-    }
-    d.seg_walk = up.upload(walk.data(), walk.size());
-  }
+  d.seg_walk = up.alloc<SegWalk>(a.n_segments);
 
   // ---- chords ------------------------------------------------------------------------------------
   const uint32_t nseg = a.n_segments;
@@ -667,73 +807,15 @@ int build_scene(const rdc_scene_arrays& a, const rdc_accel_options& o, cudaStrea
     return fail(RDC_E_LIMIT);
   }
 
-  // Per-chord walk hints: where each stop walk stands once it has consumed every stop below the chord's
-  // smallest curve parameter (rdc_walk_hint). Hits on the chord start their walks there — usually zero
-  // steps — instead of at the segment's hint. Exact by the same argument as the per-segment hints.
-  {
-    std::vector<uint32_t> h_base(nseg + 1);
-    BUILD_CUDA(cudaMemcpyAsync(h_base.data(), base, (nseg + 1) * sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
-    BUILD_CUDA(cudaStreamSynchronize(stream));
-    std::vector<uint4> hints(2 * (size_t)n_chords);
-    // the table only pays while it stays in L2 next to everything else: 32 MB at most (250 k chords)
-    const bool with_records = (size_t)n_chords * 128 <= (32u << 20) && o.shading_records >= 0;
-    std::vector<float4> records(with_records ? 8 * (size_t)n_chords : 0);
-    const float* scalar_v[3] = {a.blur, a.weight, a.weight_degree};
-    const float* colour_v[2] = {a.color_left, a.color_right};
-    for (uint32_t sg = 0; sg < nseg; ++sg) {
-      const uint32_t c = a.curve_map[sg];
-      const int K = (int)(h_base[sg + 1] - h_base[sg]);
-      uint32_t prev[6] = {a.color_left_index[2 * c], a.color_right_index[2 * c], a.blur_index[2 * c], a.weight_index[2 * c],
-                          a.weight_degree_index[2 * c], a.color_right_index[2 * c]};
-      const uint32_t* idx[6] = {a.color_left_index, a.color_right_index, a.blur_index, a.weight_index, a.weight_degree_index,
-                                a.color_right_index};
-      const float* us[6] = {a.color_left_u, a.color_right_u, a.blur_u, a.weight_u, a.weight_degree_u, a.color_left_u};
-      for (int k = 0; k < K; ++k) {
-        const float cu_min = rdc_hit_u(k, K, 0.0f) + a.curve_index[sg];
-        uint32_t f[6];
-        for (int fam = 0; fam < 6; ++fam) {
-          // continue from the previous chord's position: the walk is monotone in the parameter
-          const uint32_t start = idx[fam][2 * c], end = start + idx[fam][2 * c + 1];
-          uint32_t j = prev[fam];
-          while (j < end && us[fam][j + 1] < cu_min) j++;
-          prev[fam] = f[fam] = j;
-        }
-        hints[2 * (size_t)(h_base[sg] + k)] = make_uint4(f[0], f[1], f[2], f[3]);
-        hints[2 * (size_t)(h_base[sg] + k) + 1] = make_uint4(f[4], f[5], 0u, 0u);
-        if (with_records) {
-          // the largest parameter a hit on this chord can have: s = 1 (rounding is monotone, so every hit lies in between)
-          const float cu_max = rdc_hit_u(k, K, 1.0f) + a.curve_index[sg];
-          uint32_t flags = 0;
-          for (int fam = 0; fam < 5; ++fam) {  // family `fam` is simple when the walk would not step even at cu_max
-            const uint32_t end = idx[fam][2 * c] + idx[fam][2 * c + 1];
-            if (!(f[fam] < end && us[fam][f[fam] + 1] < cu_max)) flags |= 1u << fam;
-          }
-          float4* rec = &records[8 * (size_t)(h_base[sg] + k)];
-          for (int sf = 0; sf < 3; ++sf) {  // blur, weight, exponent: families 2, 3, 4
-            const uint32_t j = f[2 + sf];
-            rec[sf] = make_float4(us[2 + sf][j], us[2 + sf][j + 1], scalar_v[sf][j], scalar_v[sf][j + 1]);
-          }
-          for (int side = 0; side < 2; ++side) {  // left, right colour: families 0, 1
-            const uint32_t j = f[side];
-            const float* v = colour_v[side];
-            rec[3 + 2 * side] = make_float4(v[3 * j], v[3 * j + 1], v[3 * j + 2], us[side][j]);
-            rec[4 + 2 * side] = make_float4(v[3 * (j + 1)], v[3 * (j + 1) + 1], v[3 * (j + 1) + 2], us[side][j + 1]);
-          }
-          uint4 meta = make_uint4(sg, a.curve_index[sg], (uint32_t)k | ((uint32_t)K << 16), (c & 0x07FFFFFFu) | (flags << 27));
-          if (K > 0xFFFF || c > 0x07FFFFFFu) meta.w &= 0x07FFFFFFu;  // does not fit the packing: never simple
-          std::memcpy(&rec[7], &meta, sizeof meta);
-        }
-      }
-    }
-    d.chord_walk = up.upload(hints.data(), hints.size());
-    d.chord_records = with_records ? up.upload(records.data(), records.size()) : nullptr;
-    BUILD_CUDA(cudaStreamSynchronize(stream));  // `hints` leaves scope
-    if (up.status) return fail(up.status);
-  }
-
   // chords stay in original order (hit ids, download hook); runs + tree are what rays touch
   float4* chord_geom = up.alloc<float4>(n_chords);
   uint4* chord_ids = up.alloc<uint4>(n_chords);
+  // Per-chord walk starts: where each stop walk stands once it has consumed every stop below the chord's smallest curve
+  // parameter. Hits on the chord start their walks there (usually zero steps) instead of at the segment's hint.
+  d.chord_walk = up.alloc<uint4>(2 * (size_t)n_chords);
+  // the shading records only pay while they stay in L2 next to everything else: 32 MB at most (250 k chords)
+  const bool with_records = (size_t)n_chords * 128 <= (32u << 20) && o.shading_records >= 0;
+  d.chord_records = with_records ? up.alloc<float4>(8 * (size_t)n_chords) : nullptr;
   uint32_t* run_counts = up.alloc<uint32_t>(nseg + 1);
   uint32_t* run_base = up.alloc<uint32_t>(nseg + 1);
   unsigned int* max_depth = up.alloc<unsigned int>(1);
@@ -745,6 +827,9 @@ int build_scene(const rdc_scene_arrays& a, const rdc_accel_options& o, cudaStrea
   k_emit_chords<<<blocks_for(n_chords), kThreads, 0, stream>>>(d.vertices, d.segment_indices, base, nseg, n_chords,
                                                                chord_geom, chord_ids, bounds);
   BUILD_CUDA(cudaGetLastError());
+  d.chord_ids = chord_ids;
+  d.n_chords = n_chords;
+  if (int rc = launch_stop_tables(s, stream)) return fail(rc);
   BUILD_CUDA(cudaMemsetAsync(run_counts, 0, (nseg + 1) * sizeof(uint32_t), stream));
   // Leaf size: long runs make a shallow tree (good when curves are sparse: few boxes overlap), short runs
   // keep leaf boxes tight (good when curves are dense). Mean chord spacing ~ extent / sqrt(#chords).
@@ -878,14 +963,12 @@ int build_scene(const rdc_scene_arrays& a, const rdc_accel_options& o, cudaStrea
   }
 
   d.chord_geom = chord_geom;
-  d.chord_ids = chord_ids;
   d.seg_chord_base = base;
   d.seg_chord_count = counts;
   d.runs = runs;
   d.run_ids = run_ids;
   d.run_box = run_box;
   d.nodes = nodes;
-  d.n_chords = n_chords;
   d.n_runs = n_runs;
   d.n_nodes = n_nodes;
   d.root_box = make_float4(hb.xmin - pad, hb.ymin - pad, hb.xmax + pad, hb.ymax + pad);
@@ -918,6 +1001,82 @@ int download_chords(const rdc_scene* s, float* geom, uint32_t* ids) {
     }
     ids[3 * i + 0] = id[i].y; ids[3 * i + 1] = id[i].z; ids[3 * i + 2] = id[i].w;
   }
+  return 0;
+}
+
+// New stop lists on a built handle: validate everything first (a rejection leaves the handle as it was), make room, then
+// pack into the pinned staging buffer and enqueue copy + k_stop_tables behind the handle's previous launch or update.
+int update_stops(rdc_scene* s, const rdc_scene_arrays& a, cudaStream_t stream) {
+  if (a.n_vertices != s->n_vertices || a.n_segments != s->dev.n_segments || a.n_curves != s->dev.n_curves) {
+    set_error("update stops: the arrays have %u vertices, %u segments and %u curves, the scene was built from %u, %u and %u",
+              a.n_vertices, a.n_segments, a.n_curves, s->n_vertices, s->dev.n_segments, s->dev.n_curves);
+    return RDC_E_INVALID;
+  }
+  if (int rc = check_stops(a, "update stops")) return rc;
+  const StopLayout L = stop_layout(a);
+  if (!s->launched) RDC_CUDA(cudaEventCreateWithFlags(&s->launched, cudaEventDisableTiming));
+  const bool grow = L.bytes > s->stops_capacity;
+  const size_t capacity = grow ? L.bytes : s->stops_capacity;
+  if (s->staging_capacity < capacity) {  // the handle's first update, or lists larger than any it has held
+    void* fresh = nullptr;
+    RDC_CUDA(cudaMallocHost(&fresh, capacity));
+    if (s->staged) {
+      cudaError_t e = cudaEventSynchronize(s->staged);
+      if (e != cudaSuccess) {
+        cudaFreeHost(fresh);
+        return cuda_fail(e, "cudaEventSynchronize(staged)");
+      }
+    } else {
+      cudaError_t e = cudaEventCreateWithFlags(&s->staged, cudaEventDisableTiming);
+      if (e != cudaSuccess) {
+        cudaFreeHost(fresh);
+        return cuda_fail(e, "cudaEventCreate(staged)");
+      }
+    }
+    cudaFreeHost(s->staging);
+    s->staging = fresh;
+    s->staging_capacity = capacity;
+  } else {
+    RDC_CUDA(cudaEventSynchronize(s->staged));  // the previous update's copy has left the staging buffer
+  }
+  if (grow) {  // the old block may still be read by the handle's last launch: wait for it, then replace the block
+    void* fresh = nullptr;
+    RDC_CUDA(cudaMalloc(&fresh, capacity));
+    if (s->launched_any) {
+      cudaError_t e = cudaEventSynchronize(s->launched);
+      if (e != cudaSuccess) {
+        cudaFree(fresh);
+        return cuda_fail(e, "cudaEventSynchronize(launched)");
+      }
+    }
+    cudaFree(s->stops);
+    s->info.device_bytes += capacity - s->stops_capacity;
+    s->stops = fresh;
+    s->stops_capacity = capacity;
+  }
+  pack_stops(a, L, s->staging);
+  // like a launch: the device work waits for the handle's previous launch or update, whatever stream that was on
+  if (s->launched_any && s->launched_on != stream) RDC_CUDA(cudaStreamWaitEvent(stream, s->launched, 0));
+  RDC_CUDA(cudaMemcpyAsync(s->stops, s->staging, L.bytes, cudaMemcpyHostToDevice, stream));
+  RDC_CUDA(cudaEventRecord(s->staged, stream));
+  point_stops(s->dev, s->stops, L);
+  if (int rc = launch_stop_tables(s, stream)) return rc;
+  RDC_CUDA(cudaEventRecord(s->launched, stream));
+  s->launched_on = stream;
+  s->launched_any = true;
+  return 0;
+}
+
+int download_stop_tables(const rdc_scene* s, void* seg_walk, void* chord_walk, void* chord_records) {
+  const DevScene& d = s->dev;
+  if (chord_records && !d.chord_records) {
+    set_error("download stop tables: the scene has no shading records");
+    return RDC_E_INVALID;
+  }
+  if (s->launched_any) RDC_CUDA(cudaEventSynchronize(s->launched));
+  RDC_CUDA(cudaMemcpy(seg_walk, d.seg_walk, d.n_segments * sizeof(SegWalk), cudaMemcpyDeviceToHost));
+  RDC_CUDA(cudaMemcpy(chord_walk, d.chord_walk, 2 * (size_t)d.n_chords * sizeof(uint4), cudaMemcpyDeviceToHost));
+  if (chord_records) RDC_CUDA(cudaMemcpy(chord_records, d.chord_records, 8 * (size_t)d.n_chords * sizeof(float4), cudaMemcpyDeviceToHost));
   return 0;
 }
 

@@ -286,6 +286,22 @@ int rdc_scene_download_chords(const rdc_scene* scene, float* geom, uint32_t* ids
   return guarded(RDC_E_INVALID, [&]() { return rdc::download_chords(scene, geom, ids); });
 }
 
+int rdc_scene_update_stops(rdc_scene* scene, const rdc_scene_arrays* arrays, rdc_stream stream) {
+  if (!scene || !arrays) {
+    rdc::set_error("update stops: null argument");
+    return RDC_E_INVALID;
+  }
+  return guarded(RDC_E_INVALID, [&]() { return rdc::update_stops(scene, *arrays, (cudaStream_t)stream); });
+}
+
+int rdc_scene_download_stop_tables(const rdc_scene* scene, void* seg_walk, void* chord_walk, void* chord_records) {
+  if (!scene || !seg_walk || !chord_walk) {
+    rdc::set_error("download stop tables: null argument");
+    return RDC_E_INVALID;
+  }
+  return guarded(RDC_E_INVALID, [&]() { return rdc::download_stop_tables(scene, seg_walk, chord_walk, chord_records); });
+}
+
 void rdc_scene_destroy(rdc_scene* scene) { rdc::destroy_scene(scene); }
 
 void rdc_default_frame_params(rdc_frame_params* p, uint32_t width, uint32_t height, float rays_per_pixel) {

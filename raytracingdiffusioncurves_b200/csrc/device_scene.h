@@ -92,7 +92,15 @@ struct rdc_scene {
   int sm_count = 0;  // multiprocessors of `device`
   DevScene dev{};
   rdc_scene_info info{};
+  uint32_t n_vertices = 0;         // of the arrays the handle was built from (rdc_scene_update_stops checks it)
   std::vector<void*> allocations;  // everything to cudaFree on destroy
+  // the five stop families in one device block (accel.cu, StopLayout), grown by rdc_scene_update_stops and never shrunk;
+  // updates pack the caller's lists into the pinned staging buffer, which `staged` guards until the copy has read it
+  void* stops = nullptr;
+  size_t stops_capacity = 0;
+  void* staging = nullptr;
+  size_t staging_capacity = 0;
+  cudaEvent_t staged = nullptr;
   // per-N table of the iterated base directions (DeviceCode.cu:110-112,167-171)
   float2* base_dirs = nullptr;
   float base_dirs_n = -1.0f;
@@ -128,6 +136,8 @@ int cuda_fail(cudaError_t e, const char* what);
 int build_scene(const rdc_scene_arrays& a, const rdc_accel_options& o, cudaStream_t stream, rdc_scene** out);
 void destroy_scene(rdc_scene* s);
 int download_chords(const rdc_scene* s, float* geom, uint32_t* ids);
+int update_stops(rdc_scene* s, const rdc_scene_arrays& a, cudaStream_t stream);
+int download_stop_tables(const rdc_scene* s, void* seg_walk, void* chord_walk, void* chord_records);
 // render.cu
 int render(rdc_scene* s, const rdc_frame_params& p, float4* image, float* blur_map, cudaStream_t stream, uint32_t n_targets = 0,
            float* const* target_images = nullptr, float* const* target_blur_maps = nullptr);
