@@ -13,7 +13,7 @@ CXXFLAGS  := -O2 -std=c++17 -fPIC -ffp-contract=off -Wall -Iinclude
 
 LIB       := $(PKG)/librdc_b200.so
 CLI       := $(PKG)/OptixHello
-CU_SRCS   := $(CSRC)/accel.cu $(CSRC)/render.cu $(CSRC)/blur.cu $(CSRC)/capi.cu $(CSRC)/microbench.cu $(CSRC)/extras.cu $(CSRC)/peer.cu
+CU_SRCS   := $(CSRC)/accel.cu $(CSRC)/render.cu $(CSRC)/blur.cu $(CSRC)/capi.cu $(CSRC)/microbench.cu $(CSRC)/extras.cu $(CSRC)/peer.cu $(CSRC)/pick.cu
 CPP_SRCS  := $(CSRC)/xml_dom.cpp $(CSRC)/ingest.cpp $(CSRC)/synth.cpp $(CSRC)/jpeg.cpp
 CU_OBJS   := $(patsubst $(CSRC)/%.cu,$(BUILD)/%.cu.o,$(CU_SRCS))
 CPP_OBJS  := $(patsubst $(CSRC)/%.cpp,$(BUILD)/%.cpp.o,$(CPP_SRCS))

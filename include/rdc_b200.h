@@ -228,6 +228,55 @@ int rdc_render(rdc_scene* scene, const rdc_frame_params* params, float* image, f
 int rdc_render_to_frames(rdc_scene* scene, const rdc_frame_params* params, uint32_t n_targets, float* const* images,
                          float* const* blur_maps, rdc_stream stream);
 
+/* ---- picking: the curve under a point (an editor's click, or every pixel of a view for hover and selection) ----
+ *
+ * Nearest: the pick of a point p is the chord with the smallest (d2, chord id) among all chords with d2 <= max_distance^2
+ *   (fp32 product), where d2 = |p - c|^2 and c is the point of the chord nearest to p, both computed in fp32 exactly as
+ *   rdc_point_chord (csrc/rdc_math.h) computes them. max_distance = +INF takes the nearest chord whatever its distance.
+ *   The fields are those of that chord; the tree is only a faster way to the brute force's answer, so both tree builders
+ *   and every run length give the same bits.
+ * Miss: nothing within range, or a point with a NaN or infinite coordinate: chord, segment and curve RDC_PICK_NONE,
+ *   flags 0, distance +INF, u, x and y NaN, and the three stop vectors NaN.
+ * Side: RDC_PICK_RIGHT is set when rdc_is_ray_right(local u, D = c - p, control points, use_diffusion_curve_save) holds,
+ *   i.e. a ray from p toward c would shade the colour_right list. At distance 0 (D = 0) the normal's dot product is 0, so
+ *   the pick is on the right side when use_diffusion_curve_save is 0 and on the left side when it is 1.
+ * Stops: at the pick's u, with the walks terminal shading uses (the walk starts of seg_walk and chord_walk, or the chord's
+ *   shading record when it replaces the walks; rdc_interp_from, rdc_lerp_stop, rdc_lerp_color). On a portal curve they are
+ *   the curve's own left and right lists, not the portal filter (which walks the right list's range on the left arrays,
+ *   DeviceCode.cu:297).
+ * Stream order: like a launch, the pick waits (stream-ordered, no host wait) for the handle's previous launch or update,
+ *   whatever stream that was on, and the handle's next launch waits for the pick. A pick enqueued after
+ *   rdc_scene_update_stops sees the new stops on any stream.
+ * No scratch: a pick allocates nothing and never synchronises; it only enqueues, from the first call on.
+ * Validation: RDC_E_INVALID with a message for a null scene or out, null points with n > 0, max_distance NaN or <= 0,
+ *   and (frame form) null params, zero width, an empty or out-of-range row band, or strip_stride > 1. n == 0 enqueues
+ *   nothing. */
+#define RDC_PICK_NONE 0xFFFFFFFFu
+#define RDC_PICK_RIGHT 1u  /* the point lies on the side shaded with color_right (rdc_is_ray_right with D = c - p) */
+#define RDC_PICK_PORTAL 2u /* the curve is a portal (curve_connect >= 0)                                       */
+typedef struct rdc_pick {
+  uint32_t chord;   /* id of the nearest chord (rdc_scene_download_chords order); RDC_PICK_NONE: nothing within range */
+  uint32_t segment; /* its spline segment                                                                          */
+  uint32_t curve;   /* its curve                                                                                   */
+  uint32_t flags;   /* RDC_PICK_RIGHT | RDC_PICK_PORTAL                                                            */
+  float u;          /* curve parameter as the *_u stop lists use it: ordinal + (k + s) / K, the float ops of shading */
+  float distance;   /* sqrtf(d2), scene units                                                                      */
+  float x, y;       /* c, the nearest point on the chord                                                           */
+} rdc_pick;         /* 32 bytes */
+
+/* points: device float2[n], scene (XML pixel) coordinates. out: device rdc_pick[n]. stops: NULL or device float4[3n]
+ * (16-byte aligned): {left r, g, b, blur}, {right r, g, b, weight}, {weight_degree, 0, 0, 0} at the pick's u. */
+int rdc_scene_pick(rdc_scene* scene, const float* points, uint32_t n, float max_distance, int use_diffusion_curve_save,
+                   rdc_pick* out, float* stops, rdc_stream stream);
+/* One pick per pixel centre (rdc_view_pixel_to_scene) of rows [row_begin,row_end) of the view `params` describes: out
+ * and stops are band-local like rdc_render's image (row row_begin first). Reads image_width, image_height, zoom_factor,
+ * offset_x, offset_y, use_diffusion_curve_save and the row band; ignores the ray fields. strip_stride > 1 is rejected. */
+int rdc_scene_pick_frame(rdc_scene* scene, const rdc_frame_params* params, float max_distance, rdc_pick* out, float* stops,
+                         rdc_stream stream);
+/* Host: the scene point rdc_scene_pick_frame picks for pixel (ix, iy) of the full frame — the render's ray origin before
+ * the anti-aliasing jitter plus half a pixel, the centre of the square the pixel's rays start from. For a cursor click. */
+int rdc_view_pixel_to_scene(const rdc_frame_params* params, uint32_t ix, uint32_t iy, float* x, float* y);
+
 /* ---- one frame over the GPUs of a box (SURVEY.md 8e), all in C: frames the ranks share, a barrier in peer memory,
  *      and the per-frame drivers. A "rank" is one GPU with its own rdc_scene (scene and tree are replicated); ranks may
  *      live in one process (one host thread enqueueing on every device: rdc_peer_frames_connect_local) or in one process

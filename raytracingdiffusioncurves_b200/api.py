@@ -85,6 +85,10 @@ TRAVERSAL_BRUTE_FORCE = 1
 ROUTE_AUTO, ROUTE_TREE, ROUTE_LOCAL_TABLE, ROUTE_CUT_TABLE = 0, 1, 2, 3
 TREE_AUTO, TREE_MORTON, TREE_SAH = 0, 1, 2
 MODE_TREE, MODE_TABLE, MODE_LOCAL, MODE_CUT = 0, 1, 2, 3  # rdc_launch_plan::mode
+PICK_NONE, PICK_RIGHT, PICK_PORTAL = 0xFFFFFFFF, 1, 2  # rdc_pick::chord for a miss, rdc_pick::flags bits
+# struct rdc_pick (32 bytes); stops of a pick are three float4: {left rgb, blur}, {right rgb, weight}, {weight_degree, 0, 0, 0}
+PICK_DTYPE = np.dtype([("chord", np.uint32), ("segment", np.uint32), ("curve", np.uint32), ("flags", np.uint32),
+                       ("u", np.float32), ("distance", np.float32), ("x", np.float32), ("y", np.float32)])
 
 # every symbol include/rdc_b200.h declares, with its prototype (tests check the library exports them all)
 PROTOTYPES = {
@@ -110,6 +114,9 @@ PROTOTYPES = {
     "rdc_render": (C.c_int, [C.c_void_p, C.POINTER(FrameParams), C.c_void_p, C.c_void_p, C.c_void_p]),
     "rdc_render_to_frames": (C.c_int, [C.c_void_p, C.POINTER(FrameParams), C.c_uint32, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p),
                                        C.c_void_p]),
+    "rdc_scene_pick": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_float, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "rdc_scene_pick_frame": (C.c_int, [C.c_void_p, C.POINTER(FrameParams), C.c_float, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "rdc_view_pixel_to_scene": (C.c_int, [C.POINTER(FrameParams), C.c_uint32, C.c_uint32, f32p, f32p]),
     "rdc_peer_frames_create": (C.c_int, [C.c_uint32, C.c_uint32, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
     "rdc_peer_frames_export": (C.c_int, [C.c_void_p, C.c_void_p]),
     "rdc_peer_frames_connect_ipc": (C.c_int, [C.c_void_p, C.c_void_p]),
@@ -433,6 +440,19 @@ class Scene:
         sigmas = (C.c_void_p * n)(*blur_map_ptrs)
         _check(_lib.rdc_render_to_frames(self._h, C.byref(params), n, images, sigmas, C.c_void_p(stream)), "rdc_render_to_frames")
 
+    def pick(self, points_ptr: int, n: int, out_ptr: int, stops_ptr: int = 0, max_distance: float = float("inf"),
+             use_diffusion_curve_save: int = 1, stream: int = 0) -> None:
+        """rdc_scene_pick: the nearest chord to each of n device float2 points, into device records of PICK_DTYPE (and,
+        when stops_ptr is given, three float4 of stop values per point). Enqueue-only."""
+        _check(_lib.rdc_scene_pick(self._h, C.c_void_p(points_ptr), n, max_distance, int(use_diffusion_curve_save),
+                                   C.c_void_p(out_ptr), C.c_void_p(stops_ptr), C.c_void_p(stream)), "rdc_scene_pick")
+
+    def pick_frame(self, params: FrameParams, out_ptr: int, stops_ptr: int = 0, max_distance: float = float("inf"),
+                   stream: int = 0) -> None:
+        """rdc_scene_pick_frame: one pick per pixel centre of the band of `params` (band-local, like render)."""
+        _check(_lib.rdc_scene_pick_frame(self._h, C.byref(params), max_distance, C.c_void_p(out_ptr), C.c_void_p(stops_ptr),
+                                         C.c_void_p(stream)), "rdc_scene_pick_frame")
+
     def render_frame_to_host(self, params: FrameParams, use_blur: bool, host_image_ptr: int, stream: int = 0) -> None:
         _check(_lib.rdc_render_frame_to_host(self._h, C.byref(params), int(use_blur), C.c_void_p(host_image_ptr),
                                              C.c_void_p(stream)), "rdc_render_frame_to_host")
@@ -545,6 +565,13 @@ def gaussian_blur_band(dest_ptr: int, src_ptr: int, sigma_ptr: int, scratch_ptr:
     _check(_lib.rdc_gaussian_blur_band(C.c_void_p(dest_ptr), C.c_void_p(src_ptr), C.c_void_p(sigma_ptr), C.c_void_p(scratch_ptr),
                                        width, height, row_begin, row_end, halo_rows, C.c_void_p(max_sigma_ptr),
                                        C.c_void_p(stream)), "rdc_gaussian_blur_band")
+
+
+def view_pixel_to_scene(params: FrameParams, ix: int, iy: int) -> tuple[float, float]:
+    """rdc_view_pixel_to_scene: the scene point Scene.pick_frame picks for pixel (ix, iy), e.g. under a cursor click."""
+    x, y = C.c_float(), C.c_float()
+    _check(_lib.rdc_view_pixel_to_scene(C.byref(params), ix, iy, C.byref(x), C.byref(y)), "rdc_view_pixel_to_scene")
+    return x.value, y.value
 
 
 def image_to_rgba8(image: np.ndarray, flip: bool) -> np.ndarray:

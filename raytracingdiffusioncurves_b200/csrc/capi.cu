@@ -352,6 +352,32 @@ int rdc_render_to_frames(rdc_scene* scene, const rdc_frame_params* params, uint3
   });
 }
 
+int rdc_scene_pick(rdc_scene* scene, const float* points, uint32_t n, float max_distance, int use_diffusion_curve_save,
+                   rdc_pick* out, float* stops, rdc_stream stream) {
+  return guarded(RDC_E_INVALID, [&]() {
+    return rdc::pick(scene, points, n, max_distance, use_diffusion_curve_save, out, stops, (cudaStream_t)stream);
+  });
+}
+
+int rdc_scene_pick_frame(rdc_scene* scene, const rdc_frame_params* params, float max_distance, rdc_pick* out, float* stops,
+                         rdc_stream stream) {
+  return guarded(RDC_E_INVALID, [&]() { return rdc::pick_frame(scene, params, max_distance, out, stops, (cudaStream_t)stream); });
+}
+
+int rdc_view_pixel_to_scene(const rdc_frame_params* params, uint32_t ix, uint32_t iy, float* x, float* y) {
+  if (!params || !x || !y) {
+    rdc::set_error("view pixel to scene: null argument");
+    return RDC_E_INVALID;
+  }
+  if (ix >= params->image_width || iy >= params->image_height) {
+    rdc::set_error("view pixel to scene: pixel (%u, %u) is outside the %ux%u frame", ix, iy, params->image_width, params->image_height);
+    return RDC_E_INVALID;
+  }
+  *x = rdc_pixel_centre_x(params->image_width, params->zoom_factor, params->offset_x, ix);
+  *y = rdc_pixel_centre_y(params->image_height, params->zoom_factor, params->offset_y, params->use_diffusion_curve_save != 0, iy);
+  return 0;
+}
+
 int rdc_gaussian_blur(void* dest, const void* source, const float* sigma, void* scratch, int width, int height,
                       int row_begin, int row_end, const float* max_sigma, rdc_stream stream) {
   return rdc::gaussian_blur(static_cast<float4*>(dest), static_cast<const float4*>(source), sigma,

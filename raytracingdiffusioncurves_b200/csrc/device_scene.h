@@ -143,6 +143,10 @@ int render(rdc_scene* s, const rdc_frame_params& p, float4* image, float* blur_m
            float* const* target_images = nullptr, float* const* target_blur_maps = nullptr);
 int reserve(rdc_scene* s, const rdc_frame_params& p, cudaStream_t stream);
 int launch_plan(const rdc_scene* s, const rdc_frame_params& p, rdc_launch_plan* out);
+// pick.cu
+int pick(rdc_scene* s, const float* points, uint32_t n, float max_distance, int orzan, rdc_pick* out, float* stops,
+         cudaStream_t stream);
+int pick_frame(rdc_scene* s, const rdc_frame_params* p, float max_distance, rdc_pick* out, float* stops, cudaStream_t stream);
 // blur.cu
 int gaussian_blur(float4* dest, const float4* src, const float* sigma, float4* scratch, int width, int height,
                   int row_begin, int row_end, const float* max_sigma, cudaStream_t stream, int halo_rows = -1);

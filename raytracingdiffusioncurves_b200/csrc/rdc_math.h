@@ -285,6 +285,49 @@ RDC_HD float rdc_slab(float ox, float oy, float idx, float idy, float xmin, floa
 // rdc_slab so that a chord that would win is never culled.
 #define RDC_CULL_SLACK 1.000002f
 
+// ------------------------------------------------------------------------------------------------
+// Point vs chord (rdc_scene_pick). s = the fraction along the chord of the point nearest to p, c = a + s e that
+// point, d2 = |p - c|^2. No rdc_fma: one rounding per C operator, so a float32 numpy restatement gives the same bits.
+// ------------------------------------------------------------------------------------------------
+RDC_HD void rdc_point_chord(float px, float py, float ax, float ay, float bx, float by, float* s, float* cx, float* cy,
+                            float* d2) {
+  const float ex = bx - ax, ey = by - ay;
+  const float wx = px - ax, wy = py - ay;
+  const float ee = ex * ex + ey * ey;
+  float sv = ee > 0.0f ? (wx * ex + wy * ey) / ee : 0.0f;
+  sv = fminf(fmaxf(sv, 0.0f), 1.0f);
+  const float x = ax + sv * ex, y = ay + sv * ey;
+  const float dx = px - x, dy = py - y;
+  *s = sv; *cx = x; *cy = y;
+  *d2 = dx * dx + dy * dy;
+}
+
+// Squared distance from p to a box, in the same operations as d2 above: for any point c inside the box, |b.x - px| <=
+// |cx - px| per axis, and rounding is monotone, so this never exceeds rdc_point_chord's d2 of c (pick.cu).
+RDC_HD float rdc_point_box_d2(float px, float py, float xmin, float ymin, float xmax, float ymax) {
+  const float dx = fmaxf(fmaxf(xmin - px, px - xmax), 0.0f);
+  const float dy = fmaxf(fmaxf(ymin - py, py - ymax), 0.0f);
+  return dx * dx + dy * dy;
+}
+
+// nearest-chord ordering: smaller d2 wins, equal d2 -> smaller chord id (the role rdc_hit_closer plays for rays: any
+// visit order gives the brute force's answer)
+RDC_HD bool rdc_pick_closer(float d2, uint32_t id, float best_d2, uint32_t best_id) {
+  return d2 < best_d2 || (d2 == best_d2 && id < best_id);
+}
+
+// Centre of pixel (ix, iy) in scene coordinates: the render kernel's ray origin before the jitter (render.cu origin_x /
+// origin_y, DeviceCode.cu:103-107: unsigned arithmetic, then a signed cast) plus half a pixel. Anti-aliasing jitters
+// that origin by (0,1] x zoom per axis, so this is the centre of the square the pixel's rays start from, for negative
+// zoom too.
+RDC_HD float rdc_pixel_centre_x(uint32_t width, float zoom, float off_x, uint32_t ix) {
+  return ((float)(int)(ix - (width / 2)) * zoom + off_x) + 0.5f * zoom;
+}
+RDC_HD float rdc_pixel_centre_y(uint32_t height, float zoom, float off_y, bool orzan, uint32_t iy) {
+  const float base = orzan ? (float)(int)((height - iy) - (height / 2)) * zoom + off_y : (float)(int)(iy - (height / 2)) * zoom + off_y;
+  return base + 0.5f * zoom;
+}
+
 // w = wm * t^-e  (DeviceCode.cu:330). Host and oracle use libm powf; the device build uses CUDA powf or a
 // reciprocal square root when e == 0.5 (the default exponent, optixHello.cpp:94). Weights only scale
 // colours, never decide a hit, so this is inside the 1e-4 RGB tolerance and outside the bit-exact set.
