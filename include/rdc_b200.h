@@ -228,6 +228,37 @@ int rdc_render(rdc_scene* scene, const rdc_frame_params* params, float* image, f
 int rdc_render_to_frames(rdc_scene* scene, const rdc_frame_params* params, uint32_t n_targets, float* const* images,
                          float* const* blur_maps, rdc_stream stream);
 
+/* ---- colour stops from an image: the transpose of rdc_render in the colour stops ----
+ *
+ * For fixed frame parameters the image rdc_render writes is linear in the colour values: a pixel is
+ * sum_i w_i c_i / sum_i w_i over its rays, with c_i = col[ind] (1 - rho) + col[ind + 1] rho, and ind, rho and the weights
+ * w_i follow from the geometry and the *_u, weight and weight_degree lists alone. So image = A x, with x the color_left and
+ * color_right values, and fitting colours to a target picture is linear least squares (INTEGRATION.md §4).
+ *   Transpose: grad_color_left and grad_color_right receive A^T image_grad, where A is the map from the colour values to the
+ *     image rdc_render writes for `params`, over the rows of `params`' band: sum over pixels of <image_grad, A x> equals
+ *     <x, grad> up to the fp32 rounding of the render. The rays are the render's (tile grid, Philox draws, culling, closest
+ *     hits, terminal shading walks). Pixels the render leaves NaN (no ray hit, or all weights zero) contribute nothing.
+ *   Layout: image_grad is a device float4[rows * W], band-local like rdc_render's image, dL/dRGB per pixel (.w ignored).
+ *     The outputs are device double arrays laid out like rdc_scene_arrays::color_left / color_right of the handle's current
+ *     stops: 3 * (max(n_color_left, n_color_right) + 2) entries each, padding and sentinels included.
+ *   Overwrite: the call zeroes both arrays first, on the stream, then accumulates with atomicAdd(double): the result is
+ *     not bit-reproducible from call to call (the order of the additions varies), only to fp64 rounding.
+ *   Parameters read: the fields rdc_render uses for its rays, traversal included; route, units_per_tile, local_radius,
+ *     hit_ids, stats and max_sigma are ignored. strip_stride > 1 is rejected.
+ *   Portals: a scene with portal curves is rejected unless max_trace_depth == 0 (through a portal the image is a product of
+ *     colour stops, so not linear in them); at depth 0 a hit on a portal curve contributes nothing, as in the render.
+ *   Blur: the transpose is of the unblurred image; the blur map and gaussianBlur are outside it.
+ *   Non-finite gradients: a non-finite image_grad on a pixel the render does not leave NaN propagates into the outputs;
+ *     the caller zeroes such entries. A pixel whose gradient is zero traces no rays.
+ *   Stream order and memory: like rdc_render. The call waits (stream-ordered, no host wait) for the handle's previous
+ *     launch or update, whatever stream that was on, and the handle's next launch waits for it, so an adjoint enqueued after
+ *     rdc_scene_update_stops sees the new u lists on any stream. It allocates nothing after rdc_scene_reserve for the same
+ *     rays per pixel; without it the first call at a new rays-per-pixel count may synchronise once.
+ *   Validation: RDC_E_INVALID with a message for a null scene, params, image_grad or output array, for what rdc_render
+ *     rejects in the parameters, for strips, and for the portal case above. */
+int rdc_render_color_adjoint(rdc_scene* scene, const rdc_frame_params* params, const float* image_grad,
+                             double* grad_color_left, double* grad_color_right, rdc_stream stream);
+
 /* ---- picking: the curve under a point (an editor's click, or every pixel of a view for hover and selection) ----
  *
  * Nearest: the pick of a point p is the chord with the smallest (d2, chord id) among all chords with d2 <= max_distance^2

@@ -114,6 +114,7 @@ PROTOTYPES = {
     "rdc_render": (C.c_int, [C.c_void_p, C.POINTER(FrameParams), C.c_void_p, C.c_void_p, C.c_void_p]),
     "rdc_render_to_frames": (C.c_int, [C.c_void_p, C.POINTER(FrameParams), C.c_uint32, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p),
                                        C.c_void_p]),
+    "rdc_render_color_adjoint": (C.c_int, [C.c_void_p, C.POINTER(FrameParams), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "rdc_scene_pick": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_float, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "rdc_scene_pick_frame": (C.c_int, [C.c_void_p, C.POINTER(FrameParams), C.c_float, C.c_void_p, C.c_void_p, C.c_void_p]),
     "rdc_view_pixel_to_scene": (C.c_int, [C.POINTER(FrameParams), C.c_uint32, C.c_uint32, f32p, f32p]),
@@ -440,6 +441,13 @@ class Scene:
         sigmas = (C.c_void_p * n)(*blur_map_ptrs)
         _check(_lib.rdc_render_to_frames(self._h, C.byref(params), n, images, sigmas, C.c_void_p(stream)), "rdc_render_to_frames")
 
+    def color_adjoint(self, params: FrameParams, grad_ptr: int, left_ptr: int, right_ptr: int, stream: int = 0) -> None:
+        """rdc_render_color_adjoint: A^T grad, the transpose of render in the colour stops. grad_ptr: device float32 [rows, W, 4]
+        (dL/dRGB, band-local like render's image); left_ptr, right_ptr: device float64 [max(n_color_left, n_color_right) + 2, 3],
+        overwritten. Enqueue-only."""
+        _check(_lib.rdc_render_color_adjoint(self._h, C.byref(params), C.c_void_p(grad_ptr), C.c_void_p(left_ptr),
+                                             C.c_void_p(right_ptr), C.c_void_p(stream)), "rdc_render_color_adjoint")
+
     def pick(self, points_ptr: int, n: int, out_ptr: int, stops_ptr: int = 0, max_distance: float = float("inf"),
              use_diffusion_curve_save: int = 1, stream: int = 0) -> None:
         """rdc_scene_pick: the nearest chord to each of n device float2 points, into device records of PICK_DTYPE (and,
@@ -565,6 +573,146 @@ def gaussian_blur_band(dest_ptr: int, src_ptr: int, sigma_ptr: int, scratch_ptr:
     _check(_lib.rdc_gaussian_blur_band(C.c_void_p(dest_ptr), C.c_void_p(src_ptr), C.c_void_p(sigma_ptr), C.c_void_p(scratch_ptr),
                                        width, height, row_begin, row_end, halo_rows, C.c_void_p(max_sigma_ptr),
                                        C.c_void_p(stream)), "rdc_gaussian_blur_band")
+
+
+def _is_torch(a) -> bool:
+    return type(a).__module__.startswith("torch")
+
+
+def _dot(a, b) -> float:
+    return float((a * b).sum())
+
+
+def cgls(apply_a, apply_at, b, x0, iterations: int):
+    """Conjugate gradients on the normal equations (CGLS) for min ||A x - b||, in float64, on numpy arrays or torch tensors.
+    apply_a(p) -> A p has the type and shape of b; apply_at(r) -> A^T r those of x0. Returns (x, residuals): residuals[0] is
+    ||b - A x0|| and residuals[k] the residual after iteration k. Stops early when A^T r or A p vanishes (x is then a
+    least-squares solution, or the step would be undefined), and when a step would raise the residual: in exact arithmetic
+    it never does, so that only happens once rounding (fp32 images) dominates the remaining progress; the step is not
+    taken, so the residuals returned never increase."""
+    if _is_torch(x0):
+        import torch
+
+        x = x0.to(dtype=torch.float64, copy=True)
+    else:
+        x = np.array(x0, np.float64)
+    r = b - apply_a(x)
+    s = apply_at(r)
+    p = s * 1.0
+    gamma = _dot(s, s)
+    residuals = [_dot(r, r) ** 0.5]
+    for _ in range(iterations):
+        if gamma == 0.0:
+            break
+        q = apply_a(p)
+        qq = _dot(q, q)
+        if qq == 0.0:
+            break
+        alpha = gamma / qq
+        r_next = r - alpha * q
+        res_next = _dot(r_next, r_next) ** 0.5
+        if res_next > residuals[-1]:
+            break
+        x = x + alpha * p
+        r = r_next
+        residuals.append(res_next)
+        s = apply_at(r)
+        gamma_next = _dot(s, s)
+        p = s + (gamma_next / gamma) * p
+        gamma = gamma_next
+    return x, residuals
+
+
+def fit_stops(d: dict, target, render, adjoint, iterations: int):
+    """The least-squares colour fit behind fit_colors, over any render / adjoint pair (numpy or torch images).
+    render(left, right) -> image [rows, W, >=3] for float32 colour arrays laid out like d["color_left"] / d["color_right"];
+    adjoint(grad) -> (left, right) float64 arrays of that layout, the transpose of render at the same pixels, for a float32
+    grad [rows, W, 4]. Only the real stops (j < n_color_*) are unknowns: padding entries and sentinels keep d's values and
+    their gradient is dropped. Pixels that are NaN in the target or in the render have zero residual. The image is affine in
+    the unknowns (the fixed entries add a constant), so the fit is CGLS on its linear part: render with zeros in the fixed
+    entries. Returns (fitted copy of d, residual norms as cgls returns them)."""
+    nl, nr = int(d["n_color_left"]), int(d["n_color_right"])
+    base_l = np.asarray(d["color_left"], np.float32)
+    base_r = np.asarray(d["color_right"], np.float32)
+
+    def colours(x, fixed):
+        x = x.cpu().numpy() if _is_torch(x) else np.asarray(x)
+        left = base_l.copy() if fixed else np.zeros_like(base_l)
+        right = base_r.copy() if fixed else np.zeros_like(base_r)
+        left[:nl] = x[:3 * nl].reshape(nl, 3)
+        right[:nr] = x[3 * nl:].reshape(nr, 3)
+        return left, right
+
+    torch_images = _is_torch(target)
+    if torch_images:
+        import torch
+
+        isnan, where = torch.isnan, lambda m, a: torch.where(m, a, torch.zeros_like(a))
+        f64 = lambda a: a.to(torch.float64)  # noqa: E731
+    else:
+        isnan, where = np.isnan, lambda m, a: np.where(m, a, 0.0)
+        f64 = lambda a: np.asarray(a, np.float64)  # noqa: E731
+    target3 = f64(target[..., :3])
+    n = 3 * (nl + nr)
+    constant = f64(render(*colours(np.zeros(n), True))[..., :3])  # what the fixed entries alone give
+    keep = ~(isnan(constant).any(-1) | isnan(target3).any(-1))[..., None]
+    b = where(keep, target3 - constant)
+
+    def apply_a(p):
+        return where(keep, f64(render(*colours(p, False))[..., :3]))
+
+    def apply_at(r):
+        if torch_images:
+            g = torch.zeros(r.shape[:-1] + (4,), dtype=torch.float32, device=r.device)
+        else:
+            g = np.zeros(r.shape[:-1] + (4,), np.float32)
+        g[..., :3] = r
+        gl, gr = adjoint(g)
+        return np.concatenate([np.asarray(gl, np.float64)[:nl].ravel(), np.asarray(gr, np.float64)[:nr].ravel()])
+
+    x0 = np.concatenate([base_l[:nl].ravel(), base_r[:nr].ravel()]).astype(np.float64)
+    x, residuals = cgls(apply_a, apply_at, b, x0, iterations)
+    fitted = {k: (v.copy() if isinstance(v, np.ndarray) else v) for k, v in d.items()}
+    fitted["color_left"], fitted["color_right"] = colours(x, True)
+    return fitted, residuals
+
+
+def fit_colors(scene: "Scene", d: dict, params: FrameParams, target, iterations: int = 40, stream: int | None = None):
+    """Colour stops whose render of `params` comes closest to `target` in least squares, for the curves, u lists, weights
+    and exponents of `d` (HostScene.to_numpy() layout, the scene `scene` was built from). target: float32 [rows, W, 3|4],
+    numpy or torch, the band of `params`; NaN pixels are ignored. A p is Scene.update_stops + Scene.render, A^T r is
+    Scene.color_adjoint (fit_stops). During the fit the handle holds the search directions (zeros in the fixed entries);
+    on return it holds the fitted stops. Returns (fitted copy of d, residual norm of every iteration). `stream` must be
+    torch's current stream (the default): the residuals are formed there."""
+    import torch
+
+    if stream is None:
+        stream = torch.cuda.current_stream().cuda_stream
+
+    rows, w = params.row_end - params.row_begin, params.image_width
+    dev = torch.device("cuda", torch.cuda.current_device())
+    image = torch.empty((rows, w, 4), dtype=torch.float32, device=dev)
+    sigma = torch.empty((rows, w), dtype=torch.float32, device=dev)
+    grad_left = torch.empty(np.asarray(d["color_left"]).shape, dtype=torch.float64, device=dev)
+    grad_right = torch.empty(np.asarray(d["color_right"]).shape, dtype=torch.float64, device=dev)
+    work = dict(d)
+    scene.reserve(params, False, stream)
+
+    def render(left, right):
+        work["color_left"], work["color_right"] = left, right
+        scene.update_stops(arrays_from_numpy(work), stream)
+        scene.render(params, image.data_ptr(), sigma.data_ptr(), stream)
+        return image
+
+    def adjoint(g):
+        g = g.contiguous()
+        scene.color_adjoint(params, g.data_ptr(), grad_left.data_ptr(), grad_right.data_ptr(), stream)
+        return grad_left.cpu().numpy(), grad_right.cpu().numpy()
+
+    target = torch.as_tensor(target, dtype=torch.float32, device=dev)
+    fitted, residuals = fit_stops(d, target, render, adjoint, iterations)
+    scene.update_stops(arrays_from_numpy(fitted), stream)
+    return fitted, residuals
 
 
 def view_pixel_to_scene(params: FrameParams, ix: int, iy: int) -> tuple[float, float]:

@@ -764,6 +764,7 @@ int build_scene(const rdc_scene_arrays& a, const rdc_accel_options& o, cudaStrea
     if (e != cudaSuccess) up.status = cuda_fail(e, "stop lists");
   }
   point_stops(d, s->stops, stop_at);
+  s->colour_stops = (uint32_t)stop_at.len[0];
   d.n_segments = a.n_segments;
   d.n_curves = a.n_curves;
   d.seg_walk = up.alloc<SegWalk>(a.n_segments);
@@ -1060,6 +1061,7 @@ int update_stops(rdc_scene* s, const rdc_scene_arrays& a, cudaStream_t stream) {
   RDC_CUDA(cudaMemcpyAsync(s->stops, s->staging, L.bytes, cudaMemcpyHostToDevice, stream));
   RDC_CUDA(cudaEventRecord(s->staged, stream));
   point_stops(s->dev, s->stops, L);
+  s->colour_stops = (uint32_t)L.len[0];
   if (int rc = launch_stop_tables(s, stream)) return rc;
   RDC_CUDA(cudaEventRecord(s->launched, stream));
   s->launched_on = stream;

@@ -352,6 +352,18 @@ int rdc_render_to_frames(rdc_scene* scene, const rdc_frame_params* params, uint3
   });
 }
 
+int rdc_render_color_adjoint(rdc_scene* scene, const rdc_frame_params* params, const float* image_grad,
+                             double* grad_color_left, double* grad_color_right, rdc_stream stream) {
+  if (!params) {
+    rdc::set_error("color adjoint: null params");
+    return RDC_E_INVALID;
+  }
+  return guarded(RDC_E_INVALID, [&]() {
+    return rdc::color_adjoint(scene, *params, reinterpret_cast<const float4*>(image_grad), grad_color_left, grad_color_right,
+                              (cudaStream_t)stream);
+  });
+}
+
 int rdc_scene_pick(rdc_scene* scene, const float* points, uint32_t n, float max_distance, int use_diffusion_curve_save,
                    rdc_pick* out, float* stops, rdc_stream stream) {
   return guarded(RDC_E_INVALID, [&]() {

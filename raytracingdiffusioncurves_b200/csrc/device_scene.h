@@ -101,6 +101,7 @@ struct rdc_scene {
   void* staging = nullptr;
   size_t staging_capacity = 0;
   cudaEvent_t staged = nullptr;
+  uint32_t colour_stops = 0;  // stops per colour family in the block: max(n_color_left, n_color_right) + 2
   // per-N table of the iterated base directions (DeviceCode.cu:110-112,167-171)
   float2* base_dirs = nullptr;
   float base_dirs_n = -1.0f;
@@ -143,6 +144,8 @@ int render(rdc_scene* s, const rdc_frame_params& p, float4* image, float* blur_m
            float* const* target_images = nullptr, float* const* target_blur_maps = nullptr);
 int reserve(rdc_scene* s, const rdc_frame_params& p, cudaStream_t stream);
 int launch_plan(const rdc_scene* s, const rdc_frame_params& p, rdc_launch_plan* out);
+int color_adjoint(rdc_scene* s, const rdc_frame_params& p, const float4* image_grad, double* grad_left, double* grad_right,
+                  cudaStream_t stream);
 // pick.cu
 int pick(rdc_scene* s, const float* points, uint32_t n, float max_distance, int orzan, rdc_pick* out, float* stops,
          cudaStream_t stream);

@@ -1710,6 +1710,145 @@ int ensure_capacity(rdc_scene* s, const LaunchPlan& L, cudaStream_t stream) {
   return 0;
 }
 
+// ---- rdc_render_color_adjoint: the transpose of the frame in the colour stops ----
+// For fixed frame parameters a pixel is sum_i w_i c_i / sum_i w_i with c_i = col[ind] (1 - rho) + col[ind+1] rho: ind, rho
+// and w_i follow from the geometry and the u, weight and exponent lists only, so the image is linear in the colour values,
+// and its transpose sends a pixel's gradient g to g w_i / W (1 - rho) at ind and g w_i / W rho at ind + 1 of the family
+// the ray shades. The rays are the render's: its tile grid, Philox draws, pixel culling and closest hit (the tree, which
+// finds the first hits every route finds, or the brute force), and the terminal shading walks of trace_from.
+struct AdjointArgs {
+  RenderArgs r;                // the view (the output and work-unit fields stay unset)
+  const float4* grad;          // [local rows * width] dL/dRGB of each pixel of the band; .w ignored
+  double* left;                // [3 * colour_stops] Aᵀ grad in color_left ...
+  double* right;               // ... and in color_right
+  uint32_t tiles_x, n_tiles;
+  int portals;                 // the scene has portal curves: a hit on one contributes nothing (max_trace_depth 0)
+};
+
+constexpr uint32_t kNoStop = 0xFFFFFFFFu;
+
+// One primary ray of the adjoint: its weight w_i (0 for a miss or a portal hit) and, with COLOUR, the stop it interpolates
+// from, as key = ind << 1 | right, and the ratio rho. Same operands and operations as trace_from's terminal walk path.
+template <bool COLOUR>
+__device__ __forceinline__ float adjoint_ray(const AdjointArgs& aa, const Accel& ac, const Pixel& px, int i, bool small_angle,
+                                             uint32_t& key, float& ratio) {
+  const RenderArgs& a = aa.r;
+  const DevScene& sc = a.sc;
+  Counters cnt;
+  float ox, oy, dx, dy;
+  gen_ray(a, px.pixel, px.base_x, px.base_y, i, small_angle, ox, oy, dx, dy);
+  const Hit h = closest_chord<false, false, false>(ac, a.brute != 0, ox, oy, dx, dy, true, 1u, 0u, __int_as_float(0x7f800000), cnt);
+  key = kNoStop;
+  if (h.leaf < 0) return 0.0f;
+  const uint4 id = __ldg(sc.run_ids + h.leaf);
+  const uint32_t seg = id.y;
+  const uint4* wp = reinterpret_cast<const uint4*>(sc.seg_walk + seg);
+  const uint4 wc = __ldg(wp), ws = __ldg(wp + 1), wd = __ldg(wp + 2);
+  if (aa.portals && __ldg(sc.curve_connect + wd.z) >= 0) return 0.0f;
+  const float u = rdc_hit_u((int)id.z + h.j, (int)id.w, h.s);
+  const uint4 cw = __ldg(sc.chord_walk + 2 * (size_t)h.id), cw2 = __ldg(sc.chord_walk + 2 * (size_t)h.id + 1);
+  const float cu = u + wd.w;
+  const float wm = scalar_stop(sc.weight, cw.w, ws.w, cu);
+  const float e = scalar_stop(sc.weight_degree, cw2.x, wd.y, cu);
+  const float w = wm * rdc_weight_falloff(h.t, e);
+  if (COLOUR) {
+    rdc_f2 v[4];
+    load_control_points(sc, seg, v);
+    const bool right = rdc_is_ray_right(u, dx, dy, v[0], v[1], v[2], v[3], a.orzan != 0);
+    const int ind = right ? rdc_interp_from(cw.y, wc.w, cu, sc.color_right.u, &ratio)
+                          : rdc_interp_from(cw.x, wc.y, cu, sc.color_left.u, &ratio);
+    key = ((uint32_t)ind << 1) | (right ? 1u : 0u);
+  }
+  return w;
+}
+
+// One warp per 8x4 tile of the render's grid, one lane per pixel, all lanes on the same ray index. Pass 1 sums a pixel's
+// weights W in the render's ray order; pass 2 traces the rays again and scatters. Lanes whose rays end on the same stop of
+// the same family (usually most of the tile) add their six terms up first (__match_any_sync, then a butterfly in fp64
+// per group), and the group's first lane issues the six atomicAdd(double).
+__global__ void __launch_bounds__(kBlock) k_color_adjoint(const AdjointArgs aa) {
+  const RenderArgs& a = aa.r;
+  const uint32_t lane = threadIdx.x & 31, tile = blockIdx.x * (kBlock / 32) + (threadIdx.x >> 5);
+  if (tile >= aa.n_tiles) return;  // (whole warps)
+  Accel ac;
+  ac.nodes = a.sc.nodes;
+  ac.runs = reinterpret_cast<const float4*>(a.sc.runs);
+  ac.run_box = a.sc.run_box;
+  ac.n_runs = a.sc.n_runs;
+  ac.slot_box = nullptr;
+  ac.slot_node = nullptr;
+  const bool small_angle = a.two_over_n <= 0.25f && a.two_over_n >= 0.0f;
+  const int n = a.n_iter;
+  const Pixel px = tile_pixel(a, tile, aa.tiles_x, lane);
+  float4 g = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+  if (px.valid) g = __ldg(aa.grad + px.local);
+  // a pixel whose gradient is zero contributes nothing: its rays are not traced
+  bool live = px.valid && (g.x != 0.0f || g.y != 0.0f || g.z != 0.0f);
+  int cull_first = 0, cull_span = n - 1;
+  const float jit = jitter(a);
+  if (!pixel_cull(a, Rect{px.base_x - jit, px.base_x + jit, px.base_y - jit, px.base_y + jit}, cull_first, cull_span)) {
+    cull_first = 0;
+    cull_span = n - 1;
+  }
+  auto reaches = [&](int i) {  // ray i can reach the scene (tree_rays' intervals, visited in the same ascending order)
+    int rel = i - cull_first;
+    if (rel < 0) rel += n;
+    return rel <= cull_span;
+  };
+  uint32_t key = kNoStop;
+  float ratio = 0.0f;
+  // pass 1: W = sum of the weights, in fp32 and in ray order like PixelSums::add
+  float W = 0.0f;
+  if (live) {
+#pragma unroll 1
+    for (int i = 0; i < n; ++i)
+      if (reaches(i)) W += adjoint_ray<false>(aa, ac, px, i, small_angle, key, ratio);
+  }
+  live = live && W != 0.0f;  // W == 0: the render writes NaN, the pixel is outside the image's linear map
+  const double inv_w = live ? 1.0 / (double)W : 0.0;
+  // pass 2
+#pragma unroll 1
+  for (int i = 0; i < n; ++i) {
+    const bool on = live && reaches(i);
+    if (!__any_sync(0xFFFFFFFFu, on)) continue;
+    key = kNoStop;
+    float w = 0.0f;
+    if (on) w = adjoint_ray<true>(aa, ac, px, i, small_angle, key, ratio);
+    const double f = (double)w * inv_w, f1 = f * (double)ratio, f0 = f * (double)(1.0f - ratio);
+    const double gx = g.x, gy = g.y, gz = g.z;
+    const uint32_t peers = __match_any_sync(0xFFFFFFFFu, key);
+    const bool leader = key != kNoStop && lane == (uint32_t)(__ffs(peers) - 1);
+    uint32_t leaders = __ballot_sync(0xFFFFFFFFu, leader);
+    while (leaders) {  // one group (one stop of one family) at a time; all lanes take part in its butterfly
+      const uint32_t l = (uint32_t)(__ffs(leaders) - 1);
+      leaders &= leaders - 1;
+      const uint32_t group = __shfl_sync(0xFFFFFFFFu, peers, l);
+      const bool mine = (group >> lane) & 1u;
+      double v[6] = {mine ? gx * f0 : 0.0, mine ? gy * f0 : 0.0, mine ? gz * f0 : 0.0,
+                     mine ? gx * f1 : 0.0, mine ? gy * f1 : 0.0, mine ? gz * f1 : 0.0};
+#pragma unroll
+      for (int off = 16; off > 0; off >>= 1)
+#pragma unroll
+        for (int c = 0; c < 6; ++c) v[c] += __shfl_xor_sync(0xFFFFFFFFu, v[c], off);
+      if (lane == l) {
+        double* dst = ((key & 1u) ? aa.right : aa.left) + 3 * (size_t)(key >> 1);
+#pragma unroll
+        for (int c = 0; c < 6; ++c) atomicAdd(dst + c, v[c]);
+      }
+    }
+  }
+}
+
+// The table of base directions for the launch's rays per pixel, after ensure_capacity and the wait for the previous launch
+int ensure_base_dirs(rdc_scene* s, const LaunchPlan& L, const rdc_frame_params& p, cudaStream_t stream) {
+  if (s->base_dirs_n != p.number_of_rays_per_pixel) {
+    k_base_dirs<<<1, 32, 0, stream>>>(s->base_dirs, L.n_iter, 2 / p.number_of_rays_per_pixel);
+    RDC_CUDA(cudaGetLastError());
+    s->base_dirs_n = p.number_of_rays_per_pixel;
+  }
+  return 0;
+}
+
 }  // namespace
 
 int reserve(rdc_scene* s, const rdc_frame_params& p, cudaStream_t stream) {
@@ -1781,11 +1920,7 @@ int render(rdc_scene* s, const rdc_frame_params& p, float4* image, float* blur_m
   // One launch at a time per handle (shared work counters, partial sums, base directions): a launch on another
   // stream waits — on the device — for the handle's previous one.
   if (s->launched_any && s->launched_on != stream) RDC_CUDA(cudaStreamWaitEvent(stream, s->launched, 0));
-  if (s->base_dirs_n != p.number_of_rays_per_pixel) {
-    k_base_dirs<<<1, 32, 0, stream>>>(s->base_dirs, L.n_iter, 2 / p.number_of_rays_per_pixel);
-    RDC_CUDA(cudaGetLastError());
-    s->base_dirs_n = p.number_of_rays_per_pixel;
-  }
+  if (int rc = ensure_base_dirs(s, L, p, stream)) return rc;
 
   RenderArgs a{};
   a.sc = s->dev;
@@ -1850,6 +1985,71 @@ int render(rdc_scene* s, const rdc_frame_params& p, float4* image, float* blur_m
   // the work counters rewind themselves when a launch ends; a launch that was cut short must not poison the next
   RDC_CUDA(cudaMemsetAsync(s->work_counters, 0, 2 * sizeof(unsigned int), stream));
   kernel<<<grid, kBlock, L.dyn, stream>>>(a);
+  RDC_CUDA(cudaGetLastError());
+  RDC_CUDA(cudaEventRecord(s->launched, stream));
+  s->launched_on = stream;
+  s->launched_any = true;
+  return 0;
+}
+
+int color_adjoint(rdc_scene* s, const rdc_frame_params& p, const float4* image_grad, double* grad_left, double* grad_right,
+                  cudaStream_t stream) {
+  if (!s || !image_grad || !grad_left || !grad_right) {
+    set_error("color adjoint: null %s", !s ? "scene" : !image_grad ? "image_grad" : "output array");
+    return RDC_E_INVALID;
+  }
+  if (int rc = check_params(p)) return rc;
+  if (p.strip_stride > 1) {
+    set_error("color adjoint: strips (strip_stride %u) are not supported; use a contiguous row band", p.strip_stride);
+    return RDC_E_INVALID;
+  }
+  if (s->info.has_portals && p.max_trace_depth > 0) {
+    set_error("color adjoint: the scene has portals and max_trace_depth is %d; through a portal the image is a product of "
+              "colour stops, not linear in them (use max_trace_depth 0)", p.max_trace_depth);
+    return RDC_E_INVALID;
+  }
+  LaunchPlan L;  // one unit per tile: only the table of base directions is needed
+  L.n_iter = (int)ceilf(p.number_of_rays_per_pixel);
+  if (int rc = ensure_capacity(s, L, stream)) return rc;
+  if (s->launched_any && s->launched_on != stream) RDC_CUDA(cudaStreamWaitEvent(stream, s->launched, 0));
+  const size_t bytes = 3 * (size_t)s->colour_stops * sizeof(double);
+  RDC_CUDA(cudaMemsetAsync(grad_left, 0, bytes, stream));
+  RDC_CUDA(cudaMemsetAsync(grad_right, 0, bytes, stream));
+  if (int rc = ensure_base_dirs(s, L, p, stream)) return rc;
+  AdjointArgs aa{};
+  RenderArgs& a = aa.r;
+  a.sc = s->dev;
+  a.base_dirs = s->base_dirs;
+  a.width = p.image_width;
+  a.height = p.image_height;
+  a.row_begin = p.row_begin;
+  a.row_end = p.row_end;
+  a.strip_stride = 1;
+  a.strip_offset = 0;
+  a.local_rows = p.row_end - p.row_begin;
+  a.row_skew = p.row_begin % kWarpTileH;  // tiles on the full frame's grid, as in the render
+  a.split = 1;
+  a.n_iter = L.n_iter;
+  a.n_rays = p.number_of_rays_per_pixel;
+  a.two_over_n = 2 / p.number_of_rays_per_pixel;
+  a.zoom = p.zoom_factor;
+  a.off_x = p.offset_x;
+  a.off_y = p.offset_y;
+  a.frame = p.frame;
+  a.seed = p.seed;
+  a.orzan = p.use_diffusion_curve_save;
+  a.use_aa = p.use_aa;
+  a.max_depth = p.max_trace_depth;
+  a.brute = p.traversal == RDC_TRAVERSAL_BRUTE_FORCE;
+  a.cull = p.traversal == RDC_TRAVERSAL_LBVH;
+  aa.grad = image_grad;
+  aa.left = grad_left;
+  aa.right = grad_right;
+  aa.tiles_x = (p.image_width + kWarpTileW - 1) / kWarpTileW;
+  aa.n_tiles = aa.tiles_x * ((a.local_rows + a.row_skew + kWarpTileH - 1) / kWarpTileH);
+  aa.portals = s->info.has_portals;
+  const uint32_t warps_per_block = kBlock / 32;
+  k_color_adjoint<<<(aa.n_tiles + warps_per_block - 1) / warps_per_block, kBlock, 0, stream>>>(aa);
   RDC_CUDA(cudaGetLastError());
   RDC_CUDA(cudaEventRecord(s->launched, stream));
   s->launched_on = stream;
