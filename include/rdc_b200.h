@@ -247,7 +247,9 @@ int rdc_render_to_frames(rdc_scene* scene, const rdc_frame_params* params, uint3
  *     hit_ids, stats and max_sigma are ignored. strip_stride > 1 is rejected.
  *   Portals: a scene with portal curves is rejected unless max_trace_depth == 0 (through a portal the image is a product of
  *     colour stops, so not linear in them); at depth 0 a hit on a portal curve contributes nothing, as in the render.
- *   Blur: the transpose is of the unblurred image; the blur map and gaussianBlur are outside it.
+ *   Blur: the transpose is of the unblurred image; the blur map and gaussianBlur are outside it. For the blurred frame
+ *     (rdc_render_frame_to_host with use_blur) apply rdc_gaussian_blur_adjoint first, with the render's blur map: colour
+ *     values never change the blur map, so the blurred frame is B A x and its transpose A^T B^T.
  *   Non-finite gradients: a non-finite image_grad on a pixel the render does not leave NaN propagates into the outputs;
  *     the caller zeroes such entries. A pixel whose gradient is zero traces no rays.
  *   Stream order and memory: like rdc_render. The call waits (stream-ordered, no host wait) for the handle's previous
@@ -372,6 +374,27 @@ int rdc_gaussian_blur(void* dest, const void* source, const float* sigma, void* 
  * [row_begin - halo_rows, row_end + halo_rows) clipped to the buffer (halo_rows >= ceil(3 * largest sigma)). */
 int rdc_gaussian_blur_band(void* dest, const void* source, const float* sigma, void* scratch, int width, int height,
                            int row_begin, int row_end, int halo_rows, const float* max_sigma, rdc_stream stream);
+/* The transpose of the blur, for fitting through it (INTEGRATION.md §4): for a fixed sigma map the blur is linear in the
+ * image, dest = B source, and this call computes B^T.
+ *   Transpose: grad_source (float4, all `height` rows, written in full) receives B^T grad_dest, where B is the map from
+ *     `source` to rows [row_begin,row_end) of rdc_gaussian_blur's `dest` with the same sigma, sizes, band and max_sigma:
+ *     sum <B s, g> = sum <s, B^T g> up to fp32 rounding, all four channels. Rows of grad_dest outside the band are never
+ *     read. Rows of grad_source farther than the blur's reach from the band are 0. rdc_gaussian_blur_band computes the same
+ *     B on the band, so it has the same transpose.
+ *   Pixels without taps: a pixel whose sigma is NaN or <= -1/3 has no taps and a NaN forward output; it contributes nothing
+ *     here, in either pass (its gradient is dropped, and nothing is gathered through it).
+ *   Reach: the largest ceil(3 sigma) over all `height` rows of `sigma` (which rdc_gaussian_blur's horizontal pass reads), at
+ *     most 16384, reduced on the device; the host never waits for it. Each output pixel gathers over that many rows and
+ *     columns either side of it, so the cost follows the largest sigma of the buffer.
+ *   max_sigma: optional, as in the forward. When it points to 0 the call is the identity on the band rows and 0 elsewhere.
+ *   In place: grad_source == grad_dest is allowed.
+ *   Scratch: float4[width * height + 1], i.e. 16 * (width * height + 1) bytes, 16-byte aligned; its contents on entry do not
+ *     matter. The call allocates nothing and only enqueues on `stream`.
+ *   Deterministic: every output is a gather in a fixed order, so repeated calls give the same bits.
+ *   Validation: RDC_E_INVALID with a message for what rdc_gaussian_blur rejects (null pointers, width or height <= 0, an
+ *     empty band or one outside [0,height)). */
+int rdc_gaussian_blur_adjoint(void* grad_source, const void* grad_dest, const float* sigma, void* scratch, int width, int height,
+                              int row_begin, int row_end, const float* max_sigma, rdc_stream stream);
 
 /* ---- whole frame through host memory: the body of the reference's frame loop (optixHello.cpp:1176-1244)
  *      minus window system: render -> [blur] -> copy to host -> synchronise ---- */

@@ -139,6 +139,8 @@ PROTOTYPES = {
                                     C.c_void_p, C.c_void_p]),
     "rdc_gaussian_blur_band": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
                                          C.c_int, C.c_void_p, C.c_void_p]),
+    "rdc_gaussian_blur_adjoint": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
+                                            C.c_void_p, C.c_void_p]),
     "rdc_render_frame_to_host": (C.c_int, [C.c_void_p, C.POINTER(FrameParams), C.c_int, C.c_void_p, C.c_void_p]),
     "rdc_render_frame_to_host_async": (C.c_int, [C.c_void_p, C.POINTER(FrameParams), C.c_int, C.c_void_p, C.c_void_p]),
     "rdc_frame_wait": (C.c_int, [C.c_void_p]),
@@ -575,6 +577,15 @@ def gaussian_blur_band(dest_ptr: int, src_ptr: int, sigma_ptr: int, scratch_ptr:
                                        C.c_void_p(stream)), "rdc_gaussian_blur_band")
 
 
+def gaussian_blur_adjoint(grad_source_ptr: int, grad_dest_ptr: int, sigma_ptr: int, scratch_ptr: int, width: int, height: int,
+                          row_begin: int = 0, row_end: int | None = None, max_sigma_ptr: int = 0, stream: int = 0) -> None:
+    """rdc_gaussian_blur_adjoint: grad_source (float4, all `height` rows) = the transpose of gaussian_blur with the same sigma,
+    band and max_sigma, applied to grad_dest's band rows. scratch: float4[width * height + 1]."""
+    _check(_lib.rdc_gaussian_blur_adjoint(C.c_void_p(grad_source_ptr), C.c_void_p(grad_dest_ptr), C.c_void_p(sigma_ptr),
+                                          C.c_void_p(scratch_ptr), width, height, row_begin, height if row_end is None else row_end,
+                                          C.c_void_p(max_sigma_ptr), C.c_void_p(stream)), "rdc_gaussian_blur_adjoint")
+
+
 def _is_torch(a) -> bool:
     return type(a).__module__.startswith("torch")
 
@@ -677,17 +688,13 @@ def fit_stops(d: dict, target, render, adjoint, iterations: int):
     return fitted, residuals
 
 
-def fit_colors(scene: "Scene", d: dict, params: FrameParams, target, iterations: int = 40, stream: int | None = None):
-    """Colour stops whose render of `params` comes closest to `target` in least squares, for the curves, u lists, weights
-    and exponents of `d` (HostScene.to_numpy() layout, the scene `scene` was built from). target: float32 [rows, W, 3|4],
-    numpy or torch, the band of `params`; NaN pixels are ignored. A p is Scene.update_stops + Scene.render, A^T r is
-    Scene.color_adjoint (fit_stops). During the fit the handle holds the search directions (zeros in the fixed entries);
-    on return it holds the fitted stops. Returns (fitted copy of d, residual norm of every iteration). `stream` must be
-    torch's current stream (the default): the residuals are formed there."""
+def _color_operator(scene: "Scene", d: dict, params: FrameParams, use_blur: bool, stream: int):
+    """The (render, adjoint) pair fit_colors hands to fit_stops: render(left, right) puts the colour values on the handle
+    (update_stops) and renders the band of `params`, then, with use_blur, blurs it as rdc_render_frame_to_host(use_blur=1)
+    does (the band as a buffer of its own rows, with the render's max_sigma flag); adjoint(grad) is the blur's transpose with
+    the last render's blur map (colour values never change it), then Scene.color_adjoint. Device buffers are reused from
+    call to call; `stream` must be torch's current stream."""
     import torch
-
-    if stream is None:
-        stream = torch.cuda.current_stream().cuda_stream
 
     rows, w = params.row_end - params.row_begin, params.image_width
     dev = torch.device("cuda", torch.cuda.current_device())
@@ -697,19 +704,54 @@ def fit_colors(scene: "Scene", d: dict, params: FrameParams, target, iterations:
     grad_right = torch.empty(np.asarray(d["color_right"]).shape, dtype=torch.float64, device=dev)
     work = dict(d)
     scene.reserve(params, False, stream)
+    if use_blur:
+        blurred = torch.empty_like(image)
+        grad_image = torch.empty_like(image)
+        scratch = torch.empty((rows * w + 1, 4), dtype=torch.float32, device=dev)  # the blur's and its transpose's
+        flag = torch.zeros((1,), dtype=torch.float32, device=dev)
+        blur_params = FrameParams.from_buffer_copy(params)
+        blur_params.max_sigma = flag.data_ptr()
 
     def render(left, right):
         work["color_left"], work["color_right"] = left, right
         scene.update_stops(arrays_from_numpy(work), stream)
-        scene.render(params, image.data_ptr(), sigma.data_ptr(), stream)
-        return image
+        if not use_blur:
+            scene.render(params, image.data_ptr(), sigma.data_ptr(), stream)
+            return image
+        flag.zero_()
+        scene.render(blur_params, image.data_ptr(), sigma.data_ptr(), stream)
+        gaussian_blur(blurred.data_ptr(), image.data_ptr(), sigma.data_ptr(), scratch.data_ptr(), w, rows, 0, rows, flag.data_ptr(),
+                      stream)
+        return blurred
 
     def adjoint(g):
         g = g.contiguous()
+        if use_blur:
+            gaussian_blur_adjoint(grad_image.data_ptr(), g.data_ptr(), sigma.data_ptr(), scratch.data_ptr(), w, rows, 0, rows,
+                                  flag.data_ptr(), stream)
+            g = grad_image
         scene.color_adjoint(params, g.data_ptr(), grad_left.data_ptr(), grad_right.data_ptr(), stream)
         return grad_left.cpu().numpy(), grad_right.cpu().numpy()
 
-    target = torch.as_tensor(target, dtype=torch.float32, device=dev)
+    return render, adjoint
+
+
+def fit_colors(scene: "Scene", d: dict, params: FrameParams, target, iterations: int = 40, stream: int | None = None,
+               use_blur: bool = False):
+    """Colour stops whose render of `params` comes closest to `target` in least squares, for the curves, u lists, weights
+    and exponents of `d` (HostScene.to_numpy() layout, the scene `scene` was built from). target: float32 [rows, W, 3|4],
+    numpy or torch, the band of `params`; NaN pixels are ignored. A p is Scene.update_stops + Scene.render, A^T r is
+    Scene.color_adjoint (fit_stops). use_blur: fit the blurred frame instead, exactly what rdc_render_frame_to_host(params,
+    use_blur=1) writes: A p is followed by gaussian_blur with the render's blur map, and A^T r starts with
+    gaussian_blur_adjoint. During the fit the handle holds the search directions (zeros in the fixed entries); on return it
+    holds the fitted stops. Returns (fitted copy of d, residual norm of every iteration). `stream` must be torch's current
+    stream (the default): the residuals are formed there."""
+    import torch
+
+    if stream is None:
+        stream = torch.cuda.current_stream().cuda_stream
+    render, adjoint = _color_operator(scene, d, params, use_blur, stream)
+    target = torch.as_tensor(target, dtype=torch.float32, device=torch.device("cuda", torch.cuda.current_device()))
     fitted, residuals = fit_stops(d, target, render, adjoint, iterations)
     scene.update_stops(arrays_from_numpy(fitted), stream)
     return fitted, residuals

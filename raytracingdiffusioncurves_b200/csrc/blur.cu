@@ -40,6 +40,9 @@ __device__ __forceinline__ Taps taps_for(float sigma) {
   return t;
 }
 
+// weight of tap k; the forward passes and the transpose share it, so the transpose's tap sums have the forward's bits
+__device__ __forceinline__ float tap_weight(int k, const Taps& t) { return expf(-(k * k) / t.sig_square); }
+
 __device__ __forceinline__ bool all_sigma_zero(const float* max_sigma) {
   return max_sigma != nullptr && __ldg(max_sigma) == 0.0f;
 }
@@ -65,7 +68,7 @@ __global__ void k_blur_horizontal(const float4* __restrict__ source, float4* scr
     float4 d = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
     for (int k = t.first; k <= t.last; ++k) {
       const int sx = max(0, min(x + k, width - 1));
-      const float g = expf(-(k * k) / t.sig_square);
+      const float g = tap_weight(k, t);
       const float4 s = source[row + sx];
       accum += g;
       d.x += s.x * g;
@@ -93,7 +96,7 @@ __global__ void k_blur_vertical(const float4* __restrict__ scratch, float4* __re
     float4 d = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
     for (int k = t.first; k <= t.last; ++k) {
       const int sy = max(0, min(y + k, height - 1));
-      const float g = expf(-(k * k) / t.sig_square);
+      const float g = tap_weight(k, t);
       const float4 s = scratch[(size_t)sy * width + x];
       accum += g;
       d.x += s.x * g;
@@ -102,6 +105,140 @@ __global__ void k_blur_vertical(const float4* __restrict__ scratch, float4* __re
       d.w += s.w * g;
     }
     dest[i] = make_float4(d.x / accum, d.y / accum, d.z / accum, d.w / accum);
+  }
+}
+
+// ---- the transpose of the two passes (gaussian_blur_adjoint) ----
+//
+// Forward, per pixel p with taps [f, l] and a = sum_k g(k) (tap order):
+//   T(x,y) = sum_k g(k) S(clampx(x+k), y) / a,   D(x,y) = sum_k g(k) T(x, clampy(y+k)) / a,   g and a of the pixel written.
+// Transpose, gradient G on the band:  G^ = G / a on the band;  vertical: G_T(x,y') = sum_y G^(x,y) sum_{k: clampy(y+k)=y'} g(k);
+// G_T / a(x,y');  horizontal: G_S(x',y') = sum_x (G_T/a)(x,y') sum_{k: clampx(x+k)=x'} g(k). Each sum is a gather (one thread
+// per output pixel, no atomics, so repeats give the same bits) over the sources within the reach R = max(-f, l) of any
+// pixel. Clamp-to-edge: output row / column 0 collects the taps at or below it, the last one the taps at or above it (a
+// buffer one pixel wide collects all of them). A pixel without taps (NaN sigma, sigma <= -1/3) has a NaN forward output:
+// it contributes nothing here.
+
+// sum of the weights of taps [lo, hi], in tap order (the forward's accum when [lo, hi] = [first, last])
+__device__ __forceinline__ float tap_sum(const Taps& t, int lo, int hi) {
+  float s = 0.0f;
+  for (int k = lo; k <= hi; ++k) s += tap_weight(k, t);
+  return s;
+}
+
+// weight with which a pass at source position `from` (taps t) reads position `to` of a line of n: the taps k with
+// clamp(from + k, 0, n - 1) == to
+__device__ __forceinline__ float clamped_weight(const Taps& t, int from, int to, int n) {
+  const int lo = to == 0 ? t.first : max(t.first, to - from);
+  const int hi = to == n - 1 ? t.last : min(t.last, to - from);
+  return lo <= hi ? tap_sum(t, lo, hi) : 0.0f;
+}
+
+// *reach = max(-first, last) over the buffer's pixels that have taps (the caller zeroes it); taps_for caps it at kMaxTaps
+__global__ void k_blur_reach(const float* __restrict__ sigma, size_t count, const float* max_sigma, int* reach) {
+  if (all_sigma_zero(max_sigma)) return;
+  const size_t stride = (size_t)blockDim.x * gridDim.x;
+  int r = 0;
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += stride) {
+    const Taps t = taps_for(sigma[i]);
+    if (t.first <= t.last) r = max(r, max(-t.first, t.last));
+  }
+  r = __reduce_max_sync(0xffffffffu, r);
+  if ((threadIdx.x & 31) == 0 && r > 0) atomicMax(reach, r);
+}
+
+// band rows: grad_source = grad_dest / a, 0 where the pixel has no taps (in place when the two are the same buffer). With
+// an all-zero sigma map the blur is the identity on the band: a copy.
+__global__ void k_blur_adjoint_scale(const float4* grad_dest, float4* grad_source, const float* __restrict__ sigma, int width,
+                                     int row_begin, int row_end, const float* max_sigma) {
+  const size_t count = (size_t)width * (row_end - row_begin), first = (size_t)row_begin * width;
+  const size_t stride = (size_t)blockDim.x * gridDim.x;
+  const bool identity = all_sigma_zero(max_sigma);
+  if (identity && grad_dest == grad_source) return;
+  for (size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x; j < count; j += stride) {
+    const size_t i = first + j;
+    const float4 g = grad_dest[i];
+    if (identity) {
+      grad_source[i] = g;
+      continue;
+    }
+    const Taps t = taps_for(sigma[i]);
+    if (t.first > t.last) {
+      grad_source[i] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+      continue;
+    }
+    const float accum = tap_sum(t, t.first, t.last);
+    grad_source[i] = make_float4(g.x / accum, g.y / accum, g.z / accum, g.w / accum);
+  }
+}
+
+// rows [row_begin - R, row_end + R) of the buffer: scratch = (vertical transpose of the scaled band) / a, 0 where the
+// pixel has no taps (the horizontal pass there reads nothing)
+__global__ void k_blur_adjoint_vertical(const float4* __restrict__ scaled, float4* __restrict__ scratch,
+                                        const float* __restrict__ sigma, int width, int height, int row_begin, int row_end,
+                                        const int* __restrict__ reach, const float* max_sigma) {
+  if (all_sigma_zero(max_sigma)) return;
+  const int r = *reach;
+  const int lo_row = max(0, row_begin - r), hi_row = min(height, row_end + r);
+  const size_t count = (size_t)width * (hi_row - lo_row), first = (size_t)lo_row * width;
+  const size_t stride = (size_t)blockDim.x * gridDim.x;
+  for (size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x; j < count; j += stride) {
+    const size_t i = first + j;
+    const int x = (int)(i % width);
+    const int y = (int)(i / width);
+    float4 d = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+    const int y_end = min(row_end - 1, y + r);
+    for (int sy = max(row_begin, y - r); sy <= y_end; ++sy) {
+      const size_t s_i = (size_t)sy * width + x;
+      const float w = clamped_weight(taps_for(sigma[s_i]), sy, y, height);
+      if (w == 0.0f) continue;
+      const float4 s = scaled[s_i];
+      d.x += s.x * w;
+      d.y += s.y * w;
+      d.z += s.z * w;
+      d.w += s.w * w;
+    }
+    const Taps t = taps_for(sigma[i]);
+    if (t.first > t.last) {
+      scratch[i] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+      continue;
+    }
+    const float accum = tap_sum(t, t.first, t.last);
+    scratch[i] = make_float4(d.x / accum, d.y / accum, d.z / accum, d.w / accum);
+  }
+}
+
+// every row: grad_source = horizontal transpose of scratch on rows [row_begin - R, row_end + R), 0 on the other rows.
+// With an all-zero sigma map, 0 outside the band and the band rows as k_blur_adjoint_scale left them.
+__global__ void k_blur_adjoint_horizontal(const float4* __restrict__ scratch, float4* __restrict__ grad_source,
+                                          const float* __restrict__ sigma, int width, int height, int row_begin, int row_end,
+                                          const int* __restrict__ reach, const float* max_sigma) {
+  const bool identity = all_sigma_zero(max_sigma);
+  const int r = identity ? 0 : *reach;
+  const int lo_row = max(0, row_begin - r), hi_row = min(height, row_end + r);
+  const size_t count = (size_t)width * height;
+  const size_t stride = (size_t)blockDim.x * gridDim.x;
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += stride) {
+    const int x = (int)(i % width);
+    const int y = (int)(i / width);
+    if (y < lo_row || y >= hi_row) {
+      grad_source[i] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+      continue;
+    }
+    if (identity) continue;
+    const size_t row = i - x;
+    float4 d = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+    const int x_end = min(width - 1, x + r);
+    for (int sx = max(0, x - r); sx <= x_end; ++sx) {
+      const float w = clamped_weight(taps_for(sigma[row + sx]), sx, x, width);
+      if (w == 0.0f) continue;
+      const float4 s = scratch[row + sx];
+      d.x += s.x * w;
+      d.y += s.y * w;
+      d.z += s.z * w;
+      d.w += s.w * w;
+    }
+    grad_source[i] = d;
   }
 }
 
@@ -136,6 +273,31 @@ int gaussian_blur(float4* dest, const float4* src, const float* sigma, float4* s
   k_blur_horizontal<<<grid_for(n_all), kThreads, 0, stream>>>(src, scratch, dest, sigma, width, h_begin, h_end, max_sigma);
   RDC_CUDA(cudaGetLastError());
   k_blur_vertical<<<grid_for(n_band), kThreads, 0, stream>>>(scratch, dest, sigma, width, height, row_begin, row_end, max_sigma);
+  RDC_CUDA(cudaGetLastError());
+  return 0;
+}
+
+int gaussian_blur_adjoint(float4* grad_source, const float4* grad_dest, const float* sigma, float4* scratch, int width,
+                          int height, int row_begin, int row_end, const float* max_sigma, cudaStream_t stream) {
+  if (!grad_source || !grad_dest || !sigma || !scratch || width <= 0 || height <= 0 || row_begin < 0 || row_end > height ||
+      row_begin >= row_end) {
+    set_error("blur adjoint: bad argument");
+    return RDC_E_INVALID;
+  }
+  const size_t n_all = (size_t)width * height;
+  const size_t n_band = (size_t)width * (row_end - row_begin);
+  int* reach = reinterpret_cast<int*>(scratch + n_all);
+  RDC_CUDA(cudaMemsetAsync(reach, 0, sizeof(int), stream));
+  k_blur_reach<<<grid_for(n_all), kThreads, 0, stream>>>(sigma, n_all, max_sigma, reach);
+  RDC_CUDA(cudaGetLastError());
+  k_blur_adjoint_scale<<<grid_for(n_band), kThreads, 0, stream>>>(grad_dest, grad_source, sigma, width, row_begin, row_end,
+                                                                   max_sigma);
+  RDC_CUDA(cudaGetLastError());
+  k_blur_adjoint_vertical<<<grid_for(n_all), kThreads, 0, stream>>>(grad_source, scratch, sigma, width, height, row_begin,
+                                                                    row_end, reach, max_sigma);
+  RDC_CUDA(cudaGetLastError());
+  k_blur_adjoint_horizontal<<<grid_for(n_all), kThreads, 0, stream>>>(scratch, grad_source, sigma, width, height, row_begin,
+                                                                      row_end, reach, max_sigma);
   RDC_CUDA(cudaGetLastError());
   return 0;
 }

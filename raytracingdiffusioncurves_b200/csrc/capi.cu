@@ -404,6 +404,13 @@ int rdc_gaussian_blur_band(void* dest, const void* source, const float* sigma, v
                             (cudaStream_t)stream, halo_rows);
 }
 
+int rdc_gaussian_blur_adjoint(void* grad_source, const void* grad_dest, const float* sigma, void* scratch, int width, int height,
+                              int row_begin, int row_end, const float* max_sigma, rdc_stream stream) {
+  return rdc::gaussian_blur_adjoint(static_cast<float4*>(grad_source), static_cast<const float4*>(grad_dest), sigma,
+                                    static_cast<float4*>(scratch), width, height, row_begin, row_end, max_sigma,
+                                    (cudaStream_t)stream);
+}
+
 // Reference-named helpers. They return void like the originals; failures are readable through
 // rdc_last_error_string() and, being CUDA errors, through cudaGetLastError().
 void gaussianBlur(void* dest, void* source, float* sigma, int width, int height, rdc_stream stream) {

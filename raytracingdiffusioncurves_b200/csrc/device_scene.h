@@ -153,6 +153,9 @@ int pick_frame(rdc_scene* s, const rdc_frame_params* p, float max_distance, rdc_
 // blur.cu
 int gaussian_blur(float4* dest, const float4* src, const float* sigma, float4* scratch, int width, int height,
                   int row_begin, int row_end, const float* max_sigma, cudaStream_t stream, int halo_rows = -1);
+// scratch: float4[width * height + 1] (the last element holds the reach)
+int gaussian_blur_adjoint(float4* grad_source, const float4* grad_dest, const float* sigma, float4* scratch, int width,
+                          int height, int row_begin, int row_end, const float* max_sigma, cudaStream_t stream);
 int set_float(float* dest, unsigned n, float v, cudaStream_t stream);
 int blur_preload();
 }  // namespace rdc
