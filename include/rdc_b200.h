@@ -261,6 +261,30 @@ int rdc_render_to_frames(rdc_scene* scene, const rdc_frame_params* params, uint3
 int rdc_render_color_adjoint(rdc_scene* scene, const rdc_frame_params* params, const float* image_grad,
                              double* grad_color_left, double* grad_color_right, rdc_stream stream);
 
+/* ---- blur stops from an image: the transpose of rdc_render's blur map in the blur stops ----
+ *
+ * The blur map rdc_render writes is linear in the blur values the same way: sigma = sum_i w_i b_i / sum_i w_i over a pixel's
+ * rays, with b_i = blur[ind] (1 - rho) + blur[ind + 1] rho, and ind, rho and w_i follow from the geometry and the blur_u,
+ * weight and weight_degree lists alone. So sigma = A_b x, with x the blur values (one channel, one list).
+ *   Transpose: grad_blur receives A_b^T sigma_grad, where A_b is the map from the blur values to the blur map rdc_render
+ *     writes for `params`, over the rows of `params`' band: sum over pixels of sigma_grad * (A_b x) equals <x, grad_blur> up
+ *     to the fp32 rounding of the render. The rays are the render's, as in rdc_render_color_adjoint. Pixels the render leaves
+ *     NaN contribute nothing.
+ *   Layout: sigma_grad is a device float[rows * W], band-local like rdc_render's blur_map, dL/dsigma per pixel. grad_blur is
+ *     a device double array laid out like rdc_scene_arrays::blur of the handle's current stops: n_blur + 2 entries,
+ *     sentinels included.
+ *   Everything else as rdc_render_color_adjoint: zeroed first, then atomicAdd(double), so not bit-reproducible from call to
+ *     call; the same parameter fields read; strips rejected; a scene with portal curves rejected unless
+ *     max_trace_depth == 0 (through a portal the blur map is Bp * blur_T, a product of blur stops); a pixel whose gradient is
+ *     zero traces no rays; stream-ordered through the handle's previous launch or update on any stream; nothing allocated
+ *     after rdc_scene_reserve.
+ *   Chain: the blurred frame depends on the blur values through the sigma map only, so a loss on the blurred frame has the
+ *     gradient A_b^T (dB(sigma) I / dsigma)^T G: rdc_gaussian_blur_sigma_adjoint, then this call (INTEGRATION.md §4).
+ *   Validation: RDC_E_INVALID with a message for a null scene, params, sigma_grad or grad_blur, for what rdc_render rejects
+ *     in the parameters, for strips, and for the portal case above. */
+int rdc_render_blur_adjoint(rdc_scene* scene, const rdc_frame_params* params, const float* sigma_grad, double* grad_blur,
+                            rdc_stream stream);
+
 /* ---- picking: the curve under a point (an editor's click, or every pixel of a view for hover and selection) ----
  *
  * Nearest: the pick of a point p is the chord with the smallest (d2, chord id) among all chords with d2 <= max_distance^2
@@ -395,6 +419,26 @@ int rdc_gaussian_blur_band(void* dest, const void* source, const float* sigma, v
  *     empty band or one outside [0,height)). */
 int rdc_gaussian_blur_adjoint(void* grad_source, const void* grad_dest, const float* sigma, void* scratch, int width, int height,
                               int row_begin, int row_end, const float* max_sigma, rdc_stream stream);
+/* The blur's derivative in its sigma map, for fitting the blur stops (INTEGRATION.md §4). With every pixel's taps
+ * [-ceil(3 sigma), ceil(3 sigma)] held fixed, each pass sum_k g(k) x / sum_k g(k), g(k) = exp(-k^2 / (sigma + 1e-6)^2), is
+ * smooth in the sigma of the pixel it writes: dg/dsigma = g 2 k^2 / (sigma + 1e-6)^3. The blur steps only where ceil(3 sigma)
+ * does, and there the edge tap weighs about e^-9 of the centre tap.
+ *   Derivative: take dest = rdc_gaussian_blur(source, sigma) on rows [row_begin,row_end) with the same sizes and max_sigma.
+ *     grad_sigma[q] = sum over band pixels p of <grad_dest[p], d dest[p] / d sigma[q]>, all four channels: the derivative
+ *     of the smooth piece sigma lies on. grad_sigma (float, all `height` rows) is written in full; rows farther than the
+ *     blur's reach (as in rdc_gaussian_blur_adjoint) from the band are 0. Rows of grad_dest outside the band are never read.
+ *   Terms: sigma[q] moves the vertical pass's output at q (band rows) and the horizontal pass's output at q (rows the band's
+ *     vertical pass reads). A term whose gradient factor is 0 in a channel adds nothing there, even when the image is NaN:
+ *     zero grad_dest where the blurred frame is NaN, and pixels the render leaves NaN never reach grad_sigma.
+ *   Pixels without taps: a pixel whose sigma is NaN or <= -1/3 gets 0 and contributes nothing. With max_sigma pointing to 0
+ *     the result is 0 everywhere.
+ *   Scratch: float4[2 * width * height + 1], i.e. 16 * (2 * width * height + 1) bytes, 16-byte aligned; its contents on
+ *     entry do not matter. The call allocates nothing and only enqueues on `stream`.
+ *   Deterministic: gathers in a fixed order, no atomics, so repeated calls give the same bits.
+ *   Validation: RDC_E_INVALID with a message for what rdc_gaussian_blur_adjoint rejects and for a null source. */
+int rdc_gaussian_blur_sigma_adjoint(float* grad_sigma, const void* grad_dest, const void* source, const float* sigma,
+                                    void* scratch, int width, int height, int row_begin, int row_end,
+                                    const float* max_sigma, rdc_stream stream);
 
 /* ---- whole frame through host memory: the body of the reference's frame loop (optixHello.cpp:1176-1244)
  *      minus window system: render -> [blur] -> copy to host -> synchronise ---- */

@@ -115,6 +115,7 @@ PROTOTYPES = {
     "rdc_render_to_frames": (C.c_int, [C.c_void_p, C.POINTER(FrameParams), C.c_uint32, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p),
                                        C.c_void_p]),
     "rdc_render_color_adjoint": (C.c_int, [C.c_void_p, C.POINTER(FrameParams), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "rdc_render_blur_adjoint": (C.c_int, [C.c_void_p, C.POINTER(FrameParams), C.c_void_p, C.c_void_p, C.c_void_p]),
     "rdc_scene_pick": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_float, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "rdc_scene_pick_frame": (C.c_int, [C.c_void_p, C.POINTER(FrameParams), C.c_float, C.c_void_p, C.c_void_p, C.c_void_p]),
     "rdc_view_pixel_to_scene": (C.c_int, [C.POINTER(FrameParams), C.c_uint32, C.c_uint32, f32p, f32p]),
@@ -141,6 +142,8 @@ PROTOTYPES = {
                                          C.c_int, C.c_void_p, C.c_void_p]),
     "rdc_gaussian_blur_adjoint": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
                                             C.c_void_p, C.c_void_p]),
+    "rdc_gaussian_blur_sigma_adjoint": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
+                                                  C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "rdc_render_frame_to_host": (C.c_int, [C.c_void_p, C.POINTER(FrameParams), C.c_int, C.c_void_p, C.c_void_p]),
     "rdc_render_frame_to_host_async": (C.c_int, [C.c_void_p, C.POINTER(FrameParams), C.c_int, C.c_void_p, C.c_void_p]),
     "rdc_frame_wait": (C.c_int, [C.c_void_p]),
@@ -450,6 +453,12 @@ class Scene:
         _check(_lib.rdc_render_color_adjoint(self._h, C.byref(params), C.c_void_p(grad_ptr), C.c_void_p(left_ptr),
                                              C.c_void_p(right_ptr), C.c_void_p(stream)), "rdc_render_color_adjoint")
 
+    def blur_adjoint(self, params: FrameParams, grad_ptr: int, out_ptr: int, stream: int = 0) -> None:
+        """rdc_render_blur_adjoint: A_b^T grad, the transpose of render's blur map in the blur stops. grad_ptr: device float32
+        [rows, W] (band-local); out_ptr: device float64 laid out like the handle's blur array (n_blur + 2)."""
+        _check(_lib.rdc_render_blur_adjoint(self._h, C.byref(params), C.c_void_p(grad_ptr), C.c_void_p(out_ptr),
+                                            C.c_void_p(stream)), "rdc_render_blur_adjoint")
+
     def pick(self, points_ptr: int, n: int, out_ptr: int, stops_ptr: int = 0, max_distance: float = float("inf"),
              use_diffusion_curve_save: int = 1, stream: int = 0) -> None:
         """rdc_scene_pick: the nearest chord to each of n device float2 points, into device records of PICK_DTYPE (and,
@@ -584,6 +593,17 @@ def gaussian_blur_adjoint(grad_source_ptr: int, grad_dest_ptr: int, sigma_ptr: i
     _check(_lib.rdc_gaussian_blur_adjoint(C.c_void_p(grad_source_ptr), C.c_void_p(grad_dest_ptr), C.c_void_p(sigma_ptr),
                                           C.c_void_p(scratch_ptr), width, height, row_begin, height if row_end is None else row_end,
                                           C.c_void_p(max_sigma_ptr), C.c_void_p(stream)), "rdc_gaussian_blur_adjoint")
+
+
+def gaussian_blur_sigma_adjoint(grad_sigma_ptr: int, grad_dest_ptr: int, src_ptr: int, sigma_ptr: int, scratch_ptr: int,
+                                width: int, height: int, row_begin: int = 0, row_end: int | None = None, max_sigma_ptr: int = 0,
+                                stream: int = 0) -> None:
+    """rdc_gaussian_blur_sigma_adjoint: grad_sigma (float, all `height` rows) = the derivative of <grad_dest, gaussian_blur(src,
+    sigma)> on the band in each pixel's sigma, taps held fixed. scratch: float4[2 * width * height + 1]."""
+    _check(_lib.rdc_gaussian_blur_sigma_adjoint(C.c_void_p(grad_sigma_ptr), C.c_void_p(grad_dest_ptr), C.c_void_p(src_ptr),
+                                                C.c_void_p(sigma_ptr), C.c_void_p(scratch_ptr), width, height, row_begin,
+                                                height if row_end is None else row_end, C.c_void_p(max_sigma_ptr),
+                                                C.c_void_p(stream)), "rdc_gaussian_blur_sigma_adjoint")
 
 
 def _is_torch(a) -> bool:
@@ -755,6 +775,113 @@ def fit_colors(scene: "Scene", d: dict, params: FrameParams, target, iterations:
     fitted, residuals = fit_stops(d, target, render, adjoint, iterations)
     scene.update_stops(arrays_from_numpy(fitted), stream)
     return fitted, residuals
+
+
+def projected_descent(f_and_grad, x0, lower, iterations: int):
+    """Minimise f over x >= lower by projected gradient descent, in float64 on numpy arrays. f_and_grad(x) -> (f, gradient).
+    Each iteration steps to P(x - alpha g) (P clips to the bound) with alpha the Barzilai-Borwein length s.s / s.y of the
+    last step (the first from the gradient's largest entry), and backtracks along that direction until Armijo's condition
+    f(x + t d) <= f(x) + 1e-4 t g.d holds. A trial whose f is NaN or larger is never taken, so the objective never increases.
+    Stops early when the projected step is zero (x is stationary: a zero gradient returns the start) or 40 halvings find no
+    decrease. Returns (x, objectives): objectives[0] is f at the projected start, objectives[k] f after iteration k."""
+    lower = np.asarray(lower, np.float64)
+    x = np.maximum(np.array(x0, np.float64), lower)
+    f, g = f_and_grad(x)
+    g = np.asarray(g, np.float64)
+    objectives = [float(f)]
+    peak = float(np.abs(g).max()) if g.size else 0.0
+    alpha = 1.0 / peak if peak > 0.0 else 1.0
+    for _ in range(iterations):
+        d = np.maximum(x - alpha * g, lower) - x
+        slope = float(g @ d)
+        if not np.any(d) or not slope < 0.0:
+            break
+        t = 1.0
+        for _ in range(40):
+            x_new = np.maximum(x + t * d, lower)
+            f_new, g_new = f_and_grad(x_new)
+            if f_new <= f + 1e-4 * t * slope:
+                break
+            t *= 0.5
+        else:
+            break
+        g_new = np.asarray(g_new, np.float64)
+        s, y = x_new - x, g_new - g
+        sy = float(s @ y)
+        if sy > 0.0:
+            alpha = min(max(float(s @ s) / sy, 1e-30), 1e30)
+        elif np.any(g_new):  # no curvature along the step: restart from the gradient's scale
+            alpha = 1.0 / float(np.abs(g_new).max())
+        x, f, g = x_new, f_new, g_new
+        objectives.append(float(f))
+    return x, objectives
+
+
+def fit_blur(scene: "Scene", d: dict, params: FrameParams, target, iterations: int = 30, stream: int | None = None):
+    """Blur stops whose blurred render of `params` comes closest to `target`: minimises 1/2 ||blurred frame - target||^2 over
+    the real blur stops (j < n_blur), each >= 0, with the curves, colours, u lists, weights and exponents of `d`
+    (HostScene.to_numpy() layout, the scene `scene` was built from) fixed. The blurred frame is exactly what
+    rdc_render_frame_to_host(params, use_blur=1) writes. target: float32 [rows, W, 3|4], numpy or torch, the band of
+    `params`; pixels NaN in the target or in the blurred frame of the start are ignored. Padding and sentinels keep d's values.
+    One evaluation is update_stops, render (with the max_sigma flag), gaussian_blur of the band as its own buffer, the
+    residual, gaussian_blur_sigma_adjoint and Scene.blur_adjoint; projected_descent drives them.
+    The objective is not convex, and its gradient vanishes as sigma -> 0: the outer taps weigh g'(+-1) = 2 sigma^-3 e^{-1/sigma^2}.
+    A stop that starts at 0 stays there, so start from a nonzero blur (a constant 1 px does). The tap count steps where
+    ceil(3 sigma) does; the line search absorbs those small jumps. Returns (fitted copy of d, objective of every iteration);
+    on return the handle holds the fitted stops. `stream` must be torch's current stream (the default)."""
+    import torch
+
+    if stream is None:
+        stream = torch.cuda.current_stream().cuda_stream
+    rows, w = params.row_end - params.row_begin, params.image_width
+    dev = torch.device("cuda", torch.cuda.current_device())
+    nb = int(d["n_blur"])
+    base = np.asarray(d["blur"], np.float32)
+    image = torch.empty((rows, w, 4), dtype=torch.float32, device=dev)
+    sigma = torch.empty((rows, w), dtype=torch.float32, device=dev)
+    blurred = torch.empty_like(image)
+    grad_image = torch.zeros_like(image)
+    grad_sigma = torch.empty_like(sigma)
+    grad_blur = torch.empty(base.shape, dtype=torch.float64, device=dev)
+    scratch = torch.empty((2 * rows * w + 1, 4), dtype=torch.float32, device=dev)  # the blur's and its derivative's
+    flag = torch.zeros((1,), dtype=torch.float32, device=dev)
+    blur_params = FrameParams.from_buffer_copy(params)
+    blur_params.max_sigma = flag.data_ptr()
+    target3 = torch.as_tensor(target, dtype=torch.float32, device=dev)[..., :3].to(torch.float64)
+    work = dict(d)
+    scene.reserve(params, False, stream)
+
+    def stops(x):
+        b = base.copy()
+        b[:nb] = x
+        return b
+
+    def frame(x):
+        work["blur"] = stops(x)
+        scene.update_stops(arrays_from_numpy(work), stream)
+        flag.zero_()
+        scene.render(blur_params, image.data_ptr(), sigma.data_ptr(), stream)
+        gaussian_blur(blurred.data_ptr(), image.data_ptr(), sigma.data_ptr(), scratch.data_ptr(), w, rows, 0, rows, flag.data_ptr(),
+                      stream)
+        return blurred[..., :3].to(torch.float64)
+
+    x0 = base[:nb].astype(np.float64)
+    keep = ~(torch.isnan(frame(x0)).any(-1) | torch.isnan(target3).any(-1))[..., None]
+
+    def f_and_grad(x):
+        r = torch.where(keep, frame(x) - target3, torch.zeros((), dtype=torch.float64, device=dev))
+        f = 0.5 * float((r * r).sum())
+        grad_image[..., :3] = r
+        gaussian_blur_sigma_adjoint(grad_sigma.data_ptr(), grad_image.data_ptr(), image.data_ptr(), sigma.data_ptr(),
+                                    scratch.data_ptr(), w, rows, 0, rows, flag.data_ptr(), stream)
+        scene.blur_adjoint(params, grad_sigma.data_ptr(), grad_blur.data_ptr(), stream)
+        return f, grad_blur[:nb].cpu().numpy()
+
+    x, objectives = projected_descent(f_and_grad, x0, np.zeros(nb), iterations)
+    fitted = {k: (v.copy() if isinstance(v, np.ndarray) else v) for k, v in d.items()}
+    fitted["blur"] = stops(x)
+    scene.update_stops(arrays_from_numpy(fitted), stream)
+    return fitted, objectives
 
 
 def view_pixel_to_scene(params: FrameParams, ix: int, iy: int) -> tuple[float, float]:

@@ -242,6 +242,75 @@ __global__ void k_blur_adjoint_horizontal(const float4* __restrict__ scratch, fl
   }
 }
 
+// ---- the derivative in sigma (gaussian_blur_sigma_adjoint) ----
+//
+// With the taps [f, l] of a pixel held fixed, a pass Y(p) = sum_k g(k) X(clamp(p+k)) / a is smooth in the sigma of the pixel
+// it writes: g(k) = exp(-k^2 / s^2), s = sigma + 1e-6, dg/dsigma = g'(k) = g(k) 2 k^2 / s^3, and
+//   dY(p)/dsigma(p) = sum_k g'(k) (X(clamp(p+k)) - Y(p)) / a.
+// dest = V(H(S)) and each pass reads the sigma of the pixel it writes, so for a gradient G on the band
+//   grad_sigma(q) = <G(q) / a(q),   sum_k g'(k) (T(x, clampy(y+k)) - D(q))>   (vertical pass, band rows)
+//                 + <G_T(q) / a(q), sum_k g'(k) (S(clampx(x+k), y) - T(q))>   (horizontal pass, rows band +- R)
+// with G / a what k_blur_adjoint_scale writes and G_T / a what k_blur_adjoint_vertical writes. Y is recomputed at the pixel
+// with the forward's operations, so it has the forward's bits, and the difference X - Y is formed before the sum.
+
+// one pass's term at pixel i: <factor, sum_k g'(k) (X(clamp(pos+k)) - Y)>, the line of X given by base + clamp(pos+k) * step
+// for positions [0, n). A channel whose factor is 0 adds nothing, not even a NaN of the image; a pixel without taps gives 0.
+__device__ __forceinline__ float sigma_term(const float4* __restrict__ image, float4 f, float sigma, size_t base, size_t step,
+                                            int pos, int n) {
+  const Taps t = taps_for(sigma);
+  if (t.first > t.last || (f.x == 0.0f && f.y == 0.0f && f.z == 0.0f && f.w == 0.0f)) return 0.0f;
+  float accum = 0.0f;
+  float4 y = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+  for (int k = t.first; k <= t.last; ++k) {
+    const float g = tap_weight(k, t);
+    const float4 s = image[base + (size_t)max(0, min(pos + k, n - 1)) * step];
+    accum += g;
+    y.x += s.x * g;
+    y.y += s.y * g;
+    y.z += s.z * g;
+    y.w += s.w * g;
+  }
+  y = make_float4(y.x / accum, y.y / accum, y.z / accum, y.w / accum);
+  const float c = 2.0f / (t.sig_square * (sigma + kMinSigma));  // 2 / s^3
+  float4 d = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+  for (int k = t.first; k <= t.last; ++k) {
+    if (k == 0) continue;  // g'(0) = 0
+    const float gp = tap_weight(k, t) * (float)(k * k) * c;
+    const float4 s = image[base + (size_t)max(0, min(pos + k, n - 1)) * step];
+    d.x += gp * (s.x - y.x);
+    d.y += gp * (s.y - y.y);
+    d.z += gp * (s.z - y.z);
+    d.w += gp * (s.w - y.w);
+  }
+  return (f.x != 0.0f ? f.x * d.x : 0.0f) + (f.y != 0.0f ? f.y * d.y : 0.0f) + (f.z != 0.0f ? f.z * d.z : 0.0f) +
+         (f.w != 0.0f ? f.w * d.w : 0.0f);
+}
+
+// VERTICAL: every row of grad_sigma is written, the band rows with the vertical term (factor = G / a, image = T), the others
+// with 0. Otherwise rows [row_begin - R, row_end + R) add the horizontal term (factor = G_T / a, image = S). With an all-zero
+// sigma map, 0 everywhere.
+template <bool VERTICAL>
+__global__ void k_blur_sigma_adjoint(const float4* __restrict__ factor, const float4* __restrict__ image,
+                                     float* __restrict__ grad_sigma, const float* __restrict__ sigma, int width, int height,
+                                     int row_begin, int row_end, const int* __restrict__ reach, const float* max_sigma) {
+  const bool zero = all_sigma_zero(max_sigma);
+  if (!VERTICAL && zero) return;
+  const int r = VERTICAL ? 0 : *reach;
+  const int lo_row = VERTICAL ? 0 : max(0, row_begin - r), hi_row = VERTICAL ? height : min(height, row_end + r);
+  const size_t count = (size_t)width * (hi_row - lo_row), first = (size_t)lo_row * width;
+  const size_t stride = (size_t)blockDim.x * gridDim.x;
+  for (size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x; j < count; j += stride) {
+    const size_t i = first + j;
+    const int x = (int)(i % width);
+    const int y = (int)(i / width);
+    if (VERTICAL) {
+      grad_sigma[i] = zero || y < row_begin || y >= row_end ? 0.0f : sigma_term(image, factor[i], sigma[i], x, width, y, height);
+    } else {
+      grad_sigma[i] += sigma_term(image, factor[i], sigma[i], i - x, 1, x, width);
+    }
+  }
+}
+
 inline unsigned grid_for(size_t n) {
   const size_t blocks = (n + kThreads - 1) / kThreads;
   return (unsigned)(blocks < kMaxBlocks ? blocks : kMaxBlocks);
@@ -298,6 +367,41 @@ int gaussian_blur_adjoint(float4* grad_source, const float4* grad_dest, const fl
   RDC_CUDA(cudaGetLastError());
   k_blur_adjoint_horizontal<<<grid_for(n_all), kThreads, 0, stream>>>(scratch, grad_source, sigma, width, height, row_begin,
                                                                       row_end, reach, max_sigma);
+  RDC_CUDA(cudaGetLastError());
+  return 0;
+}
+
+// Scratch: T, then (once the vertical term has read it) G_T / a, in the first W*H float4; G / a of the band in the second;
+// the reach after them.
+int gaussian_blur_sigma_adjoint(float* grad_sigma, const float4* grad_dest, const float4* source, const float* sigma,
+                                float4* scratch, int width, int height, int row_begin, int row_end, const float* max_sigma,
+                                cudaStream_t stream) {
+  if (!grad_sigma || !grad_dest || !source || !sigma || !scratch || width <= 0 || height <= 0 || row_begin < 0 ||
+      row_end > height || row_begin >= row_end) {
+    set_error("blur sigma adjoint: bad argument");
+    return RDC_E_INVALID;
+  }
+  const size_t n_all = (size_t)width * height;
+  const size_t n_band = (size_t)width * (row_end - row_begin);
+  float4* pass = scratch;
+  float4* scaled = scratch + n_all;
+  int* reach = reinterpret_cast<int*>(scratch + 2 * n_all);
+  RDC_CUDA(cudaMemsetAsync(reach, 0, sizeof(int), stream));
+  k_blur_reach<<<grid_for(n_all), kThreads, 0, stream>>>(sigma, n_all, max_sigma, reach);
+  RDC_CUDA(cudaGetLastError());
+  k_blur_horizontal<<<grid_for(n_all), kThreads, 0, stream>>>(source, pass, pass, sigma, width, 0, height, max_sigma);
+  RDC_CUDA(cudaGetLastError());
+  k_blur_adjoint_scale<<<grid_for(n_band), kThreads, 0, stream>>>(grad_dest, scaled, sigma, width, row_begin, row_end,
+                                                                   max_sigma);
+  RDC_CUDA(cudaGetLastError());
+  k_blur_sigma_adjoint<true><<<grid_for(n_all), kThreads, 0, stream>>>(scaled, pass, grad_sigma, sigma, width, height, row_begin,
+                                                                       row_end, reach, max_sigma);
+  RDC_CUDA(cudaGetLastError());
+  k_blur_adjoint_vertical<<<grid_for(n_all), kThreads, 0, stream>>>(scaled, pass, sigma, width, height, row_begin, row_end,
+                                                                    reach, max_sigma);
+  RDC_CUDA(cudaGetLastError());
+  k_blur_sigma_adjoint<false><<<grid_for(n_all), kThreads, 0, stream>>>(pass, source, grad_sigma, sigma, width, height,
+                                                                        row_begin, row_end, reach, max_sigma);
   RDC_CUDA(cudaGetLastError());
   return 0;
 }

@@ -364,6 +364,17 @@ int rdc_render_color_adjoint(rdc_scene* scene, const rdc_frame_params* params, c
   });
 }
 
+int rdc_render_blur_adjoint(rdc_scene* scene, const rdc_frame_params* params, const float* sigma_grad, double* grad_blur,
+                            rdc_stream stream) {
+  if (!params) {
+    rdc::set_error("render blur adjoint: null params");
+    return RDC_E_INVALID;
+  }
+  return guarded(RDC_E_INVALID, [&]() {
+    return rdc::blur_adjoint(scene, *params, sigma_grad, grad_blur, (cudaStream_t)stream);
+  });
+}
+
 int rdc_scene_pick(rdc_scene* scene, const float* points, uint32_t n, float max_distance, int use_diffusion_curve_save,
                    rdc_pick* out, float* stops, rdc_stream stream) {
   return guarded(RDC_E_INVALID, [&]() {
@@ -409,6 +420,14 @@ int rdc_gaussian_blur_adjoint(void* grad_source, const void* grad_dest, const fl
   return rdc::gaussian_blur_adjoint(static_cast<float4*>(grad_source), static_cast<const float4*>(grad_dest), sigma,
                                     static_cast<float4*>(scratch), width, height, row_begin, row_end, max_sigma,
                                     (cudaStream_t)stream);
+}
+
+int rdc_gaussian_blur_sigma_adjoint(float* grad_sigma, const void* grad_dest, const void* source, const float* sigma,
+                                    void* scratch, int width, int height, int row_begin, int row_end,
+                                    const float* max_sigma, rdc_stream stream) {
+  return rdc::gaussian_blur_sigma_adjoint(grad_sigma, static_cast<const float4*>(grad_dest), static_cast<const float4*>(source),
+                                          sigma, static_cast<float4*>(scratch), width, height, row_begin, row_end, max_sigma,
+                                          (cudaStream_t)stream);
 }
 
 // Reference-named helpers. They return void like the originals; failures are readable through

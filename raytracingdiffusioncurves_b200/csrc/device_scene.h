@@ -102,6 +102,7 @@ struct rdc_scene {
   size_t staging_capacity = 0;
   cudaEvent_t staged = nullptr;
   uint32_t colour_stops = 0;  // stops per colour family in the block: max(n_color_left, n_color_right) + 2
+  uint32_t blur_stops = 0;    // blur stops in the block: n_blur + 2
   // per-N table of the iterated base directions (DeviceCode.cu:110-112,167-171)
   float2* base_dirs = nullptr;
   float base_dirs_n = -1.0f;
@@ -146,6 +147,7 @@ int reserve(rdc_scene* s, const rdc_frame_params& p, cudaStream_t stream);
 int launch_plan(const rdc_scene* s, const rdc_frame_params& p, rdc_launch_plan* out);
 int color_adjoint(rdc_scene* s, const rdc_frame_params& p, const float4* image_grad, double* grad_left, double* grad_right,
                   cudaStream_t stream);
+int blur_adjoint(rdc_scene* s, const rdc_frame_params& p, const float* sigma_grad, double* grad_blur, cudaStream_t stream);
 // pick.cu
 int pick(rdc_scene* s, const float* points, uint32_t n, float max_distance, int orzan, rdc_pick* out, float* stops,
          cudaStream_t stream);
@@ -156,6 +158,10 @@ int gaussian_blur(float4* dest, const float4* src, const float* sigma, float4* s
 // scratch: float4[width * height + 1] (the last element holds the reach)
 int gaussian_blur_adjoint(float4* grad_source, const float4* grad_dest, const float* sigma, float4* scratch, int width,
                           int height, int row_begin, int row_end, const float* max_sigma, cudaStream_t stream);
+// scratch: float4[2 * width * height + 1]
+int gaussian_blur_sigma_adjoint(float* grad_sigma, const float4* grad_dest, const float4* source, const float* sigma,
+                                float4* scratch, int width, int height, int row_begin, int row_end, const float* max_sigma,
+                                cudaStream_t stream);
 int set_float(float* dest, unsigned n, float v, cudaStream_t stream);
 int blur_preload();
 }  // namespace rdc

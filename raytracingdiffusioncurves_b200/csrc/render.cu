@@ -1710,26 +1710,32 @@ int ensure_capacity(rdc_scene* s, const LaunchPlan& L, cudaStream_t stream) {
   return 0;
 }
 
-// ---- rdc_render_color_adjoint: the transpose of the frame in the colour stops ----
+// ---- rdc_render_color_adjoint / rdc_render_blur_adjoint: the transpose of the frame in the colour or the blur stops ----
 // For fixed frame parameters a pixel is sum_i w_i c_i / sum_i w_i with c_i = col[ind] (1 - rho) + col[ind+1] rho: ind, rho
 // and w_i follow from the geometry and the u, weight and exponent lists only, so the image is linear in the colour values,
 // and its transpose sends a pixel's gradient g to g w_i / W (1 - rho) at ind and g w_i / W rho at ind + 1 of the family
-// the ray shades. The rays are the render's: its tile grid, Philox draws, pixel culling and closest hit (the tree, which
+// the ray shades. The blur map is the same kind of map in the blur values (sigma = sum_i w_i b_i / sum_i w_i, one channel,
+// one list). The rays are the render's: its tile grid, Philox draws, pixel culling and closest hit (the tree, which
 // finds the first hits every route finds, or the brute force), and the terminal shading walks of trace_from.
 struct AdjointArgs {
   RenderArgs r;                // the view (the output and work-unit fields stay unset)
-  const float4* grad;          // [local rows * width] dL/dRGB of each pixel of the band; .w ignored
-  double* left;                // [3 * colour_stops] Aᵀ grad in color_left ...
+  const float4* grad;          // colour: [local rows * width] dL/dRGB of each pixel of the band; .w ignored
+  double* left;                // colour: [3 * colour_stops] Aᵀ grad in color_left ...
   double* right;               // ... and in color_right
   uint32_t tiles_x, n_tiles;
   int portals;                 // the scene has portal curves: a hit on one contributes nothing (max_trace_depth 0)
+  const float* sigma_grad;     // blur: [local rows * width] dL/dsigma of each pixel of the band
+  double* blur;                // blur: [blur_stops] A_bᵀ sigma_grad
 };
+
+enum StopFamily : int { kColourStops, kBlurStops };
 
 constexpr uint32_t kNoStop = 0xFFFFFFFFu;
 
-// One primary ray of the adjoint: its weight w_i (0 for a miss or a portal hit) and, with COLOUR, the stop it interpolates
-// from, as key = ind << 1 | right, and the ratio rho. Same operands and operations as trace_from's terminal walk path.
-template <bool COLOUR>
+// One primary ray of the adjoint: its weight w_i (0 for a miss or a portal hit) and, with KEY, the stop of FAMILY it
+// interpolates from (colour: key = ind << 1 | right; blur: key = ind) and the ratio rho. Same operands and operations as
+// trace_from's terminal walk path.
+template <int FAMILY, bool KEY>
 __device__ __forceinline__ float adjoint_ray(const AdjointArgs& aa, const Accel& ac, const Pixel& px, int i, bool small_angle,
                                              uint32_t& key, float& ratio) {
   const RenderArgs& a = aa.r;
@@ -1751,7 +1757,7 @@ __device__ __forceinline__ float adjoint_ray(const AdjointArgs& aa, const Accel&
   const float wm = scalar_stop(sc.weight, cw.w, ws.w, cu);
   const float e = scalar_stop(sc.weight_degree, cw2.x, wd.y, cu);
   const float w = wm * rdc_weight_falloff(h.t, e);
-  if (COLOUR) {
+  if (KEY && FAMILY == kColourStops) {
     rdc_f2 v[4];
     load_control_points(sc, seg, v);
     const bool right = rdc_is_ray_right(u, dx, dy, v[0], v[1], v[2], v[3], a.orzan != 0);
@@ -1759,14 +1765,18 @@ __device__ __forceinline__ float adjoint_ray(const AdjointArgs& aa, const Accel&
                           : rdc_interp_from(cw.x, wc.y, cu, sc.color_left.u, &ratio);
     key = ((uint32_t)ind << 1) | (right ? 1u : 0u);
   }
+  if (KEY && FAMILY == kBlurStops) key = (uint32_t)rdc_interp_from(cw.z, ws.y, cu, sc.blur.u, &ratio);
   return w;
 }
 
 // One warp per 8x4 tile of the render's grid, one lane per pixel, all lanes on the same ray index. Pass 1 sums a pixel's
 // weights W in the render's ray order; pass 2 traces the rays again and scatters. Lanes whose rays end on the same stop of
-// the same family (usually most of the tile) add their six terms up first (__match_any_sync, then a butterfly in fp64
-// per group), and the group's first lane issues the six atomicAdd(double).
-__global__ void __launch_bounds__(kBlock) k_color_adjoint(const AdjointArgs aa) {
+// the same family (usually most of the tile) add their terms up first (__match_any_sync, then a butterfly in fp64 per
+// group), and the group's first lane issues the atomicAdd(double): six per group for the colours, two for the blur.
+template <int FAMILY>
+__global__ void __launch_bounds__(kBlock) k_stop_adjoint(const AdjointArgs aa) {
+  constexpr bool kColour = FAMILY == kColourStops;
+  constexpr int kTerms = kColour ? 6 : 2;
   const RenderArgs& a = aa.r;
   const uint32_t lane = threadIdx.x & 31, tile = blockIdx.x * (kBlock / 32) + (threadIdx.x >> 5);
   if (tile >= aa.n_tiles) return;  // (whole warps)
@@ -1781,7 +1791,10 @@ __global__ void __launch_bounds__(kBlock) k_color_adjoint(const AdjointArgs aa) 
   const int n = a.n_iter;
   const Pixel px = tile_pixel(a, tile, aa.tiles_x, lane);
   float4 g = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
-  if (px.valid) g = __ldg(aa.grad + px.local);
+  if (px.valid) {
+    if (kColour) g = __ldg(aa.grad + px.local);
+    else g.x = __ldg(aa.sigma_grad + px.local);
+  }
   // a pixel whose gradient is zero contributes nothing: its rays are not traced
   bool live = px.valid && (g.x != 0.0f || g.y != 0.0f || g.z != 0.0f);
   int cull_first = 0, cull_span = n - 1;
@@ -1802,7 +1815,7 @@ __global__ void __launch_bounds__(kBlock) k_color_adjoint(const AdjointArgs aa) 
   if (live) {
 #pragma unroll 1
     for (int i = 0; i < n; ++i)
-      if (reaches(i)) W += adjoint_ray<false>(aa, ac, px, i, small_angle, key, ratio);
+      if (reaches(i)) W += adjoint_ray<FAMILY, false>(aa, ac, px, i, small_angle, key, ratio);
   }
   live = live && W != 0.0f;  // W == 0: the render writes NaN, the pixel is outside the image's linear map
   const double inv_w = live ? 1.0 / (double)W : 0.0;
@@ -1813,7 +1826,7 @@ __global__ void __launch_bounds__(kBlock) k_color_adjoint(const AdjointArgs aa) 
     if (!__any_sync(0xFFFFFFFFu, on)) continue;
     key = kNoStop;
     float w = 0.0f;
-    if (on) w = adjoint_ray<true>(aa, ac, px, i, small_angle, key, ratio);
+    if (on) w = adjoint_ray<FAMILY, true>(aa, ac, px, i, small_angle, key, ratio);
     const double f = (double)w * inv_w, f1 = f * (double)ratio, f0 = f * (double)(1.0f - ratio);
     const double gx = g.x, gy = g.y, gz = g.z;
     const uint32_t peers = __match_any_sync(0xFFFFFFFFu, key);
@@ -1824,16 +1837,21 @@ __global__ void __launch_bounds__(kBlock) k_color_adjoint(const AdjointArgs aa) 
       leaders &= leaders - 1;
       const uint32_t group = __shfl_sync(0xFFFFFFFFu, peers, l);
       const bool mine = (group >> lane) & 1u;
-      double v[6] = {mine ? gx * f0 : 0.0, mine ? gy * f0 : 0.0, mine ? gz * f0 : 0.0,
-                     mine ? gx * f1 : 0.0, mine ? gy * f1 : 0.0, mine ? gz * f1 : 0.0};
+      double v[kTerms];
+      if (kColour) {
+        v[0] = mine ? gx * f0 : 0.0, v[1] = mine ? gy * f0 : 0.0, v[2] = mine ? gz * f0 : 0.0;
+        v[3] = mine ? gx * f1 : 0.0, v[4] = mine ? gy * f1 : 0.0, v[5] = mine ? gz * f1 : 0.0;
+      } else {
+        v[0] = mine ? gx * f0 : 0.0, v[1] = mine ? gx * f1 : 0.0;
+      }
 #pragma unroll
       for (int off = 16; off > 0; off >>= 1)
 #pragma unroll
-        for (int c = 0; c < 6; ++c) v[c] += __shfl_xor_sync(0xFFFFFFFFu, v[c], off);
+        for (int c = 0; c < kTerms; ++c) v[c] += __shfl_xor_sync(0xFFFFFFFFu, v[c], off);
       if (lane == l) {
-        double* dst = ((key & 1u) ? aa.right : aa.left) + 3 * (size_t)(key >> 1);
+        double* dst = kColour ? ((key & 1u) ? aa.right : aa.left) + 3 * (size_t)(key >> 1) : aa.blur + key;
 #pragma unroll
-        for (int c = 0; c < 6; ++c) atomicAdd(dst + c, v[c]);
+        for (int c = 0; c < kTerms; ++c) atomicAdd(dst + c, v[c]);
       }
     }
   }
@@ -1992,31 +2010,37 @@ int render(rdc_scene* s, const rdc_frame_params& p, float4* image, float* blur_m
   return 0;
 }
 
-int color_adjoint(rdc_scene* s, const rdc_frame_params& p, const float4* image_grad, double* grad_left, double* grad_right,
-                  cudaStream_t stream) {
-  if (!s || !image_grad || !grad_left || !grad_right) {
-    set_error("color adjoint: null %s", !s ? "scene" : !image_grad ? "image_grad" : "output array");
-    return RDC_E_INVALID;
-  }
+namespace {
+
+// The common part of color_adjoint and blur_adjoint: the checks, the wait for the handle's previous launch, the zeroing of
+// the outputs and the launch of k_stop_adjoint<FAMILY>. `aa` carries the family's gradient and outputs; `what` names the call
+// in messages, `stops` the family.
+template <int FAMILY>
+int stop_adjoint(rdc_scene* s, const rdc_frame_params& p, AdjointArgs aa, const char* what, const char* stops,
+                 cudaStream_t stream) {
   if (int rc = check_params(p)) return rc;
   if (p.strip_stride > 1) {
-    set_error("color adjoint: strips (strip_stride %u) are not supported; use a contiguous row band", p.strip_stride);
+    set_error("%s: strips (strip_stride %u) are not supported; use a contiguous row band", what, p.strip_stride);
     return RDC_E_INVALID;
   }
   if (s->info.has_portals && p.max_trace_depth > 0) {
-    set_error("color adjoint: the scene has portals and max_trace_depth is %d; through a portal the image is a product of "
-              "colour stops, not linear in them (use max_trace_depth 0)", p.max_trace_depth);
+    set_error("%s: the scene has portals and max_trace_depth is %d; through a portal the %s is a product of "
+              "%s stops, not linear in them (use max_trace_depth 0)", what, p.max_trace_depth,
+              FAMILY == kColourStops ? "image" : "blur map", stops);
     return RDC_E_INVALID;
   }
   LaunchPlan L;  // one unit per tile: only the table of base directions is needed
   L.n_iter = (int)ceilf(p.number_of_rays_per_pixel);
   if (int rc = ensure_capacity(s, L, stream)) return rc;
   if (s->launched_any && s->launched_on != stream) RDC_CUDA(cudaStreamWaitEvent(stream, s->launched, 0));
-  const size_t bytes = 3 * (size_t)s->colour_stops * sizeof(double);
-  RDC_CUDA(cudaMemsetAsync(grad_left, 0, bytes, stream));
-  RDC_CUDA(cudaMemsetAsync(grad_right, 0, bytes, stream));
+  if (FAMILY == kColourStops) {
+    const size_t bytes = 3 * (size_t)s->colour_stops * sizeof(double);
+    RDC_CUDA(cudaMemsetAsync(aa.left, 0, bytes, stream));
+    RDC_CUDA(cudaMemsetAsync(aa.right, 0, bytes, stream));
+  } else {
+    RDC_CUDA(cudaMemsetAsync(aa.blur, 0, (size_t)s->blur_stops * sizeof(double), stream));
+  }
   if (int rc = ensure_base_dirs(s, L, p, stream)) return rc;
-  AdjointArgs aa{};
   RenderArgs& a = aa.r;
   a.sc = s->dev;
   a.base_dirs = s->base_dirs;
@@ -2042,19 +2066,42 @@ int color_adjoint(rdc_scene* s, const rdc_frame_params& p, const float4* image_g
   a.max_depth = p.max_trace_depth;
   a.brute = p.traversal == RDC_TRAVERSAL_BRUTE_FORCE;
   a.cull = p.traversal == RDC_TRAVERSAL_LBVH;
-  aa.grad = image_grad;
-  aa.left = grad_left;
-  aa.right = grad_right;
   aa.tiles_x = (p.image_width + kWarpTileW - 1) / kWarpTileW;
   aa.n_tiles = aa.tiles_x * ((a.local_rows + a.row_skew + kWarpTileH - 1) / kWarpTileH);
   aa.portals = s->info.has_portals;
   const uint32_t warps_per_block = kBlock / 32;
-  k_color_adjoint<<<(aa.n_tiles + warps_per_block - 1) / warps_per_block, kBlock, 0, stream>>>(aa);
+  k_stop_adjoint<FAMILY><<<(aa.n_tiles + warps_per_block - 1) / warps_per_block, kBlock, 0, stream>>>(aa);
   RDC_CUDA(cudaGetLastError());
   RDC_CUDA(cudaEventRecord(s->launched, stream));
   s->launched_on = stream;
   s->launched_any = true;
   return 0;
+}
+
+}  // namespace
+
+int color_adjoint(rdc_scene* s, const rdc_frame_params& p, const float4* image_grad, double* grad_left, double* grad_right,
+                  cudaStream_t stream) {
+  if (!s || !image_grad || !grad_left || !grad_right) {
+    set_error("color adjoint: null %s", !s ? "scene" : !image_grad ? "image_grad" : "output array");
+    return RDC_E_INVALID;
+  }
+  AdjointArgs aa{};
+  aa.grad = image_grad;
+  aa.left = grad_left;
+  aa.right = grad_right;
+  return stop_adjoint<kColourStops>(s, p, aa, "color adjoint", "colour", stream);
+}
+
+int blur_adjoint(rdc_scene* s, const rdc_frame_params& p, const float* sigma_grad, double* grad_blur, cudaStream_t stream) {
+  if (!s || !sigma_grad || !grad_blur) {
+    set_error("render blur adjoint: null %s", !s ? "scene" : !sigma_grad ? "sigma_grad" : "output array");
+    return RDC_E_INVALID;
+  }
+  AdjointArgs aa{};
+  aa.sigma_grad = sigma_grad;
+  aa.blur = grad_blur;
+  return stop_adjoint<kBlurStops>(s, p, aa, "render blur adjoint", "blur", stream);
 }
 
 }  // namespace rdc
