@@ -262,7 +262,8 @@ __global__ void k_pad_boxes(const float4* leaf_box, uint32_t n, float pad, float
 __global__ void k_single_leaf_root(const float4* leaf_box, float pad, BvhNode* nodes) {
   const float inf = __int_as_float(0x7f800000);
   nodes[0].lbox = padded(leaf_box[0], pad);
-  nodes[0].rbox = make_float4(inf, inf, -inf, -inf);  // never entered
+  nodes[0].rbox = make_float4(inf, inf, -inf, -inf);  // a placeholder: pick's box distance is +inf; the render's fused slab
+                                                      // test would enter it, so closest_chord tests the one run directly
   nodes[0].left = ~0;
   nodes[0].right = ~0;
   nodes[0].parent = -1;

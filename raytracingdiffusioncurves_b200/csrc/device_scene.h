@@ -116,6 +116,11 @@ struct rdc_scene {
   uint32_t grid_blocks[32] = {};  // SM-filling grid size per k_render variant (render.cu, variant_index) ...
   size_t grid_dyn[32] = {};       // ... at this much dynamic shared memory
   float mean_run_w = 0.0f, mean_run_h = 0.0f;  // mean padded run box (local-table radius estimate)
+  // launches whose ray origins lie far from the scene read copies of the boxes widened by wide_w (render.cu, widened_boxes)
+  BvhNode* wide_nodes = nullptr;
+  float4* wide_run_box = nullptr;
+  float4* wide_cut_box = nullptr;
+  float wide_w = 0.0f;
   // partial sums of k_render's work units (a tile's rays are dealt to several units), grown on demand
   float4* part_rgbw = nullptr;
   float* part_blur = nullptr;

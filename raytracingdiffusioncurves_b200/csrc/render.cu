@@ -174,9 +174,13 @@ __device__ __forceinline__ float slab_rcp(float d) {
 }
 
 // Slab test of a padded box in fused form: t = x * (1/d) - o * (1/d), the second product computed once per ray.
-// Culling only — never decides a hit: against rdc_slab the entry and exit distances move by a few ulp of |o / d|, i.e. the
-// box is displaced by ~1e-7 of the origin's coordinates, which the boxes' padding (curve_width + 4e-6 x scene extent,
-// accel.cu) covers forty times over. 12 operations per box instead of 16: lady_bug.xml 1080p 8.92 -> 8.49 ms, the 21-scene
+// Culling only — never decides a hit. Against exact arithmetic, the fused test, the approximate reciprocal and the chord
+// test's own differences p - o move the box as the ray sees it by a few ulp of the coordinates involved: up to ~6 x 2^-23
+// x max(M, extent), M the largest origin coordinate. So the rounding scales with the ORIGINS, not with the scene: the
+// boxes' padding (curve_width + 4e-6 x extent, accel.cu) alone covers it only while M stays within about twice the
+// extent. A launch whose origins lie farther out reads boxes widened by w (slab_widening, widened_boxes), which makes the
+// padding and w together >= 16 x 2^-23 x max(M, extent), more than twice the displacement, for any view; views near the
+// scene read the scene's own boxes. 12 operations per box instead of 16: lady_bug.xml 1080p 8.92 -> 8.49 ms, the 21-scene
 // 4K sweep 834 -> 805 ms (profiles/r02b/variants.log).
 struct SlabRay {
   float idx, idy, nox, noy;  // 1/dx, 1/dy, -ox/dx, -oy/dy
@@ -356,7 +360,8 @@ __device__ __forceinline__ Hit closest_chord(const Accel& ac, bool brute, float 
   const SlabRay sr = slab_ray(ox, oy, dx, dy);
   int2 stack[kStack];  // (node, entry distance bits)
   int sp = 0;
-  int node = root;
+  // a scene of one run: its root's second child is a placeholder, and the run is tested without a box test at all
+  int node = ac.n_runs == 1 ? ~0 : root;
   // while-while form (Aila & Laine 2009): every lane first walks inner nodes until it stands on a leaf (or has nothing
   // left), then the warp tests leaves together — a lane on a leaf no longer waits out its neighbours' node steps one
   // iteration at a time, and vice versa. Same visits in the same order per lane as the single if/else loop it replaces:
@@ -1535,6 +1540,62 @@ struct LaunchPlan {
   size_t local_pixels = 0;
 };
 
+// Widening of every box for a launch (SlabRay): the largest coordinate any of its ray origins can have is
+// M = max(|offset_x|, |offset_y|) + (max(width, height) / 2 + 2) |zoom| (pixel index, anti-aliasing jitter and rounding);
+// portal continuation rays start on the scene, within its extent. The slab and chord tests move a box by up to
+// ~6 x 2^-23 x max(M, extent); the padding alone exceeds 16 x 2^-23 x extent (4e-6 = 33.5 x 2^-23), so
+// w = max(0, 16 x 2^-23 x M - pad) makes padding + w >= 16 x 2^-23 x max(M, extent).
+float slab_widening(const rdc_scene* s, const rdc_frame_params& p) {
+  const double m = std::fmax(std::fabs((double)p.offset_x), std::fabs((double)p.offset_y)) +
+                   (0.5 * std::max(p.image_width, p.image_height) + 2.0) * std::fabs((double)p.zoom_factor);
+  const double w = 16.0 * std::ldexp(1.0, -23) * m * (1.0 + 1e-6) - (double)s->info.pad;
+  return std::isfinite(w) && w > 0.0 ? (float)w : 0.0f;
+}
+
+__device__ __forceinline__ float4 widen_box(float4 b, float w) { return make_float4(b.x - w, b.y - w, b.z + w, b.w + w); }
+
+// every box the traversal and the tables read, widened by w: node child boxes, run boxes, seed-cut boxes
+__global__ void k_widen_boxes(DevScene src, float w, BvhNode* nodes, float4* run_box, float4* cut_box) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < src.n_nodes) {
+    BvhNode n = src.nodes[i];
+    n.lbox = widen_box(n.lbox, w);
+    n.rbox = widen_box(n.rbox, w);
+    nodes[i] = n;
+  }
+  if (i < src.n_runs) run_box[i] = widen_box(src.run_box[i], w);
+  if (i < src.n_cut) cut_box[i] = widen_box(src.cut_box[i], w);
+}
+
+// The scene as a launch with widening w reads it: the scene itself for w = 0, else the handle's widened copies of its
+// boxes, (re)made on `stream` when w differs from the last launch's (the handle's launches are serialised).
+int widened_boxes(rdc_scene* s, float w, cudaStream_t stream, DevScene* out) {
+  *out = s->dev;
+  if (w == 0.0f) return 0;
+  if (!s->wide_nodes) {
+    RDC_CUDA(cudaMalloc((void**)&s->wide_nodes, (size_t)s->dev.n_nodes * sizeof(BvhNode)));
+    s->allocations.push_back(s->wide_nodes);
+  }
+  if (!s->wide_run_box) {
+    RDC_CUDA(cudaMalloc((void**)&s->wide_run_box, (size_t)s->dev.n_runs * sizeof(float4)));
+    s->allocations.push_back(s->wide_run_box);
+  }
+  if (s->dev.n_cut && !s->wide_cut_box) {
+    RDC_CUDA(cudaMalloc((void**)&s->wide_cut_box, (size_t)s->dev.n_cut * sizeof(float4)));
+    s->allocations.push_back(s->wide_cut_box);
+  }
+  if (s->wide_w != w) {
+    const uint32_t n = std::max(std::max(s->dev.n_nodes, s->dev.n_runs), s->dev.n_cut);
+    k_widen_boxes<<<(n + 255) / 256, 256, 0, stream>>>(s->dev, w, s->wide_nodes, s->wide_run_box, s->wide_cut_box);
+    RDC_CUDA(cudaGetLastError());
+    s->wide_w = w;
+  }
+  out->nodes = s->wide_nodes;
+  out->run_box = s->wide_run_box;
+  if (s->dev.n_cut) out->cut_box = s->wide_cut_box;
+  return 0;
+}
+
 int check_params(const rdc_frame_params& p) {
   if (p.image_width == 0 || p.image_height == 0 || p.row_begin >= p.row_end || p.row_end > p.image_height) {
     set_error("render: bad image size or row band [%u,%u) of %u", p.row_begin, p.row_end, p.image_height);
@@ -1941,7 +2002,7 @@ int render(rdc_scene* s, const rdc_frame_params& p, float4* image, float* blur_m
   if (int rc = ensure_base_dirs(s, L, p, stream)) return rc;
 
   RenderArgs a{};
-  a.sc = s->dev;
+  if (int rc = widened_boxes(s, slab_widening(s, p), stream, &a.sc)) return rc;
   a.image = image;
   a.blur_map = blur_map;
   a.n_targets = n_targets;
@@ -2042,7 +2103,7 @@ int stop_adjoint(rdc_scene* s, const rdc_frame_params& p, AdjointArgs aa, const 
   }
   if (int rc = ensure_base_dirs(s, L, p, stream)) return rc;
   RenderArgs& a = aa.r;
-  a.sc = s->dev;
+  if (int rc = widened_boxes(s, slab_widening(s, p), stream, &a.sc)) return rc;
   a.base_dirs = s->base_dirs;
   a.width = p.image_width;
   a.height = p.image_height;

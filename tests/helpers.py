@@ -118,6 +118,40 @@ class GpuRenderer:
         return out
 
 
+def curve_xml(points, colour=(255, 64, 0)) -> str:
+    """One curve of the CurveSetXML format: control points as given, two colour stops per side, blur 0 -> 2."""
+    pts = "".join(f'<control_point x="{x:.9g}" y="{y:.9g}" />' for x, y in points)
+    r, g, b = colour
+    return (f'<curve nb_control_points="{len(points)}"><control_points_set>{pts}</control_points_set>'
+            f'<left_colors_set><left_color G="{g}" R="{r}" globalID="0" B="{b}" /><left_color G="{b}" R="{g}" globalID="10" B="{r}" />'
+            f'</left_colors_set><right_colors_set><right_color G="{r}" R="{b}" globalID="0" B="{g}" />'
+            f'<right_color G="{g}" R="{r}" globalID="10" B="{b}" /></right_colors_set>'
+            '<blur_points_set><best_scale value="0" globalID="0" /><best_scale value="2" globalID="10" /></blur_points_set></curve>\n')
+
+
+def straight(ax, ay, bx, by):
+    """Control points of a straight segment from a to b (equally spaced, so its chords are one chord)."""
+    return [(ax + (bx - ax) * k / 3.0, ay + (by - ay) * k / 3.0) for k in range(4)]
+
+
+def scene_xml(curves, size=512) -> str:
+    return (f'<!DOCTYPE CurveSetXML>\n<curve_set image_width="{size}" image_height="{size}" nb_curves="{len(curves)}">\n'
+            + "".join(curves) + "</curve_set>\n")
+
+
+def dust_curves(n=3000, seed=7, size=512):
+    """n straight segments of length 0.02-0.5 scattered over a size x size box: every segment is its own run, so most hits
+    land near a corner of its padded box."""
+    rng = np.random.default_rng(seed)
+    out = []
+    for k in range(n):
+        cx, cy = rng.uniform(4, size - 4, 2)
+        half, ang = 0.5 * rng.uniform(0.02, 0.5), rng.uniform(0, np.pi)
+        dx, dy = half * np.cos(ang), half * np.sin(ang)
+        out.append(curve_xml(straight(cx - dx, cy - dy, cx + dx, cy + dy), (k % 256, (7 * k) % 256, (31 * k) % 256)))
+    return out
+
+
 def compare_images(got, want, tol=1e-4):
     """RGB within tol where both finite; NaN pattern identical. Returns (max abs diff, psnr)."""
     g, w = got[..., :3], want[..., :3]
