@@ -285,6 +285,36 @@ int rdc_render_color_adjoint(rdc_scene* scene, const rdc_frame_params* params, c
 int rdc_render_blur_adjoint(rdc_scene* scene, const rdc_frame_params* params, const float* sigma_grad, double* grad_blur,
                             rdc_stream stream);
 
+/* ---- weight and exponent stops from an image: the derivative of rdc_render's image and blur map in those stops ----
+ *
+ * A ray's weight is w_i = m_i t_i^-e_i, with m_i = weight[iw] (1 - rho_w) + weight[iw + 1] rho_w and
+ * e_i = weight_degree[ie] (1 - rho_e) + weight_degree[ie + 1] rho_e; the hits, colours c_i, blur values b_i, iw, ie and the
+ * ratios follow from the geometry and the other lists alone. A pixel is P = sum_i w_i c_i / W and sigma = sum_i w_i b_i / W,
+ * W = sum_i w_i: smooth, not linear, in the weight and exponent values wherever W > 0, and unchanged when every weight is
+ * scaled by the same factor.
+ *   Derivative: a vector-Jacobian product at the handle's current stops. With s_i = <image_grad, c_i> + sigma_grad b_i and
+ *     K = sum_i w_i s_i / W per pixel, dL/dw_i = (s_i - K) / W; grad_weight[iw] receives (1 - rho_w) t_i^-e_i (s_i - K) / W
+ *     and grad_weight_degree[ie] receives -(1 - rho_e) w_i ln(t_i) (s_i - K) / W (rho at iw + 1 and ie + 1), summed over
+ *     the pixels of `params`' band and their rays. Since the frame does not change when all weights are scaled,
+ *     sum_k weight[k] grad_weight[k] = 0 up to rounding. The rays are the render's, as in rdc_render_color_adjoint. Pixels
+ *     the render leaves NaN contribute nothing.
+ *   Layout: image_grad is a device float4[rows * W] as in rdc_render_color_adjoint (.w ignored), sigma_grad a device
+ *     float[rows * W] as in rdc_render_blur_adjoint; either may be NULL, which means zero, but not both. grad_weight and
+ *     grad_weight_degree are device double arrays laid out like rdc_scene_arrays::weight and ::weight_degree of the handle's
+ *     current stops: n_weight + 2 and n_weight_degree + 2 entries, sentinels included.
+ *   Everything else as rdc_render_color_adjoint: both outputs zeroed first, then atomicAdd(double), so not bit-reproducible
+ *     from call to call; the same parameter fields read; strips rejected; a scene with portal curves rejected unless
+ *     max_trace_depth == 0 (through a portal w = 1/(1/w_T + S) mixes the stops of several curves, and the colour is a
+ *     product); a pixel whose four gradient components are zero traces no rays; stream-ordered through the handle's previous
+ *     launch or update on any stream; nothing allocated after rdc_scene_reserve.
+ *   Chain: for a loss on the blurred frame (rdc_render_frame_to_host with use_blur), the weights move both the image and the
+ *     blur map. Apply rdc_gaussian_blur_adjoint (image_grad = B^T G) and rdc_gaussian_blur_sigma_adjoint (sigma_grad) with
+ *     the render's blur map first, then this call with both results (INTEGRATION.md §4).
+ *   Validation: RDC_E_INVALID with a message for a null scene, params or output array, for image_grad and sigma_grad both
+ *     NULL, for what rdc_render rejects in the parameters, for strips, and for the portal case above. */
+int rdc_render_weight_adjoint(rdc_scene* scene, const rdc_frame_params* params, const float* image_grad, const float* sigma_grad,
+                              double* grad_weight, double* grad_weight_degree, rdc_stream stream);
+
 /* ---- picking: the curve under a point (an editor's click, or every pixel of a view for hover and selection) ----
  *
  * Nearest: the pick of a point p is the chord with the smallest (d2, chord id) among all chords with d2 <= max_distance^2

@@ -116,6 +116,8 @@ PROTOTYPES = {
                                        C.c_void_p]),
     "rdc_render_color_adjoint": (C.c_int, [C.c_void_p, C.POINTER(FrameParams), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "rdc_render_blur_adjoint": (C.c_int, [C.c_void_p, C.POINTER(FrameParams), C.c_void_p, C.c_void_p, C.c_void_p]),
+    "rdc_render_weight_adjoint": (C.c_int, [C.c_void_p, C.POINTER(FrameParams), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                            C.c_void_p]),
     "rdc_scene_pick": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_float, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "rdc_scene_pick_frame": (C.c_int, [C.c_void_p, C.POINTER(FrameParams), C.c_float, C.c_void_p, C.c_void_p, C.c_void_p]),
     "rdc_view_pixel_to_scene": (C.c_int, [C.POINTER(FrameParams), C.c_uint32, C.c_uint32, f32p, f32p]),
@@ -458,6 +460,16 @@ class Scene:
         [rows, W] (band-local); out_ptr: device float64 laid out like the handle's blur array (n_blur + 2)."""
         _check(_lib.rdc_render_blur_adjoint(self._h, C.byref(params), C.c_void_p(grad_ptr), C.c_void_p(out_ptr),
                                             C.c_void_p(stream)), "rdc_render_blur_adjoint")
+
+    def weight_adjoint(self, params: FrameParams, image_grad_ptr: int, sigma_grad_ptr: int, weight_ptr: int, degree_ptr: int,
+                       stream: int = 0) -> None:
+        """rdc_render_weight_adjoint: the gradient of the render's image and blur map in the weight and exponent stops, for
+        a device float4 image gradient and a device float32 sigma gradient ([rows, W], band-local; 0 means zero, not both).
+        weight_ptr / degree_ptr: device float64 laid out like the handle's weight (n_weight + 2) and weight_degree
+        (n_weight_degree + 2) arrays."""
+        _check(_lib.rdc_render_weight_adjoint(self._h, C.byref(params), C.c_void_p(image_grad_ptr), C.c_void_p(sigma_grad_ptr),
+                                              C.c_void_p(weight_ptr), C.c_void_p(degree_ptr), C.c_void_p(stream)),
+               "rdc_render_weight_adjoint")
 
     def pick(self, points_ptr: int, n: int, out_ptr: int, stops_ptr: int = 0, max_distance: float = float("inf"),
              use_diffusion_curve_save: int = 1, stream: int = 0) -> None:
@@ -880,6 +892,109 @@ def fit_blur(scene: "Scene", d: dict, params: FrameParams, target, iterations: i
     x, objectives = projected_descent(f_and_grad, x0, np.zeros(nb), iterations)
     fitted = {k: (v.copy() if isinstance(v, np.ndarray) else v) for k, v in d.items()}
     fitted["blur"] = stops(x)
+    scene.update_stops(arrays_from_numpy(fitted), stream)
+    return fitted, objectives
+
+
+def weight_unknowns(d: dict):
+    """The unknowns of fit_weights for a scene laid out like HostScene.to_numpy(): the real weight stops (j < n_weight) that
+    are > 0, as log(weight), then the real exponent stops (j < n_weight_degree), raw. Returns (x0, lower, stops, chain):
+    x0 the start and lower the bounds (-inf for the logs, min(0, start) for the exponents), float64; stops(x) -> (weight,
+    weight_degree), float32 arrays laid out like d's in which every other entry (weights <= 0, padding, sentinels) keeps d's
+    value; chain(x, grad_weight, grad_weight_degree) -> the gradient in x of a loss whose gradient in the two arrays is given
+    (weight * dL/dweight for the logs). With log weights the weights stay positive, and scaling them all, which leaves the
+    frame unchanged, is a shift of the logs that the fit never needs to resolve."""
+    nw, ne = int(d["n_weight"]), int(d["n_weight_degree"])
+    base_w = np.asarray(d["weight"], np.float32)
+    base_e = np.asarray(d["weight_degree"], np.float32)
+    free = np.flatnonzero(base_w[:nw] > 0)
+    k = free.size
+    x0 = np.concatenate([np.log(base_w[free].astype(np.float64)), base_e[:ne].astype(np.float64)])
+    lower = np.concatenate([np.full(k, -np.inf), np.minimum(0.0, base_e[:ne].astype(np.float64))])
+
+    def stops(x):
+        weight, degree = base_w.copy(), base_e.copy()
+        weight[free] = np.exp(x[:k])
+        degree[:ne] = x[k:]
+        return weight, degree
+
+    def chain(x, grad_weight, grad_degree):
+        weight = stops(x)[0][free].astype(np.float64)
+        return np.concatenate([weight * np.asarray(grad_weight, np.float64)[free], np.asarray(grad_degree, np.float64)[:ne]])
+
+    return x0, lower, stops, chain
+
+
+def fit_weights(scene: "Scene", d: dict, params: FrameParams, target, iterations: int = 30, stream: int | None = None,
+                use_blur: bool = False):
+    """Weight and exponent stops whose render of `params` comes closest to `target`: minimises 1/2 ||frame - target||^2 over
+    the unknowns of weight_unknowns(d) with projected_descent, the curves, colours, blur and u lists of `d`
+    (HostScene.to_numpy() layout, the scene `scene` was built from) fixed. target: float32 [rows, W, 3|4], numpy or torch,
+    the band of `params`; pixels NaN in the target or in the start's frame are ignored, and a step that makes a kept pixel
+    NaN (all its weights driven to 0) has a NaN objective, which the line search refuses. One evaluation is update_stops,
+    render, the residual and Scene.weight_adjoint with the image gradient. use_blur: fit the blurred frame instead, exactly
+    what rdc_render_frame_to_host(params, use_blur=1) writes; the weights move both the image and the blur map, so the
+    gradient is gaussian_blur_adjoint and gaussian_blur_sigma_adjoint of the residual, then Scene.weight_adjoint with both.
+    Returns (fitted copy of d, objective of every iteration); on return the handle holds the fitted stops. `stream` must be
+    torch's current stream (the default)."""
+    import torch
+
+    if stream is None:
+        stream = torch.cuda.current_stream().cuda_stream
+    rows, w = params.row_end - params.row_begin, params.image_width
+    dev = torch.device("cuda", torch.cuda.current_device())
+    x0, lower, stops, chain = weight_unknowns(d)
+    image = torch.empty((rows, w, 4), dtype=torch.float32, device=dev)
+    sigma = torch.empty((rows, w), dtype=torch.float32, device=dev)
+    grad_image = torch.zeros_like(image)
+    grad_weight = torch.empty(np.asarray(d["weight"]).shape, dtype=torch.float64, device=dev)
+    grad_degree = torch.empty(np.asarray(d["weight_degree"]).shape, dtype=torch.float64, device=dev)
+    if use_blur:
+        blurred = torch.empty_like(image)
+        grad_source = torch.empty_like(image)
+        grad_sigma = torch.empty_like(sigma)
+        scratch = torch.empty((2 * rows * w + 1, 4), dtype=torch.float32, device=dev)  # the blur's and both derivatives'
+        flag = torch.zeros((1,), dtype=torch.float32, device=dev)
+        blur_params = FrameParams.from_buffer_copy(params)
+        blur_params.max_sigma = flag.data_ptr()
+    target3 = torch.as_tensor(target, dtype=torch.float32, device=dev)[..., :3].to(torch.float64)
+    work = dict(d)
+    scene.reserve(params, False, stream)
+
+    def frame(x):
+        work["weight"], work["weight_degree"] = stops(x)
+        scene.update_stops(arrays_from_numpy(work), stream)
+        if not use_blur:
+            scene.render(params, image.data_ptr(), sigma.data_ptr(), stream)
+            return image[..., :3].to(torch.float64)
+        flag.zero_()
+        scene.render(blur_params, image.data_ptr(), sigma.data_ptr(), stream)
+        gaussian_blur(blurred.data_ptr(), image.data_ptr(), sigma.data_ptr(), scratch.data_ptr(), w, rows, 0, rows, flag.data_ptr(),
+                      stream)
+        return blurred[..., :3].to(torch.float64)
+
+    keep = ~(torch.isnan(frame(x0)).any(-1) | torch.isnan(target3).any(-1))[..., None]
+
+    def f_and_grad(x):
+        r = torch.where(keep, frame(x) - target3, torch.zeros((), dtype=torch.float64, device=dev))
+        f = 0.5 * float((r * r).sum())
+        if not np.isfinite(f):  # refused by the line search: no gradient needed
+            return f, np.full_like(x, np.nan)
+        grad_image[..., :3] = r
+        if not use_blur:
+            scene.weight_adjoint(params, grad_image.data_ptr(), 0, grad_weight.data_ptr(), grad_degree.data_ptr(), stream)
+        else:
+            gaussian_blur_adjoint(grad_source.data_ptr(), grad_image.data_ptr(), sigma.data_ptr(), scratch.data_ptr(), w, rows, 0,
+                                  rows, flag.data_ptr(), stream)
+            gaussian_blur_sigma_adjoint(grad_sigma.data_ptr(), grad_image.data_ptr(), image.data_ptr(), sigma.data_ptr(),
+                                        scratch.data_ptr(), w, rows, 0, rows, flag.data_ptr(), stream)
+            scene.weight_adjoint(params, grad_source.data_ptr(), grad_sigma.data_ptr(), grad_weight.data_ptr(),
+                                 grad_degree.data_ptr(), stream)
+        return f, chain(x, grad_weight.cpu().numpy(), grad_degree.cpu().numpy())
+
+    x, objectives = projected_descent(f_and_grad, x0, lower, iterations)
+    fitted = {k: (v.copy() if isinstance(v, np.ndarray) else v) for k, v in d.items()}
+    fitted["weight"], fitted["weight_degree"] = stops(x)
     scene.update_stops(arrays_from_numpy(fitted), stream)
     return fitted, objectives
 

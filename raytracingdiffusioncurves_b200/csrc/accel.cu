@@ -767,6 +767,8 @@ int build_scene(const rdc_scene_arrays& a, const rdc_accel_options& o, cudaStrea
   point_stops(d, s->stops, stop_at);
   s->colour_stops = (uint32_t)stop_at.len[0];
   s->blur_stops = (uint32_t)stop_at.len[2];
+  s->weight_stops = (uint32_t)stop_at.len[3];
+  s->degree_stops = (uint32_t)stop_at.len[4];
   d.n_segments = a.n_segments;
   d.n_curves = a.n_curves;
   d.seg_walk = up.alloc<SegWalk>(a.n_segments);
@@ -1065,6 +1067,8 @@ int update_stops(rdc_scene* s, const rdc_scene_arrays& a, cudaStream_t stream) {
   point_stops(s->dev, s->stops, L);
   s->colour_stops = (uint32_t)L.len[0];
   s->blur_stops = (uint32_t)L.len[2];
+  s->weight_stops = (uint32_t)L.len[3];
+  s->degree_stops = (uint32_t)L.len[4];
   if (int rc = launch_stop_tables(s, stream)) return rc;
   RDC_CUDA(cudaEventRecord(s->launched, stream));
   s->launched_on = stream;

@@ -375,6 +375,18 @@ int rdc_render_blur_adjoint(rdc_scene* scene, const rdc_frame_params* params, co
   });
 }
 
+int rdc_render_weight_adjoint(rdc_scene* scene, const rdc_frame_params* params, const float* image_grad, const float* sigma_grad,
+                              double* grad_weight, double* grad_weight_degree, rdc_stream stream) {
+  if (!params) {
+    rdc::set_error("render weight adjoint: null params");
+    return RDC_E_INVALID;
+  }
+  return guarded(RDC_E_INVALID, [&]() {
+    return rdc::weight_adjoint(scene, *params, reinterpret_cast<const float4*>(image_grad), sigma_grad, grad_weight,
+                               grad_weight_degree, (cudaStream_t)stream);
+  });
+}
+
 int rdc_scene_pick(rdc_scene* scene, const float* points, uint32_t n, float max_distance, int use_diffusion_curve_save,
                    rdc_pick* out, float* stops, rdc_stream stream) {
   return guarded(RDC_E_INVALID, [&]() {

@@ -103,6 +103,8 @@ struct rdc_scene {
   cudaEvent_t staged = nullptr;
   uint32_t colour_stops = 0;  // stops per colour family in the block: max(n_color_left, n_color_right) + 2
   uint32_t blur_stops = 0;    // blur stops in the block: n_blur + 2
+  uint32_t weight_stops = 0;  // weight stops in the block: n_weight + 2
+  uint32_t degree_stops = 0;  // exponent stops in the block: n_weight_degree + 2
   // per-N table of the iterated base directions (DeviceCode.cu:110-112,167-171)
   float2* base_dirs = nullptr;
   float base_dirs_n = -1.0f;
@@ -153,6 +155,8 @@ int launch_plan(const rdc_scene* s, const rdc_frame_params& p, rdc_launch_plan* 
 int color_adjoint(rdc_scene* s, const rdc_frame_params& p, const float4* image_grad, double* grad_left, double* grad_right,
                   cudaStream_t stream);
 int blur_adjoint(rdc_scene* s, const rdc_frame_params& p, const float* sigma_grad, double* grad_blur, cudaStream_t stream);
+int weight_adjoint(rdc_scene* s, const rdc_frame_params& p, const float4* image_grad, const float* sigma_grad, double* grad_weight,
+                   double* grad_degree, cudaStream_t stream);
 // pick.cu
 int pick(rdc_scene* s, const float* points, uint32_t n, float max_distance, int orzan, rdc_pick* out, float* stops,
          cudaStream_t stream);

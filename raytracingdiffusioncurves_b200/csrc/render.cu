@@ -1778,20 +1778,56 @@ int ensure_capacity(rdc_scene* s, const LaunchPlan& L, cudaStream_t stream) {
 // the ray shades. The blur map is the same kind of map in the blur values (sigma = sum_i w_i b_i / sum_i w_i, one channel,
 // one list). The rays are the render's: its tile grid, Philox draws, pixel culling and closest hit (the tree, which
 // finds the first hits every route finds, or the brute force), and the terminal shading walks of trace_from.
+// ---- rdc_render_weight_adjoint: the derivative of the image and the blur map in the weight and exponent stops ----
+// w_i = m_i t_i^-e_i with m_i and e_i lerped from the weight and weight_degree lists; the frame is smooth in those values
+// where W > 0. With s_i = <G, c_i> + g_sigma b_i and K = sum_i w_i s_i / W, dL/dw_i = (s_i - K) / W, and the chain through
+// m_i and e_i sends (1 - rho_w) f_i (s_i - K) / W to weight[iw] (rho_w ... to iw + 1) and -(1 - rho_e) w_i ln t_i (s_i - K) / W
+// to weight_degree[ie] (rho_e ... to ie + 1), f_i = t_i^-e_i.
 struct AdjointArgs {
   RenderArgs r;                // the view (the output and work-unit fields stay unset)
-  const float4* grad;          // colour: [local rows * width] dL/dRGB of each pixel of the band; .w ignored
+  const float4* grad;          // colour, weight (or null): [local rows * width] dL/dRGB of each pixel of the band; .w ignored
   double* left;                // colour: [3 * colour_stops] Aᵀ grad in color_left ...
   double* right;               // ... and in color_right
   uint32_t tiles_x, n_tiles;
   int portals;                 // the scene has portal curves: a hit on one contributes nothing (max_trace_depth 0)
-  const float* sigma_grad;     // blur: [local rows * width] dL/dsigma of each pixel of the band
+  const float* sigma_grad;     // blur, weight (or null): [local rows * width] dL/dsigma of each pixel of the band
   double* blur;                // blur: [blur_stops] A_bᵀ sigma_grad
+  double* weight;              // weight: [weight_stops] dL/dweight
+  double* degree;              // weight: [degree_stops] dL/dweight_degree
 };
 
-enum StopFamily : int { kColourStops, kBlurStops };
+enum StopFamily : int { kColourStops, kBlurStops, kWeightStops };
 
 constexpr uint32_t kNoStop = 0xFFFFFFFFu;
+
+// Primary ray i of a pixel and its closest hit, with the walk ranges of the hit's segment and chord. False for a miss and
+// for a hit on a portal curve (max_trace_depth 0: contributes nothing).
+struct AdjointHit {
+  Hit h;
+  float dx, dy, u, cu;
+  uint32_t seg;
+  uint4 wc, ws, wd, cw, cw2;
+};
+
+__device__ __forceinline__ bool adjoint_hit(const AdjointArgs& aa, const Accel& ac, const Pixel& px, int i, bool small_angle,
+                                            AdjointHit& r) {
+  const RenderArgs& a = aa.r;
+  const DevScene& sc = a.sc;
+  Counters cnt;
+  float ox, oy;
+  gen_ray(a, px.pixel, px.base_x, px.base_y, i, small_angle, ox, oy, r.dx, r.dy);
+  r.h = closest_chord<false, false, false>(ac, a.brute != 0, ox, oy, r.dx, r.dy, true, 1u, 0u, __int_as_float(0x7f800000), cnt);
+  if (r.h.leaf < 0) return false;
+  const uint4 id = __ldg(sc.run_ids + r.h.leaf);
+  r.seg = id.y;
+  const uint4* wp = reinterpret_cast<const uint4*>(sc.seg_walk + r.seg);
+  r.wc = __ldg(wp), r.ws = __ldg(wp + 1), r.wd = __ldg(wp + 2);
+  if (aa.portals && __ldg(sc.curve_connect + r.wd.z) >= 0) return false;
+  r.u = rdc_hit_u((int)id.z + r.h.j, (int)id.w, r.h.s);
+  r.cw = __ldg(sc.chord_walk + 2 * (size_t)r.h.id), r.cw2 = __ldg(sc.chord_walk + 2 * (size_t)r.h.id + 1);
+  r.cu = r.u + r.wd.w;
+  return true;
+}
 
 // One primary ray of the adjoint: its weight w_i (0 for a miss or a portal hit) and, with KEY, the stop of FAMILY it
 // interpolates from (colour: key = ind << 1 | right; blur: key = ind) and the ratio rho. Same operands and operations as
@@ -1799,44 +1835,101 @@ constexpr uint32_t kNoStop = 0xFFFFFFFFu;
 template <int FAMILY, bool KEY>
 __device__ __forceinline__ float adjoint_ray(const AdjointArgs& aa, const Accel& ac, const Pixel& px, int i, bool small_angle,
                                              uint32_t& key, float& ratio) {
-  const RenderArgs& a = aa.r;
-  const DevScene& sc = a.sc;
-  Counters cnt;
-  float ox, oy, dx, dy;
-  gen_ray(a, px.pixel, px.base_x, px.base_y, i, small_angle, ox, oy, dx, dy);
-  const Hit h = closest_chord<false, false, false>(ac, a.brute != 0, ox, oy, dx, dy, true, 1u, 0u, __int_as_float(0x7f800000), cnt);
+  const DevScene& sc = aa.r.sc;
+  AdjointHit r;
   key = kNoStop;
-  if (h.leaf < 0) return 0.0f;
-  const uint4 id = __ldg(sc.run_ids + h.leaf);
-  const uint32_t seg = id.y;
-  const uint4* wp = reinterpret_cast<const uint4*>(sc.seg_walk + seg);
-  const uint4 wc = __ldg(wp), ws = __ldg(wp + 1), wd = __ldg(wp + 2);
-  if (aa.portals && __ldg(sc.curve_connect + wd.z) >= 0) return 0.0f;
-  const float u = rdc_hit_u((int)id.z + h.j, (int)id.w, h.s);
-  const uint4 cw = __ldg(sc.chord_walk + 2 * (size_t)h.id), cw2 = __ldg(sc.chord_walk + 2 * (size_t)h.id + 1);
-  const float cu = u + wd.w;
-  const float wm = scalar_stop(sc.weight, cw.w, ws.w, cu);
-  const float e = scalar_stop(sc.weight_degree, cw2.x, wd.y, cu);
-  const float w = wm * rdc_weight_falloff(h.t, e);
+  if (!adjoint_hit(aa, ac, px, i, small_angle, r)) return 0.0f;
+  const float wm = scalar_stop(sc.weight, r.cw.w, r.ws.w, r.cu);
+  const float e = scalar_stop(sc.weight_degree, r.cw2.x, r.wd.y, r.cu);
+  const float w = wm * rdc_weight_falloff(r.h.t, e);
   if (KEY && FAMILY == kColourStops) {
     rdc_f2 v[4];
-    load_control_points(sc, seg, v);
-    const bool right = rdc_is_ray_right(u, dx, dy, v[0], v[1], v[2], v[3], a.orzan != 0);
-    const int ind = right ? rdc_interp_from(cw.y, wc.w, cu, sc.color_right.u, &ratio)
-                          : rdc_interp_from(cw.x, wc.y, cu, sc.color_left.u, &ratio);
+    load_control_points(sc, r.seg, v);
+    const bool right = rdc_is_ray_right(r.u, r.dx, r.dy, v[0], v[1], v[2], v[3], aa.r.orzan != 0);
+    const int ind = right ? rdc_interp_from(r.cw.y, r.wc.w, r.cu, sc.color_right.u, &ratio)
+                          : rdc_interp_from(r.cw.x, r.wc.y, r.cu, sc.color_left.u, &ratio);
     key = ((uint32_t)ind << 1) | (right ? 1u : 0u);
   }
-  if (KEY && FAMILY == kBlurStops) key = (uint32_t)rdc_interp_from(cw.z, ws.y, cu, sc.blur.u, &ratio);
+  if (KEY && FAMILY == kBlurStops) key = (uint32_t)rdc_interp_from(r.cw.z, r.ws.y, r.cu, sc.blur.u, &ratio);
   return w;
 }
 
+// One primary ray of the weight adjoint: w_i and s_i = <G, c_i> + g_sigma b_i (g.w = g_sigma) with the render's weight,
+// side, colour and blur walks (all 0 for a miss or a portal hit); with KEY also the weight and exponent stops the ray
+// interpolates from, their ratios, f_i = t_i^-e_i and t_i.
+struct WeightRay {
+  float w, f, t, rw, re;
+  double s;
+  uint32_t iw, ie;
+};
+
+template <bool KEY>
+__device__ __forceinline__ WeightRay weight_ray(const AdjointArgs& aa, const Accel& ac, const Pixel& px, int i, bool small_angle,
+                                                float4 g) {
+  const DevScene& sc = aa.r.sc;
+  WeightRay out{0.0f, 0.0f, 0.0f, 0.0f, 0.0f, 0.0, kNoStop, kNoStop};
+  AdjointHit r;
+  if (!adjoint_hit(aa, ac, px, i, small_angle, r)) return out;
+  // scalar_stop's walks, with the index kept
+  float rw, re;
+  const int iw = rdc_interp_from(r.cw.w, r.ws.w, r.cu, sc.weight.u, &rw);
+  const int ie = rdc_interp_from(r.cw2.x, r.wd.y, r.cu, sc.weight_degree.u, &re);
+  const float wm = rdc_lerp_stop(__ldg(sc.weight.value + iw), __ldg(sc.weight.value + iw + 1), rw);
+  const float e = rdc_lerp_stop(__ldg(sc.weight_degree.value + ie), __ldg(sc.weight_degree.value + ie + 1), re);
+  const float f = rdc_weight_falloff(r.h.t, e);
+  out.w = wm * f;
+  rdc_f2 v[4];
+  load_control_points(sc, r.seg, v);
+  const bool right = rdc_is_ray_right(r.u, r.dx, r.dy, v[0], v[1], v[2], v[3], aa.r.orzan != 0);
+  float cr, cg, cb;
+  if (right) colour_stop(r.cw.y, r.wc.w, sc.color_right.u, sc.color_right.rgb, r.cu, cr, cg, cb);
+  else colour_stop(r.cw.x, r.wc.y, sc.color_left.u, sc.color_left.rgb, r.cu, cr, cg, cb);
+  const float blur = scalar_stop(sc.blur, r.cw.z, r.ws.y, r.cu);
+  // a zero gradient component adds nothing, whatever the stop value
+  out.s = (g.x != 0.0f ? (double)g.x * cr : 0.0) + (g.y != 0.0f ? (double)g.y * cg : 0.0) +
+          (g.z != 0.0f ? (double)g.z * cb : 0.0) + (g.w != 0.0f ? (double)g.w * blur : 0.0);
+  if (KEY) {
+    out.f = f, out.t = r.h.t, out.rw = rw, out.re = re;
+    out.iw = (uint32_t)iw, out.ie = (uint32_t)ie;
+  }
+  return out;
+}
+
+// Lanes whose rays end on the same stop `key` (usually most of the tile) add their terms up first (__match_any_sync, then
+// a butterfly in fp64 per group, all lanes taking part), and the group's first lane issues one atomicAdd(double) per term
+// at dst(key). terms(v, mine) writes a lane's terms into v, zeros unless `mine`. kNoStop: the lane adds nothing.
+template <int kTerms, typename Terms, typename Dst>
+__device__ __forceinline__ void scatter_groups(uint32_t lane, uint32_t key, Terms terms, Dst dst) {
+  const uint32_t peers = __match_any_sync(0xFFFFFFFFu, key);
+  const bool leader = key != kNoStop && lane == (uint32_t)(__ffs(peers) - 1);
+  uint32_t leaders = __ballot_sync(0xFFFFFFFFu, leader);
+  while (leaders) {  // one group (one stop of one family) at a time
+    const uint32_t l = (uint32_t)(__ffs(leaders) - 1);
+    leaders &= leaders - 1;
+    const uint32_t group = __shfl_sync(0xFFFFFFFFu, peers, l);
+    const bool mine = (group >> lane) & 1u;
+    double v[kTerms];
+    terms(v, mine);
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1)
+#pragma unroll
+      for (int c = 0; c < kTerms; ++c) v[c] += __shfl_xor_sync(0xFFFFFFFFu, v[c], off);
+    if (lane == l) {
+      double* d = dst(key);
+#pragma unroll
+      for (int c = 0; c < kTerms; ++c) atomicAdd(d + c, v[c]);
+    }
+  }
+}
+
 // One warp per 8x4 tile of the render's grid, one lane per pixel, all lanes on the same ray index. Pass 1 sums a pixel's
-// weights W in the render's ray order; pass 2 traces the rays again and scatters. Lanes whose rays end on the same stop of
-// the same family (usually most of the tile) add their terms up first (__match_any_sync, then a butterfly in fp64 per
-// group), and the group's first lane issues the atomicAdd(double): six per group for the colours, two for the blur.
+// weights W in the render's ray order (and, for the weights, sum_i w_i s_i and W in fp64); pass 2 traces the rays again and
+// scatters through scatter_groups: six terms per group for the colours, two for the blur, two per family in two rounds for
+// the weights.
 template <int FAMILY>
 __global__ void __launch_bounds__(kBlock) k_stop_adjoint(const AdjointArgs aa) {
   constexpr bool kColour = FAMILY == kColourStops;
+  constexpr bool kWeight = FAMILY == kWeightStops;
   constexpr int kTerms = kColour ? 6 : 2;
   const RenderArgs& a = aa.r;
   const uint32_t lane = threadIdx.x & 31, tile = blockIdx.x * (kBlock / 32) + (threadIdx.x >> 5);
@@ -1853,11 +1946,17 @@ __global__ void __launch_bounds__(kBlock) k_stop_adjoint(const AdjointArgs aa) {
   const Pixel px = tile_pixel(a, tile, aa.tiles_x, lane);
   float4 g = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
   if (px.valid) {
-    if (kColour) g = __ldg(aa.grad + px.local);
-    else g.x = __ldg(aa.sigma_grad + px.local);
+    if (kColour) {
+      g = __ldg(aa.grad + px.local);
+    } else if (kWeight) {  // g.w = dL/dsigma; a null gradient is zero
+      if (aa.grad) g = __ldg(aa.grad + px.local);
+      g.w = aa.sigma_grad ? __ldg(aa.sigma_grad + px.local) : 0.0f;
+    } else {
+      g.x = __ldg(aa.sigma_grad + px.local);
+    }
   }
   // a pixel whose gradient is zero contributes nothing: its rays are not traced
-  bool live = px.valid && (g.x != 0.0f || g.y != 0.0f || g.z != 0.0f);
+  bool live = px.valid && (g.x != 0.0f || g.y != 0.0f || g.z != 0.0f || (kWeight && g.w != 0.0f));
   int cull_first = 0, cull_span = n - 1;
   const float jit = jitter(a);
   if (!pixel_cull(a, Rect{px.base_x - jit, px.base_x + jit, px.base_y - jit, px.base_y + jit}, cull_first, cull_span)) {
@@ -1873,47 +1972,66 @@ __global__ void __launch_bounds__(kBlock) k_stop_adjoint(const AdjointArgs aa) {
   float ratio = 0.0f;
   // pass 1: W = sum of the weights, in fp32 and in ray order like PixelSums::add
   float W = 0.0f;
+  double W64 = 0.0, WS = 0.0;  // weights: W and sum_i w_i s_i in fp64
   if (live) {
 #pragma unroll 1
-    for (int i = 0; i < n; ++i)
-      if (reaches(i)) W += adjoint_ray<FAMILY, false>(aa, ac, px, i, small_angle, key, ratio);
+    for (int i = 0; i < n; ++i) {
+      if (!reaches(i)) continue;
+      if constexpr (kWeight) {
+        const WeightRay r = weight_ray<false>(aa, ac, px, i, small_angle, g);
+        W += r.w;
+        W64 += (double)r.w;
+        WS += (double)r.w * r.s;
+      } else {
+        W += adjoint_ray<FAMILY, false>(aa, ac, px, i, small_angle, key, ratio);
+      }
+    }
   }
   live = live && W != 0.0f;  // W == 0: the render writes NaN, the pixel is outside the image's linear map
-  const double inv_w = live ? 1.0 / (double)W : 0.0;
-  // pass 2
+  if constexpr (kWeight) {
+    // K and 1/W from the fp64 sums: sum_i w_i (s_i - K) then vanishes to fp64 rounding, so the weights' gradient keeps the
+    // frame's invariance to scaling every weight
+    const double inv_w = live ? 1.0 / W64 : 0.0, K = WS * inv_w;
 #pragma unroll 1
-  for (int i = 0; i < n; ++i) {
-    const bool on = live && reaches(i);
-    if (!__any_sync(0xFFFFFFFFu, on)) continue;
-    key = kNoStop;
-    float w = 0.0f;
-    if (on) w = adjoint_ray<FAMILY, true>(aa, ac, px, i, small_angle, key, ratio);
-    const double f = (double)w * inv_w, f1 = f * (double)ratio, f0 = f * (double)(1.0f - ratio);
-    const double gx = g.x, gy = g.y, gz = g.z;
-    const uint32_t peers = __match_any_sync(0xFFFFFFFFu, key);
-    const bool leader = key != kNoStop && lane == (uint32_t)(__ffs(peers) - 1);
-    uint32_t leaders = __ballot_sync(0xFFFFFFFFu, leader);
-    while (leaders) {  // one group (one stop of one family) at a time; all lanes take part in its butterfly
-      const uint32_t l = (uint32_t)(__ffs(leaders) - 1);
-      leaders &= leaders - 1;
-      const uint32_t group = __shfl_sync(0xFFFFFFFFu, peers, l);
-      const bool mine = (group >> lane) & 1u;
-      double v[kTerms];
-      if (kColour) {
-        v[0] = mine ? gx * f0 : 0.0, v[1] = mine ? gy * f0 : 0.0, v[2] = mine ? gz * f0 : 0.0;
-        v[3] = mine ? gx * f1 : 0.0, v[4] = mine ? gy * f1 : 0.0, v[5] = mine ? gz * f1 : 0.0;
-      } else {
-        v[0] = mine ? gx * f0 : 0.0, v[1] = mine ? gx * f1 : 0.0;
-      }
-#pragma unroll
-      for (int off = 16; off > 0; off >>= 1)
-#pragma unroll
-        for (int c = 0; c < kTerms; ++c) v[c] += __shfl_xor_sync(0xFFFFFFFFu, v[c], off);
-      if (lane == l) {
-        double* dst = kColour ? ((key & 1u) ? aa.right : aa.left) + 3 * (size_t)(key >> 1) : aa.blur + key;
-#pragma unroll
-        for (int c = 0; c < kTerms; ++c) atomicAdd(dst + c, v[c]);
-      }
+    for (int i = 0; i < n; ++i) {
+      const bool on = live && reaches(i);
+      if (!__any_sync(0xFFFFFFFFu, on)) continue;
+      WeightRay r{0.0f, 0.0f, 0.0f, 0.0f, 0.0f, 0.0, kNoStop, kNoStop};
+      if (on) r = weight_ray<true>(aa, ac, px, i, small_angle, g);
+      const double q = r.iw == kNoStop ? 0.0 : (r.s - K) * inv_w;
+      const double fw = (double)r.f * q, de = r.iw == kNoStop ? 0.0 : -(double)r.w * log((double)r.t) * q;
+      scatter_groups<2>(
+          lane, r.iw,
+          [&](double* v, bool mine) { v[0] = mine ? fw * (double)(1.0f - r.rw) : 0.0, v[1] = mine ? fw * (double)r.rw : 0.0; },
+          [&](uint32_t k) { return aa.weight + k; });
+      scatter_groups<2>(
+          lane, r.ie,
+          [&](double* v, bool mine) { v[0] = mine ? de * (double)(1.0f - r.re) : 0.0, v[1] = mine ? de * (double)r.re : 0.0; },
+          [&](uint32_t k) { return aa.degree + k; });
+    }
+  } else {
+    const double inv_w = live ? 1.0 / (double)W : 0.0;
+    // pass 2
+#pragma unroll 1
+    for (int i = 0; i < n; ++i) {
+      const bool on = live && reaches(i);
+      if (!__any_sync(0xFFFFFFFFu, on)) continue;
+      key = kNoStop;
+      float w = 0.0f;
+      if (on) w = adjoint_ray<FAMILY, true>(aa, ac, px, i, small_angle, key, ratio);
+      const double f = (double)w * inv_w, f1 = f * (double)ratio, f0 = f * (double)(1.0f - ratio);
+      const double gx = g.x, gy = g.y, gz = g.z;
+      auto terms = [&](double* v, bool mine) {
+        if constexpr (kColour) {
+          v[0] = mine ? gx * f0 : 0.0, v[1] = mine ? gy * f0 : 0.0, v[2] = mine ? gz * f0 : 0.0;
+          v[3] = mine ? gx * f1 : 0.0, v[4] = mine ? gy * f1 : 0.0, v[5] = mine ? gz * f1 : 0.0;
+        } else {
+          v[0] = mine ? gx * f0 : 0.0, v[1] = mine ? gx * f1 : 0.0;
+        }
+      };
+      scatter_groups<kTerms>(lane, key, terms, [&](uint32_t k) {
+        return kColour ? ((k & 1u) ? aa.right : aa.left) + 3 * (size_t)(k >> 1) : aa.blur + k;
+      });
     }
   }
 }
@@ -2073,7 +2191,7 @@ int render(rdc_scene* s, const rdc_frame_params& p, float4* image, float* blur_m
 
 namespace {
 
-// The common part of color_adjoint and blur_adjoint: the checks, the wait for the handle's previous launch, the zeroing of
+// The common part of color_adjoint, blur_adjoint and weight_adjoint: the checks, the wait for the handle's previous launch, the zeroing of
 // the outputs and the launch of k_stop_adjoint<FAMILY>. `aa` carries the family's gradient and outputs; `what` names the call
 // in messages, `stops` the family.
 template <int FAMILY>
@@ -2085,9 +2203,14 @@ int stop_adjoint(rdc_scene* s, const rdc_frame_params& p, AdjointArgs aa, const 
     return RDC_E_INVALID;
   }
   if (s->info.has_portals && p.max_trace_depth > 0) {
-    set_error("%s: the scene has portals and max_trace_depth is %d; through a portal the %s is a product of "
-              "%s stops, not linear in them (use max_trace_depth 0)", what, p.max_trace_depth,
-              FAMILY == kColourStops ? "image" : "blur map", stops);
+    if (FAMILY == kWeightStops)
+      set_error("%s: the scene has portals and max_trace_depth is %d; through a portal a ray's weight 1/(1/w_T + S) mixes "
+                "the %s stops of several curves and its colour is a product (use max_trace_depth 0)", what, p.max_trace_depth,
+                stops);
+    else
+      set_error("%s: the scene has portals and max_trace_depth is %d; through a portal the %s is a product of "
+                "%s stops, not linear in them (use max_trace_depth 0)", what, p.max_trace_depth,
+                FAMILY == kColourStops ? "image" : "blur map", stops);
     return RDC_E_INVALID;
   }
   LaunchPlan L;  // one unit per tile: only the table of base directions is needed
@@ -2098,8 +2221,11 @@ int stop_adjoint(rdc_scene* s, const rdc_frame_params& p, AdjointArgs aa, const 
     const size_t bytes = 3 * (size_t)s->colour_stops * sizeof(double);
     RDC_CUDA(cudaMemsetAsync(aa.left, 0, bytes, stream));
     RDC_CUDA(cudaMemsetAsync(aa.right, 0, bytes, stream));
-  } else {
+  } else if (FAMILY == kBlurStops) {
     RDC_CUDA(cudaMemsetAsync(aa.blur, 0, (size_t)s->blur_stops * sizeof(double), stream));
+  } else {
+    RDC_CUDA(cudaMemsetAsync(aa.weight, 0, (size_t)s->weight_stops * sizeof(double), stream));
+    RDC_CUDA(cudaMemsetAsync(aa.degree, 0, (size_t)s->degree_stops * sizeof(double), stream));
   }
   if (int rc = ensure_base_dirs(s, L, p, stream)) return rc;
   RenderArgs& a = aa.r;
@@ -2163,6 +2289,21 @@ int blur_adjoint(rdc_scene* s, const rdc_frame_params& p, const float* sigma_gra
   aa.sigma_grad = sigma_grad;
   aa.blur = grad_blur;
   return stop_adjoint<kBlurStops>(s, p, aa, "render blur adjoint", "blur", stream);
+}
+
+int weight_adjoint(rdc_scene* s, const rdc_frame_params& p, const float4* image_grad, const float* sigma_grad, double* grad_weight,
+                   double* grad_degree, cudaStream_t stream) {
+  if (!s || !grad_weight || !grad_degree || (!image_grad && !sigma_grad)) {
+    set_error("render weight adjoint: null %s", !s ? "scene" : (!grad_weight || !grad_degree) ? "output array"
+                                                                                                : "image_grad and sigma_grad");
+    return RDC_E_INVALID;
+  }
+  AdjointArgs aa{};
+  aa.grad = image_grad;
+  aa.sigma_grad = sigma_grad;
+  aa.weight = grad_weight;
+  aa.degree = grad_degree;
+  return stop_adjoint<kWeightStops>(s, p, aa, "render weight adjoint", "weight and exponent", stream);
 }
 
 }  // namespace rdc
