@@ -43,6 +43,18 @@ struct Stops {
   const float* u;
 };
 
+// What a primary ray decided (oracle_ray_records): the closest chord and where on it, the curve, the side. Layout mirrored
+// by pyoracle.RAY_RECORD.
+struct RayRecord {
+  uint32_t id;        // chord id, 0xFFFFFFFF for a miss
+  float t;            // ray parameter of the hit (+inf for a miss)
+  float segment_u;    // rdc_hit_u of the hit
+  uint32_t curve;
+  float curve_u;      // segment_u + the segment's ordinal in its curve: the u the stop walks compare
+  int32_t right;      // rdc_is_ray_right
+  int32_t portal;     // the hit curve connects to another (at depth 0 it shades nothing)
+};
+
 float scalar_at(const uint32_t* index, const float* value, const float* us, uint32_t curve, float cu) {
   float ratio;
   int ind = rdc_interp(index[2 * curve], index[2 * curve + 1], cu, us, &ratio);
@@ -57,10 +69,10 @@ void colour_at(const uint32_t* index, const float* rgb, const float* us, uint32_
 
 // optixTrace + closest-hit / miss programs. `depth` is payload p5.
 Payload trace(const Ctx& c, float ox, float oy, float dx, float dy, unsigned depth, uint32_t skip_lo, uint32_t skip_hi,
-              uint32_t* hit_id) {
+              RayRecord* rec) {
   const rdc_scene_arrays& a = c.a;
   Hit h = oracle::closest_hit(c.cs, ox, oy, dx, dy, depth == 0, skip_lo, skip_hi);
-  if (hit_id) *hit_id = h.id;
+  if (rec) *rec = RayRecord{h.id, h.t, 0.0f, 0u, 0.0f, 0, 0};
   Payload out;
   if (!h.valid()) return out;  // miss: all zero
   const oracle::Chord& ch = c.cs.chords[h.id];
@@ -76,6 +88,7 @@ Payload trace(const Ctx& c, float ox, float oy, float dx, float dy, unsigned dep
   rdc_f2 v[4];
   oracle::control_points(a, seg, v);
   const bool right = rdc_is_ray_right(segment_u, dx, dy, v[0], v[1], v[2], v[3], c.p.use_diffusion_curve_save != 0);
+  if (rec) *rec = RayRecord{h.id, rt, segment_u, curve, curve_u, right ? 1 : 0, a.curve_connect[curve] >= 0 ? 1 : 0};
 
   if (a.curve_connect[curve] >= 0) {
     const unsigned next_depth = depth + 1;
@@ -122,7 +135,7 @@ Payload trace(const Ctx& c, float ox, float oy, float dx, float dy, unsigned dep
 }
 
 void render_pixel(const Ctx& c, uint32_t ix, uint32_t iy, uint32_t local_row, float* image, float* blur_map,
-                  uint32_t* hit_ids) {
+                  uint32_t* hit_ids, RayRecord* records) {
   const rdc_frame_params& p = c.p;
   const float N = p.number_of_rays_per_pixel;
   float rot_sin, rot_cos;
@@ -144,9 +157,10 @@ void render_pixel(const Ctx& c, uint32_t ix, uint32_t iy, uint32_t local_row, fl
     const float jy = dir_x * rs + dir_y * rc;
     const float ox = origin_x + (p.use_aa ? (rdc_u01(rnd.y) * p.zoom_factor) : 0);
     const float oy = origin_y + (p.use_aa ? (rdc_u01(rnd.z) * p.zoom_factor) : 0);
-    uint32_t id;
-    Payload s = trace(c, ox, oy, p.use_aa ? jx : dir_x, p.use_aa ? jy : dir_y, 0, 1, 0, &id);
-    if (hit_ids) hit_ids[local * n_iter + i] = id;
+    RayRecord rec;
+    Payload s = trace(c, ox, oy, p.use_aa ? jx : dir_x, p.use_aa ? jy : dir_y, 0, 1, 0, &rec);
+    if (hit_ids) hit_ids[local * n_iter + i] = rec.id;
+    if (records) records[local * n_iter + i] = rec;
     weight_total += s.w;
     color[0] += s.r * s.w;
     color[1] += s.g * s.w;
@@ -168,7 +182,33 @@ void render_pixel(const Ctx& c, uint32_t ix, uint32_t iy, uint32_t local_row, fl
 
 namespace {
 int g_search = 0;  // 0: every chord per ray; 1: through the uniform grid of oracle_common.h (same answer, checked in tests/)
+
+// rows of the band, or (strip_stride > 1) the strips t % stride == offset of it, packed (rdc_b200.h)
+std::vector<uint32_t> band_rows(const rdc_frame_params& p) {
+  const uint32_t stride = p.strip_stride > 1 ? p.strip_stride : 1, offset = p.strip_stride > 1 ? p.strip_offset : 0;
+  std::vector<uint32_t> rows;
+  for (uint32_t iy = p.row_begin; iy < p.row_end; ++iy)
+    if (((iy - p.row_begin) / RDC_STRIP_ROWS) % stride == offset) rows.push_back(iy);
+  return rows;
 }
+
+void render_band(const rdc_scene_arrays* a, const rdc_accel_options* o, const rdc_frame_params* p, float* image,
+                 float* blur_map, uint32_t* hit_ids, RayRecord* records, int threads) {
+  ChordSet cs = oracle::build_chords(*a, *o);
+  if (g_search == 1) oracle::build_grid(cs);
+  Ctx c{*a, *p, cs};
+  if (threads <= 0) threads = omp_get_max_threads();
+  const uint32_t stride = p->strip_stride > 1 ? p->strip_stride : 1;
+  const std::vector<uint32_t> rows = band_rows(*p);
+#pragma omp parallel for schedule(dynamic, 1) num_threads(threads)
+  for (size_t r = 0; r < rows.size(); ++r) {
+    const uint32_t iy = rows[r];
+    const uint32_t rel = iy - p->row_begin;
+    const uint32_t local_row = (rel / RDC_STRIP_ROWS / stride) * RDC_STRIP_ROWS + rel % RDC_STRIP_ROWS;
+    for (uint32_t ix = 0; ix < p->image_width; ++ix) render_pixel(c, ix, iy, local_row, image, blur_map, hit_ids, records);
+  }
+}
+}  // namespace
 
 extern "C" {
 
@@ -192,22 +232,18 @@ int oracle_chords(const rdc_scene_arrays* a, const rdc_accel_options* o, float* 
 // image = float4[rows*W], blur_map = float[rows*W], hit_ids optional [rows*W*ceil(N)]; rows = band of params
 int oracle_render(const rdc_scene_arrays* a, const rdc_accel_options* o, const rdc_frame_params* p, float* image,
                   float* blur_map, uint32_t* hit_ids, int threads) {
-  ChordSet cs = oracle::build_chords(*a, *o);
-  if (g_search == 1) oracle::build_grid(cs);
-  Ctx c{*a, *p, cs};
-  if (threads <= 0) threads = omp_get_max_threads();
-  // rows of the band, or (strip_stride > 1) the strips t % stride == offset of it, packed (rdc_b200.h)
-  const uint32_t stride = p->strip_stride > 1 ? p->strip_stride : 1, offset = p->strip_stride > 1 ? p->strip_offset : 0;
-  std::vector<uint32_t> rows;
-  for (uint32_t iy = p->row_begin; iy < p->row_end; ++iy)
-    if (((iy - p->row_begin) / RDC_STRIP_ROWS) % stride == offset) rows.push_back(iy);
-#pragma omp parallel for schedule(dynamic, 1) num_threads(threads)
-  for (size_t r = 0; r < rows.size(); ++r) {
-    const uint32_t iy = rows[r];
-    const uint32_t rel = iy - p->row_begin;
-    const uint32_t local_row = (rel / RDC_STRIP_ROWS / stride) * RDC_STRIP_ROWS + rel % RDC_STRIP_ROWS;
-    for (uint32_t ix = 0; ix < p->image_width; ++ix) render_pixel(c, ix, iy, local_row, image, blur_map, hit_ids);
-  }
+  render_band(a, o, p, image, blur_map, hit_ids, nullptr, threads);
+  return 0;
+}
+
+// The frame's primary rays as render_pixel traces them (same draws, rotation, jitter and closest hit): records =
+// RayRecord[rows*W*ceil(N)], laid out like hit_ids. A portal hit is recorded as the primary ray's hit, whatever lies
+// behind the portal.
+int oracle_ray_records(const rdc_scene_arrays* a, const rdc_accel_options* o, const rdc_frame_params* p, void* records,
+                       int threads) {
+  const size_t pixels = band_rows(*p).size() * (size_t)p->image_width;
+  std::vector<float> image(4 * pixels), blur_map(pixels);
+  render_band(a, o, p, image.data(), blur_map.data(), nullptr, static_cast<RayRecord*>(records), threads);
   return 0;
 }
 

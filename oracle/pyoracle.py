@@ -338,6 +338,12 @@ def arrays_from_dict(d: dict):
     return a, keep
 
 
+# oracle_port.cpp RayRecord: what a primary ray decided
+RAY_RECORD = np.dtype([("id", np.uint32), ("t", np.float32), ("segment_u", np.float32), ("curve", np.uint32),
+                       ("curve_u", np.float32), ("right", np.int32), ("portal", np.int32)])
+MISS = 0xFFFFFFFF
+
+
 def make_params(width, height, rays_per_pixel, **kw) -> FrameParams:
     p = FrameParams()
     p.image_width, p.image_height = width, height
@@ -415,6 +421,28 @@ class Oracle:
             raise RuntimeError(f"{self.kind} oracle render returned {rc}")
         del keep
         return image, blur_map, hits
+
+    def ray_records(self, scene: dict, params: FrameParams, accel: AccelOptions | None = None, search: str = "grid",
+                    threads: int = 0) -> np.ndarray:
+        """The primary rays of the band as render() traces them (Philox draws, rotation, jitter, closest hit): a RAY_RECORD
+        array [rows, W, ceil(N)] laid out like render()'s hit ids, with the chord, t, segment_u, curve, curve_u, side and
+        whether the curve is a portal. Everything downstream of these decisions (stops, weights, the frame) is left to the
+        caller."""
+        assert self.kind == "port"
+        self._set_search({"brute": 0, "grid": 1}[search])
+        accel = accel or make_accel()
+        a, keep = arrays_from_dict(scene)
+        stride = params.strip_stride if params.strip_stride > 1 else 1
+        rows = sum(1 for iy in range(params.row_begin, params.row_end)
+                   if ((iy - params.row_begin) // 8) % stride == (params.strip_offset if stride > 1 else 0))
+        out = np.zeros((rows, params.image_width, int(np.ceil(params.number_of_rays_per_pixel))), RAY_RECORD)
+        self.lib.oracle_ray_records.argtypes = [C.POINTER(SceneArrays), C.POINTER(AccelOptions), C.POINTER(FrameParams),
+                                                C.c_void_p, C.c_int]
+        rc = self.lib.oracle_ray_records(C.byref(a), C.byref(accel), C.byref(params), out.ctypes.data, threads)
+        if rc != 0:
+            raise RuntimeError(f"oracle_ray_records returned {rc}")
+        del keep
+        return out
 
     def trace_rays(self, scene: dict, rays: np.ndarray, accel: AccelOptions | None = None, search: str = "brute"):
         """Closest hit of n primary rays (rays[n,4] = ox, oy, dx, dy): (chord id, t, segment parameter u)."""

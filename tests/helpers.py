@@ -118,15 +118,21 @@ class GpuRenderer:
         return out
 
 
-def curve_xml(points, colour=(255, 64, 0)) -> str:
-    """One curve of the CurveSetXML format: control points as given, two colour stops per side, blur 0 -> 2."""
+def curve_xml(points, colour=(255, 64, 0), weights=None, exponents=None) -> str:
+    """One curve of the CurveSetXML format: control points as given, two colour stops per side, blur 0 -> 2. `weights` and
+    `exponents`, lists of (globalID, value) (u = globalID / 10), add a weight_set and a weight_degree_set; without them the
+    curve takes the ingest's defaults (weight 1, exponent 0.5)."""
     pts = "".join(f'<control_point x="{x:.9g}" y="{y:.9g}" />' for x, y in points)
     r, g, b = colour
+    stops = "".join(f'<{set_name}>' + "".join(f'<{tag} globalID="{gid:.9g}" w="{v:.9g}" />' for gid, v in given) + f'</{set_name}>'
+                    for set_name, tag, given in (("weight_set", "weight", weights), ("weight_degree_set", "weight_degree", exponents))
+                    if given is not None)
     return (f'<curve nb_control_points="{len(points)}"><control_points_set>{pts}</control_points_set>'
             f'<left_colors_set><left_color G="{g}" R="{r}" globalID="0" B="{b}" /><left_color G="{b}" R="{g}" globalID="10" B="{r}" />'
             f'</left_colors_set><right_colors_set><right_color G="{r}" R="{b}" globalID="0" B="{g}" />'
             f'<right_color G="{g}" R="{r}" globalID="10" B="{b}" /></right_colors_set>'
-            '<blur_points_set><best_scale value="0" globalID="0" /><best_scale value="2" globalID="10" /></blur_points_set></curve>\n')
+            '<blur_points_set><best_scale value="0" globalID="0" /><best_scale value="2" globalID="10" /></blur_points_set>'
+            + stops + '</curve>\n')
 
 
 def straight(ax, ay, bx, by):

@@ -223,7 +223,8 @@ def test_far_view_against_brute_force(case, view, api, scenes):
 @pytest.mark.parametrize("R", [1e5, 1e6])
 @pytest.mark.parametrize("name", ["arch.xml", "dust.xml"])
 def test_far_view_adjoints_against_brute_force(name, R, api, scenes):
-    """color_adjoint and blur_adjoint trace with closest_chord: at a far view the tree and the brute force give the same."""
+    """color_adjoint, blur_adjoint and weight_adjoint trace with closest_chord: at a far view the tree and the brute force
+    give the same."""
     import torch
 
     r = scenes.gpu(api, name)
@@ -239,12 +240,15 @@ def test_far_view_adjoints_against_brute_force(name, R, api, scenes):
         left = torch.zeros(d["color_left"].shape, dtype=torch.float64, device="cuda")
         right = torch.zeros(d["color_right"].shape, dtype=torch.float64, device="cuda")
         blur = torch.zeros(d["blur"].shape, dtype=torch.float64, device="cuda")
+        weight = torch.zeros(d["weight"].shape, dtype=torch.float64, device="cuda")
+        degree = torch.zeros(d["weight_degree"].shape, dtype=torch.float64, device="cuda")
         s = torch.cuda.current_stream().cuda_stream
         r.scene.color_adjoint(p, g.data_ptr(), left.data_ptr(), right.data_ptr(), s)
         r.scene.blur_adjoint(p, sg.data_ptr(), blur.data_ptr(), s)
+        r.scene.weight_adjoint(p, g.data_ptr(), sg.data_ptr(), weight.data_ptr(), degree.data_ptr(), s)
         torch.cuda.synchronize()
-        out[trav] = [a.cpu().numpy() for a in (left, right, blur)]
-    assert np.abs(out[0][0]).sum() > 0, "the view sees nothing"
+        out[trav] = [a.cpu().numpy() for a in (left, right, blur, weight, degree)]
+    assert np.abs(out[0][0]).sum() > 0 and np.abs(out[0][4]).sum() > 0, "the view sees nothing"
     for a, b in zip(out[0], out[TRAVERSAL_BRUTE_FORCE]):
         np.testing.assert_allclose(a, b, rtol=1e-9, atol=1e-12)
 
