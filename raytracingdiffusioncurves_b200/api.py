@@ -720,48 +720,75 @@ def fit_stops(d: dict, target, render, adjoint, iterations: int):
     return fitted, residuals
 
 
+class _BandFrame:
+    """The band of `params` as the fits see it, built once per (scene, params, use_blur): forward(**stops) puts the stop
+    arrays given (HostScene.to_numpy() names) on the handle over `d`'s (update_stops) and renders the band, then, with
+    use_blur, blurs it as rdc_render_frame_to_host(use_blur=1) does (the band as a buffer of its own rows, with the render's
+    max_sigma flag); it returns the frame, float32 [rows, W, 4]. transpose(g) is the blur's transpose Bᵀ g with the last
+    forward's blur map (g itself without the blur) and sigma_adjoint(g) the blurred frame's derivative in that map. Device
+    buffers are reused from call to call; `stream` must be torch's current stream."""
+
+    def __init__(self, scene: "Scene", d: dict, params: FrameParams, use_blur: bool, stream: int):
+        import torch
+
+        self.scene, self.params, self.use_blur, self.stream = scene, params, use_blur, stream
+        self.rows, self.w = params.row_end - params.row_begin, params.image_width
+        self.dev = torch.device("cuda", torch.cuda.current_device())
+        self.image = torch.empty((self.rows, self.w, 4), dtype=torch.float32, device=self.dev)
+        self.sigma = torch.empty((self.rows, self.w), dtype=torch.float32, device=self.dev)
+        self.work = dict(d)
+        if use_blur:
+            self.blurred = torch.empty_like(self.image)
+            self.grad_image = torch.empty_like(self.image)
+            self.grad_sigma = torch.empty_like(self.sigma)
+            # the blur's and both derivatives'
+            self.scratch = torch.empty((2 * self.rows * self.w + 1, 4), dtype=torch.float32, device=self.dev)
+            self.flag = torch.zeros((1,), dtype=torch.float32, device=self.dev)
+            self.blur_params = FrameParams.from_buffer_copy(params)
+            self.blur_params.max_sigma = self.flag.data_ptr()
+        scene.reserve(params, False, stream)
+
+    def _blur_args(self):
+        return self.scratch.data_ptr(), self.w, self.rows, 0, self.rows, self.flag.data_ptr(), self.stream
+
+    def forward(self, **stops):
+        self.work.update(stops)
+        self.scene.update_stops(arrays_from_numpy(self.work), self.stream)
+        if not self.use_blur:
+            self.scene.render(self.params, self.image.data_ptr(), self.sigma.data_ptr(), self.stream)
+            return self.image
+        self.flag.zero_()
+        self.scene.render(self.blur_params, self.image.data_ptr(), self.sigma.data_ptr(), self.stream)
+        gaussian_blur(self.blurred.data_ptr(), self.image.data_ptr(), self.sigma.data_ptr(), *self._blur_args())
+        return self.blurred
+
+    def transpose(self, g):
+        if not self.use_blur:
+            return g
+        gaussian_blur_adjoint(self.grad_image.data_ptr(), g.data_ptr(), self.sigma.data_ptr(), *self._blur_args())
+        return self.grad_image
+
+    def sigma_adjoint(self, g):
+        gaussian_blur_sigma_adjoint(self.grad_sigma.data_ptr(), g.data_ptr(), self.image.data_ptr(), self.sigma.data_ptr(),
+                                    *self._blur_args())
+        return self.grad_sigma
+
+
 def _color_operator(scene: "Scene", d: dict, params: FrameParams, use_blur: bool, stream: int):
-    """The (render, adjoint) pair fit_colors hands to fit_stops: render(left, right) puts the colour values on the handle
-    (update_stops) and renders the band of `params`, then, with use_blur, blurs it as rdc_render_frame_to_host(use_blur=1)
-    does (the band as a buffer of its own rows, with the render's max_sigma flag); adjoint(grad) is the blur's transpose with
-    the last render's blur map (colour values never change it), then Scene.color_adjoint. Device buffers are reused from
-    call to call; `stream` must be torch's current stream."""
+    """The (render, adjoint) pair fit_colors hands to fit_stops: render(left, right) is _BandFrame.forward with those colour
+    values; adjoint(grad) is the blur's transpose with the last render's blur map (colour values never change it), then
+    Scene.color_adjoint. `stream` must be torch's current stream."""
     import torch
 
-    rows, w = params.row_end - params.row_begin, params.image_width
-    dev = torch.device("cuda", torch.cuda.current_device())
-    image = torch.empty((rows, w, 4), dtype=torch.float32, device=dev)
-    sigma = torch.empty((rows, w), dtype=torch.float32, device=dev)
-    grad_left = torch.empty(np.asarray(d["color_left"]).shape, dtype=torch.float64, device=dev)
-    grad_right = torch.empty(np.asarray(d["color_right"]).shape, dtype=torch.float64, device=dev)
-    work = dict(d)
-    scene.reserve(params, False, stream)
-    if use_blur:
-        blurred = torch.empty_like(image)
-        grad_image = torch.empty_like(image)
-        scratch = torch.empty((rows * w + 1, 4), dtype=torch.float32, device=dev)  # the blur's and its transpose's
-        flag = torch.zeros((1,), dtype=torch.float32, device=dev)
-        blur_params = FrameParams.from_buffer_copy(params)
-        blur_params.max_sigma = flag.data_ptr()
+    frame = _BandFrame(scene, d, params, use_blur, stream)
+    grad_left = torch.empty(np.asarray(d["color_left"]).shape, dtype=torch.float64, device=frame.dev)
+    grad_right = torch.empty(np.asarray(d["color_right"]).shape, dtype=torch.float64, device=frame.dev)
 
     def render(left, right):
-        work["color_left"], work["color_right"] = left, right
-        scene.update_stops(arrays_from_numpy(work), stream)
-        if not use_blur:
-            scene.render(params, image.data_ptr(), sigma.data_ptr(), stream)
-            return image
-        flag.zero_()
-        scene.render(blur_params, image.data_ptr(), sigma.data_ptr(), stream)
-        gaussian_blur(blurred.data_ptr(), image.data_ptr(), sigma.data_ptr(), scratch.data_ptr(), w, rows, 0, rows, flag.data_ptr(),
-                      stream)
-        return blurred
+        return frame.forward(color_left=left, color_right=right)
 
     def adjoint(g):
-        g = g.contiguous()
-        if use_blur:
-            gaussian_blur_adjoint(grad_image.data_ptr(), g.data_ptr(), sigma.data_ptr(), scratch.data_ptr(), w, rows, 0, rows,
-                                  flag.data_ptr(), stream)
-            g = grad_image
+        g = frame.transpose(g.contiguous())
         scene.color_adjoint(params, g.data_ptr(), grad_left.data_ptr(), grad_right.data_ptr(), stream)
         return grad_left.cpu().numpy(), grad_right.cpu().numpy()
 
@@ -829,6 +856,37 @@ def projected_descent(f_and_grad, x0, lower, iterations: int):
     return x, objectives
 
 
+def _fit_band(frame: _BandFrame, d: dict, target, stops, gradient, x0, lower, iterations: int):
+    """Minimises 1/2 ||frame.forward(**stops(x)) - target||^2 over x >= lower with projected_descent, then puts the fitted
+    stops on the handle. target: float32 [rows, W, 3|4], numpy or torch; pixels NaN in the target or in the start's frame
+    are ignored. gradient(x, g) -> the objective's gradient in x for g, float32 [rows, W, 4], whose RGB holds the residual
+    (.w zero). A trial whose objective is not finite gets no gradient: projected_descent refuses it without reading one.
+    Returns (fitted copy of d, objective of every iteration)."""
+    import torch
+
+    target3 = torch.as_tensor(target, dtype=torch.float32, device=frame.dev)[..., :3].to(torch.float64)
+
+    def frame3(x):
+        return frame.forward(**stops(x))[..., :3].to(torch.float64)
+
+    keep = ~(torch.isnan(frame3(x0)).any(-1) | torch.isnan(target3).any(-1))[..., None]
+    grad_image = torch.zeros_like(frame.image)
+
+    def f_and_grad(x):
+        r = torch.where(keep, frame3(x) - target3, torch.zeros((), dtype=torch.float64, device=frame.dev))
+        f = 0.5 * float((r * r).sum())
+        if not np.isfinite(f):
+            return f, np.full_like(x, np.nan)
+        grad_image[..., :3] = r
+        return f, gradient(x, grad_image)
+
+    x, objectives = projected_descent(f_and_grad, x0, lower, iterations)
+    fitted = {k: (v.copy() if isinstance(v, np.ndarray) else v) for k, v in d.items()}
+    fitted.update(stops(x))
+    frame.scene.update_stops(arrays_from_numpy(fitted), frame.stream)
+    return fitted, objectives
+
+
 def fit_blur(scene: "Scene", d: dict, params: FrameParams, target, iterations: int = 30, stream: int | None = None):
     """Blur stops whose blurred render of `params` comes closest to `target`: minimises 1/2 ||blurred frame - target||^2 over
     the real blur stops (j < n_blur), each >= 0, with the curves, colours, u lists, weights and exponents of `d`
@@ -845,55 +903,21 @@ def fit_blur(scene: "Scene", d: dict, params: FrameParams, target, iterations: i
 
     if stream is None:
         stream = torch.cuda.current_stream().cuda_stream
-    rows, w = params.row_end - params.row_begin, params.image_width
-    dev = torch.device("cuda", torch.cuda.current_device())
+    frame = _BandFrame(scene, d, params, True, stream)
     nb = int(d["n_blur"])
     base = np.asarray(d["blur"], np.float32)
-    image = torch.empty((rows, w, 4), dtype=torch.float32, device=dev)
-    sigma = torch.empty((rows, w), dtype=torch.float32, device=dev)
-    blurred = torch.empty_like(image)
-    grad_image = torch.zeros_like(image)
-    grad_sigma = torch.empty_like(sigma)
-    grad_blur = torch.empty(base.shape, dtype=torch.float64, device=dev)
-    scratch = torch.empty((2 * rows * w + 1, 4), dtype=torch.float32, device=dev)  # the blur's and its derivative's
-    flag = torch.zeros((1,), dtype=torch.float32, device=dev)
-    blur_params = FrameParams.from_buffer_copy(params)
-    blur_params.max_sigma = flag.data_ptr()
-    target3 = torch.as_tensor(target, dtype=torch.float32, device=dev)[..., :3].to(torch.float64)
-    work = dict(d)
-    scene.reserve(params, False, stream)
+    grad_blur = torch.empty(base.shape, dtype=torch.float64, device=frame.dev)
 
     def stops(x):
         b = base.copy()
         b[:nb] = x
-        return b
+        return {"blur": b}
 
-    def frame(x):
-        work["blur"] = stops(x)
-        scene.update_stops(arrays_from_numpy(work), stream)
-        flag.zero_()
-        scene.render(blur_params, image.data_ptr(), sigma.data_ptr(), stream)
-        gaussian_blur(blurred.data_ptr(), image.data_ptr(), sigma.data_ptr(), scratch.data_ptr(), w, rows, 0, rows, flag.data_ptr(),
-                      stream)
-        return blurred[..., :3].to(torch.float64)
+    def gradient(x, g):
+        scene.blur_adjoint(params, frame.sigma_adjoint(g).data_ptr(), grad_blur.data_ptr(), stream)
+        return grad_blur[:nb].cpu().numpy()
 
-    x0 = base[:nb].astype(np.float64)
-    keep = ~(torch.isnan(frame(x0)).any(-1) | torch.isnan(target3).any(-1))[..., None]
-
-    def f_and_grad(x):
-        r = torch.where(keep, frame(x) - target3, torch.zeros((), dtype=torch.float64, device=dev))
-        f = 0.5 * float((r * r).sum())
-        grad_image[..., :3] = r
-        gaussian_blur_sigma_adjoint(grad_sigma.data_ptr(), grad_image.data_ptr(), image.data_ptr(), sigma.data_ptr(),
-                                    scratch.data_ptr(), w, rows, 0, rows, flag.data_ptr(), stream)
-        scene.blur_adjoint(params, grad_sigma.data_ptr(), grad_blur.data_ptr(), stream)
-        return f, grad_blur[:nb].cpu().numpy()
-
-    x, objectives = projected_descent(f_and_grad, x0, np.zeros(nb), iterations)
-    fitted = {k: (v.copy() if isinstance(v, np.ndarray) else v) for k, v in d.items()}
-    fitted["blur"] = stops(x)
-    scene.update_stops(arrays_from_numpy(fitted), stream)
-    return fitted, objectives
+    return _fit_band(frame, d, target, stops, gradient, base[:nb].astype(np.float64), np.zeros(nb), iterations)
 
 
 def weight_unknowns(d: dict):
@@ -941,62 +965,19 @@ def fit_weights(scene: "Scene", d: dict, params: FrameParams, target, iterations
 
     if stream is None:
         stream = torch.cuda.current_stream().cuda_stream
-    rows, w = params.row_end - params.row_begin, params.image_width
-    dev = torch.device("cuda", torch.cuda.current_device())
+    frame = _BandFrame(scene, d, params, use_blur, stream)
     x0, lower, stops, chain = weight_unknowns(d)
-    image = torch.empty((rows, w, 4), dtype=torch.float32, device=dev)
-    sigma = torch.empty((rows, w), dtype=torch.float32, device=dev)
-    grad_image = torch.zeros_like(image)
-    grad_weight = torch.empty(np.asarray(d["weight"]).shape, dtype=torch.float64, device=dev)
-    grad_degree = torch.empty(np.asarray(d["weight_degree"]).shape, dtype=torch.float64, device=dev)
-    if use_blur:
-        blurred = torch.empty_like(image)
-        grad_source = torch.empty_like(image)
-        grad_sigma = torch.empty_like(sigma)
-        scratch = torch.empty((2 * rows * w + 1, 4), dtype=torch.float32, device=dev)  # the blur's and both derivatives'
-        flag = torch.zeros((1,), dtype=torch.float32, device=dev)
-        blur_params = FrameParams.from_buffer_copy(params)
-        blur_params.max_sigma = flag.data_ptr()
-    target3 = torch.as_tensor(target, dtype=torch.float32, device=dev)[..., :3].to(torch.float64)
-    work = dict(d)
-    scene.reserve(params, False, stream)
+    grad_weight = torch.empty(np.asarray(d["weight"]).shape, dtype=torch.float64, device=frame.dev)
+    grad_degree = torch.empty(np.asarray(d["weight_degree"]).shape, dtype=torch.float64, device=frame.dev)
 
-    def frame(x):
-        work["weight"], work["weight_degree"] = stops(x)
-        scene.update_stops(arrays_from_numpy(work), stream)
-        if not use_blur:
-            scene.render(params, image.data_ptr(), sigma.data_ptr(), stream)
-            return image[..., :3].to(torch.float64)
-        flag.zero_()
-        scene.render(blur_params, image.data_ptr(), sigma.data_ptr(), stream)
-        gaussian_blur(blurred.data_ptr(), image.data_ptr(), sigma.data_ptr(), scratch.data_ptr(), w, rows, 0, rows, flag.data_ptr(),
-                      stream)
-        return blurred[..., :3].to(torch.float64)
+    def gradient(x, g):
+        grad_image = frame.transpose(g).data_ptr()
+        grad_sigma = frame.sigma_adjoint(g).data_ptr() if use_blur else 0
+        scene.weight_adjoint(params, grad_image, grad_sigma, grad_weight.data_ptr(), grad_degree.data_ptr(), stream)
+        return chain(x, grad_weight.cpu().numpy(), grad_degree.cpu().numpy())
 
-    keep = ~(torch.isnan(frame(x0)).any(-1) | torch.isnan(target3).any(-1))[..., None]
-
-    def f_and_grad(x):
-        r = torch.where(keep, frame(x) - target3, torch.zeros((), dtype=torch.float64, device=dev))
-        f = 0.5 * float((r * r).sum())
-        if not np.isfinite(f):  # refused by the line search: no gradient needed
-            return f, np.full_like(x, np.nan)
-        grad_image[..., :3] = r
-        if not use_blur:
-            scene.weight_adjoint(params, grad_image.data_ptr(), 0, grad_weight.data_ptr(), grad_degree.data_ptr(), stream)
-        else:
-            gaussian_blur_adjoint(grad_source.data_ptr(), grad_image.data_ptr(), sigma.data_ptr(), scratch.data_ptr(), w, rows, 0,
-                                  rows, flag.data_ptr(), stream)
-            gaussian_blur_sigma_adjoint(grad_sigma.data_ptr(), grad_image.data_ptr(), image.data_ptr(), sigma.data_ptr(),
-                                        scratch.data_ptr(), w, rows, 0, rows, flag.data_ptr(), stream)
-            scene.weight_adjoint(params, grad_source.data_ptr(), grad_sigma.data_ptr(), grad_weight.data_ptr(),
-                                 grad_degree.data_ptr(), stream)
-        return f, chain(x, grad_weight.cpu().numpy(), grad_degree.cpu().numpy())
-
-    x, objectives = projected_descent(f_and_grad, x0, lower, iterations)
-    fitted = {k: (v.copy() if isinstance(v, np.ndarray) else v) for k, v in d.items()}
-    fitted["weight"], fitted["weight_degree"] = stops(x)
-    scene.update_stops(arrays_from_numpy(fitted), stream)
-    return fitted, objectives
+    return _fit_band(frame, d, target, lambda x: dict(zip(("weight", "weight_degree"), stops(x))), gradient, x0, lower,
+                     iterations)
 
 
 def view_pixel_to_scene(params: FrameParams, ix: int, iy: int) -> tuple[float, float]:

@@ -1019,7 +1019,6 @@ int update_stops(rdc_scene* s, const rdc_scene_arrays& a, cudaStream_t stream) {
   }
   if (int rc = check_stops(a, "update stops")) return rc;
   const StopLayout L = stop_layout(a);
-  if (!s->launched) RDC_CUDA(cudaEventCreateWithFlags(&s->launched, cudaEventDisableTiming));
   const bool grow = L.bytes > s->stops_capacity;
   const size_t capacity = grow ? L.bytes : s->stops_capacity;
   if (s->staging_capacity < capacity) {  // the handle's first update, or lists larger than any it has held
@@ -1061,7 +1060,7 @@ int update_stops(rdc_scene* s, const rdc_scene_arrays& a, cudaStream_t stream) {
   }
   pack_stops(a, L, s->staging);
   // like a launch: the device work waits for the handle's previous launch or update, whatever stream that was on
-  if (s->launched_any && s->launched_on != stream) RDC_CUDA(cudaStreamWaitEvent(stream, s->launched, 0));
+  if (int rc = wait_previous_launch(s, stream)) return rc;
   RDC_CUDA(cudaMemcpyAsync(s->stops, s->staging, L.bytes, cudaMemcpyHostToDevice, stream));
   RDC_CUDA(cudaEventRecord(s->staged, stream));
   point_stops(s->dev, s->stops, L);
@@ -1070,6 +1069,16 @@ int update_stops(rdc_scene* s, const rdc_scene_arrays& a, cudaStream_t stream) {
   s->weight_stops = (uint32_t)L.len[3];
   s->degree_stops = (uint32_t)L.len[4];
   if (int rc = launch_stop_tables(s, stream)) return rc;
+  return record_launch(s, stream);
+}
+
+int wait_previous_launch(rdc_scene* s, cudaStream_t stream) {
+  if (!s->launched) RDC_CUDA(cudaEventCreateWithFlags(&s->launched, cudaEventDisableTiming));
+  if (s->launched_any && s->launched_on != stream) RDC_CUDA(cudaStreamWaitEvent(stream, s->launched, 0));
+  return 0;
+}
+
+int record_launch(rdc_scene* s, cudaStream_t stream) {
   RDC_CUDA(cudaEventRecord(s->launched, stream));
   s->launched_on = stream;
   s->launched_any = true;

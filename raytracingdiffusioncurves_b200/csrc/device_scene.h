@@ -147,6 +147,11 @@ void destroy_scene(rdc_scene* s);
 int download_chords(const rdc_scene* s, float* geom, uint32_t* ids);
 int update_stops(rdc_scene* s, const rdc_scene_arrays& a, cudaStream_t stream);
 int download_stop_tables(const rdc_scene* s, void* seg_walk, void* chord_walk, void* chord_records);
+// The order of the handle's launches and updates: work on another stream than the handle's previous work waits for it
+// on the device (wait_previous_launch, which creates the event on first use), and each one is recorded after it is
+// enqueued (record_launch).
+int wait_previous_launch(rdc_scene* s, cudaStream_t stream);
+int record_launch(rdc_scene* s, cudaStream_t stream);
 // render.cu
 int render(rdc_scene* s, const rdc_frame_params& p, float4* image, float* blur_map, cudaStream_t stream, uint32_t n_targets = 0,
            float* const* target_images = nullptr, float* const* target_blur_maps = nullptr);

@@ -236,8 +236,7 @@ int check_max_distance(float max_distance, const char* who) {
 
 // like a launch: behind the handle's previous launch or update, whatever stream that was on; the next launch waits for it
 int launch(rdc_scene* s, PickArgs& a, bool frame, size_t threads, cudaStream_t stream) {
-  if (!s->launched) RDC_CUDA(cudaEventCreateWithFlags(&s->launched, cudaEventDisableTiming));
-  if (s->launched_any && s->launched_on != stream) RDC_CUDA(cudaStreamWaitEvent(stream, s->launched, 0));
+  if (int rc = wait_previous_launch(s, stream)) return rc;
   a.sc = s->dev;
   const unsigned grid = (unsigned)((threads + kPickBlock - 1) / kPickBlock);
   if (frame) {
@@ -248,10 +247,7 @@ int launch(rdc_scene* s, PickArgs& a, bool frame, size_t threads, cudaStream_t s
     else k_pick<false, false><<<grid, kPickBlock, 0, stream>>>(a);
   }
   RDC_CUDA(cudaGetLastError());
-  RDC_CUDA(cudaEventRecord(s->launched, stream));
-  s->launched_on = stream;
-  s->launched_any = true;
-  return 0;
+  return record_launch(s, stream);
 }
 
 }  // namespace

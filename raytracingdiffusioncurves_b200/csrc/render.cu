@@ -422,21 +422,60 @@ __device__ __forceinline__ void load_control_points(const DevScene& sc, uint32_t
   v[3] = {b.z, b.w};
 }
 
-__device__ __forceinline__ float scalar_stop(const DevStops& st, uint32_t first, uint32_t end, float cu) {
-  float ratio;
-  int ind = rdc_interp_from(first, end, cu, st.u, &ratio);
-  return rdc_lerp_stop(__ldg(st.value + ind), __ldg(st.value + ind + 1), ratio);
+// A hit's walk data: the segment and u from the run's ids, the walk ranges of the segment (SegWalk: the stop walks start
+// where the segment starts) and, finer, where this chord starts (chord_walk: the walks then rarely take a step); cu = u + ordinal.
+struct HitWalks {
+  uint32_t seg;
+  float u, cu;
+  uint4 wc, ws, wd, cw, cw2;
+};
+
+__device__ __forceinline__ HitWalks hit_walks(const DevScene& sc, const Hit& h) {
+  HitWalks w;
+  const uint4 id = __ldg(sc.run_ids + h.leaf);  // first chord id, segment, k of the first chord, K
+  w.seg = id.y;
+  w.u = rdc_hit_u((int)id.z + h.j, (int)id.w, h.s);
+  const uint4* wp = reinterpret_cast<const uint4*>(sc.seg_walk + w.seg);
+  w.wc = __ldg(wp), w.ws = __ldg(wp + 1), w.wd = __ldg(wp + 2);
+  w.cw = __ldg(sc.chord_walk + 2 * (size_t)h.id), w.cw2 = __ldg(sc.chord_walk + 2 * (size_t)h.id + 1);
+  w.cu = w.u + w.wd.w;
+  return w;
 }
 
-// [first,end) selects the walk range, `us`/`rgb` the arrays (the portal filter mixes families, DeviceCode.cu:297)
-__device__ __forceinline__ void colour_stop(uint32_t first, uint32_t end, const float* us, const float4* rgb, float cu,
-                                            float& r, float& g, float& b) {
-  float ratio;
+// The stop cu interpolates from on a walk over [first,end) of a family's u list, the ratio, and the lerped value
+struct ScalarStop {
+  int ind;
+  float ratio, value;
+};
+
+__device__ __forceinline__ ScalarStop stop_walk(const DevStops& st, uint32_t first, uint32_t end, float cu) {
+  ScalarStop s;
+  s.ind = rdc_interp_from(first, end, cu, st.u, &s.ratio);
+  s.value = rdc_lerp_stop(__ldg(st.value + s.ind), __ldg(st.value + s.ind + 1), s.ratio);
+  return s;
+}
+
+__device__ __forceinline__ float scalar_stop(const DevStops& st, uint32_t first, uint32_t end, float cu) {
+  return stop_walk(st, first, end, cu).value;
+}
+
+// [first,end) selects the walk range, `us`/`rgb` the arrays (the portal filter mixes families, DeviceCode.cu:297); returns
+// the index of the stop cu interpolates from
+__device__ __forceinline__ int colour_stop(uint32_t first, uint32_t end, const float* us, const float4* rgb, float cu,
+                                          float& ratio, float& r, float& g, float& b) {
   int ind = rdc_interp_from(first, end, cu, us, &ratio);
   float4 c0 = __ldg(rgb + ind), c1 = __ldg(rgb + ind + 1);
   r = rdc_lerp_color(c0.x, c1.x, ratio);
   g = rdc_lerp_color(c0.y, c1.y, ratio);
   b = rdc_lerp_color(c0.z, c1.z, ratio);
+  return ind;
+}
+
+// The colour walk of a terminal hit: the right family's for a ray on the curve's right, the left one's otherwise
+__device__ __forceinline__ int terminal_colour(const DevScene& sc, const HitWalks& w, bool right, float& ratio, float& r, float& g,
+                                               float& b) {
+  if (right) return colour_stop(w.cw.y, w.wc.w, sc.color_right.u, sc.color_right.rgb, w.cu, ratio, r, g, b);
+  else return colour_stop(w.cw.x, w.wc.y, sc.color_left.u, sc.color_left.rgb, w.cu, ratio, r, g, b);
 }
 
 struct Sample {
@@ -485,29 +524,22 @@ __device__ __forceinline__ Sample trace_from(const RenderArgs& a, const Accel& a
         return out;
       }
     }
-    const uint4 id = __ldg(sc.run_ids + h.leaf);  // first chord id, segment, k of the first chord, K
-    const uint32_t seg = id.y;
-    const float u = rdc_hit_u((int)id.z + h.j, (int)id.w, h.s);
-    // walk ranges of this segment (SegWalk): the stop walks start where the segment starts
-    const uint4* wp = reinterpret_cast<const uint4*>(sc.seg_walk + seg);
-    const uint4 wc = __ldg(wp), ws = __ldg(wp + 1), wd = __ldg(wp + 2);
-    // ... and, finer, where this chord starts (chord_walk): the walks then rarely take a step
-    const uint4 cw = __ldg(sc.chord_walk + 2 * (size_t)h.id), cw2 = __ldg(sc.chord_walk + 2 * (size_t)h.id + 1);
-    const uint32_t curve = wd.z, ordinal = wd.w;
-    const float cu = u + ordinal;
-    const float blur_here = scalar_stop(sc.blur, cw.z, ws.y, cu);
-    const float wm = scalar_stop(sc.weight, cw.w, ws.w, cu);
-    const float e = scalar_stop(sc.weight_degree, cw2.x, wd.y, cu);
+    const HitWalks hw = hit_walks(sc, h);
+    const uint4* wp = reinterpret_cast<const uint4*>(sc.seg_walk + hw.seg);  // the portal filter's walk range: wp[3]
+    const float u = hw.u, cu = hw.cu;
+    const float blur_here = scalar_stop(sc.blur, hw.cw.z, hw.ws.y, cu);
+    const float wm = scalar_stop(sc.weight, hw.cw.w, hw.ws.w, cu);
+    const float e = scalar_stop(sc.weight_degree, hw.cw2.x, hw.wd.y, cu);
     const float w_here = wm * rdc_weight_falloff(h.t, e);
     rdc_f2 v[4];
-    load_control_points(sc, seg, v);
+    load_control_points(sc, hw.seg, v);
     const bool right = rdc_is_ray_right(u, dx, dy, v[0], v[1], v[2], v[3], a.orzan != 0);
 
     if (PORTALS) {
-      const int target_curve = __ldg(sc.curve_connect + curve);
+      const int target_curve = __ldg(sc.curve_connect + hw.wd.z);
       if (target_curve >= 0) {
         if (++depth > a.max_depth) return out;  // depth cap: regarded as a miss (:313-320)
-        const uint32_t tseg = __ldg(sc.curve_map_inverse + target_curve) + ordinal;
+        const uint32_t tseg = __ldg(sc.curve_map_inverse + target_curve) + hw.wd.w;
         rdc_f2 tv[4];
         load_control_points(sc, tseg, tv);
         rdc_f2 o2 = rdc_spline_point(u, tv[0], tv[1], tv[2], tv[3]);
@@ -521,11 +553,11 @@ __device__ __forceinline__ Sample trace_from(const RenderArgs& a, const Accel& a
         m.x /= ml; m.y /= ml;
         float ndx = m.x * rc - m.y * rs;
         float ndy = m.y * rc + m.x * rs;
-        float fr, fg, fb;
-        if (right) colour_stop(cw.y, wc.w, sc.color_right.u, sc.color_right.rgb, cu, fr, fg, fb);
+        float fratio, fr, fg, fb;
+        if (right) colour_stop(hw.cw.y, hw.wc.w, sc.color_right.u, sc.color_right.rgb, cu, fratio, fr, fg, fb);
         else {  // right list's range on the left arrays (:297)
           const uint4 wq = __ldg(wp + 3);
-          colour_stop(cw2.y, wq.y, sc.color_left.u, sc.color_left.rgb, cu, fr, fg, fb);
+          colour_stop(hw.cw2.y, wq.y, sc.color_left.u, sc.color_left.rgb, cu, fratio, fr, fg, fb);
         }
         Fr *= fr; Fg *= fg; Fb *= fb;
         Bp *= blur_here;
@@ -540,9 +572,8 @@ __device__ __forceinline__ Sample trace_from(const RenderArgs& a, const Accel& a
         continue;
       }
     }
-    float r, g, b;
-    if (right) colour_stop(cw.y, wc.w, sc.color_right.u, sc.color_right.rgb, cu, r, g, b);
-    else colour_stop(cw.x, wc.y, sc.color_left.u, sc.color_left.rgb, cu, r, g, b);
+    float ratio, r, g, b;
+    terminal_colour(sc, hw, right, ratio, r, g, b);
     if (PORTALS && depth > 0) {
       out.r = Fr * r; out.g = Fg * g; out.b = Fb * b;
       out.blur = Bp * blur_here;
@@ -1741,10 +1772,9 @@ int prepare_variant(rdc_scene* s, const LaunchPlan& L, RenderKernel* out) {
   return 0;
 }
 
-// Scratch a launch of this plan needs, and the handle's launch event; grows only. Allocating means a device-wide synchronisation (cudaFree), which
+// Scratch a launch of this plan needs; grows only. Allocating means a device-wide synchronisation (cudaFree), which
 // is why rdc_scene_reserve exists.
 int ensure_capacity(rdc_scene* s, const LaunchPlan& L, cudaStream_t stream) {
-  if (!s->launched) RDC_CUDA(cudaEventCreateWithFlags(&s->launched, cudaEventDisableTiming));
   if ((uint32_t)L.n_iter > s->base_dirs_capacity) {
     float2* fresh = nullptr;
     RDC_CUDA(cudaMalloc(&fresh, (size_t)L.n_iter * sizeof(float2)));
@@ -1800,13 +1830,12 @@ enum StopFamily : int { kColourStops, kBlurStops, kWeightStops };
 
 constexpr uint32_t kNoStop = 0xFFFFFFFFu;
 
-// Primary ray i of a pixel and its closest hit, with the walk ranges of the hit's segment and chord. False for a miss and
-// for a hit on a portal curve (max_trace_depth 0: contributes nothing).
+// Primary ray i of a pixel, its closest hit and the hit's walk data. False for a miss and for a hit on a portal curve
+// (max_trace_depth 0: contributes nothing).
 struct AdjointHit {
   Hit h;
-  float dx, dy, u, cu;
-  uint32_t seg;
-  uint4 wc, ws, wd, cw, cw2;
+  float dx, dy;
+  HitWalks w;
 };
 
 __device__ __forceinline__ bool adjoint_hit(const AdjointArgs& aa, const Accel& ac, const Pixel& px, int i, bool small_angle,
@@ -1818,79 +1847,59 @@ __device__ __forceinline__ bool adjoint_hit(const AdjointArgs& aa, const Accel& 
   gen_ray(a, px.pixel, px.base_x, px.base_y, i, small_angle, ox, oy, r.dx, r.dy);
   r.h = closest_chord<false, false, false>(ac, a.brute != 0, ox, oy, r.dx, r.dy, true, 1u, 0u, __int_as_float(0x7f800000), cnt);
   if (r.h.leaf < 0) return false;
-  const uint4 id = __ldg(sc.run_ids + r.h.leaf);
-  r.seg = id.y;
-  const uint4* wp = reinterpret_cast<const uint4*>(sc.seg_walk + r.seg);
-  r.wc = __ldg(wp), r.ws = __ldg(wp + 1), r.wd = __ldg(wp + 2);
-  if (aa.portals && __ldg(sc.curve_connect + r.wd.z) >= 0) return false;
-  r.u = rdc_hit_u((int)id.z + r.h.j, (int)id.w, r.h.s);
-  r.cw = __ldg(sc.chord_walk + 2 * (size_t)r.h.id), r.cw2 = __ldg(sc.chord_walk + 2 * (size_t)r.h.id + 1);
-  r.cu = r.u + r.wd.w;
-  return true;
+  r.w = hit_walks(sc, r.h);
+  return !(aa.portals && __ldg(sc.curve_connect + r.w.wd.z) >= 0);
 }
 
-// One primary ray of the adjoint: its weight w_i (0 for a miss or a portal hit) and, with KEY, the stop of FAMILY it
-// interpolates from (colour: key = ind << 1 | right; blur: key = ind) and the ratio rho. Same operands and operations as
-// trace_from's terminal walk path.
-template <int FAMILY, bool KEY>
-__device__ __forceinline__ float adjoint_ray(const AdjointArgs& aa, const Accel& ac, const Pixel& px, int i, bool small_angle,
-                                             uint32_t& key, float& ratio) {
-  const DevScene& sc = aa.r.sc;
-  AdjointHit r;
-  key = kNoStop;
-  if (!adjoint_hit(aa, ac, px, i, small_angle, r)) return 0.0f;
-  const float wm = scalar_stop(sc.weight, r.cw.w, r.ws.w, r.cu);
-  const float e = scalar_stop(sc.weight_degree, r.cw2.x, r.wd.y, r.cu);
-  const float w = wm * rdc_weight_falloff(r.h.t, e);
-  if (KEY && FAMILY == kColourStops) {
-    rdc_f2 v[4];
-    load_control_points(sc, r.seg, v);
-    const bool right = rdc_is_ray_right(r.u, r.dx, r.dy, v[0], v[1], v[2], v[3], aa.r.orzan != 0);
-    const int ind = right ? rdc_interp_from(r.cw.y, r.wc.w, r.cu, sc.color_right.u, &ratio)
-                          : rdc_interp_from(r.cw.x, r.wc.y, r.cu, sc.color_left.u, &ratio);
-    key = ((uint32_t)ind << 1) | (right ? 1u : 0u);
-  }
-  if (KEY && FAMILY == kBlurStops) key = (uint32_t)rdc_interp_from(r.cw.z, r.ws.y, r.cu, sc.blur.u, &ratio);
-  return w;
-}
-
-// One primary ray of the weight adjoint: w_i and s_i = <G, c_i> + g_sigma b_i (g.w = g_sigma) with the render's weight,
-// side, colour and blur walks (all 0 for a miss or a portal hit); with KEY also the weight and exponent stops the ray
-// interpolates from, their ratios, f_i = t_i^-e_i and t_i.
-struct WeightRay {
-  float w, f, t, rw, re;
-  double s;
-  uint32_t iw, ie;
+// One primary ray of the adjoint, shaded with trace_from's terminal walks (hit_walks, stop_walk, terminal_colour); all
+// zero for a miss or a portal hit. w = w_i; with KEY, the stop of FAMILY the ray interpolates from and the ratio rho
+// (colour: key = ind << 1 | right; blur: key = ind). For the weights also s = <G, c_i> + g_sigma b_i (g.w = g_sigma) and,
+// with KEY, the weight and exponent stops (iw, ie), their ratios, f = t^-e and t.
+struct AdjointRay {
+  float w = 0.0f;
+  uint32_t key = kNoStop;
+  float ratio = 0.0f;
+  float f = 0.0f, t = 0.0f, rw = 0.0f, re = 0.0f;
+  double s = 0.0;
+  uint32_t iw = kNoStop, ie = kNoStop;
 };
 
-template <bool KEY>
-__device__ __forceinline__ WeightRay weight_ray(const AdjointArgs& aa, const Accel& ac, const Pixel& px, int i, bool small_angle,
-                                                float4 g) {
+template <int FAMILY, bool KEY>
+__device__ __forceinline__ AdjointRay adjoint_ray(const AdjointArgs& aa, const Accel& ac, const Pixel& px, int i, bool small_angle,
+                                                  float4 g) {
   const DevScene& sc = aa.r.sc;
-  WeightRay out{0.0f, 0.0f, 0.0f, 0.0f, 0.0f, 0.0, kNoStop, kNoStop};
+  AdjointRay out;
   AdjointHit r;
   if (!adjoint_hit(aa, ac, px, i, small_angle, r)) return out;
-  // scalar_stop's walks, with the index kept
-  float rw, re;
-  const int iw = rdc_interp_from(r.cw.w, r.ws.w, r.cu, sc.weight.u, &rw);
-  const int ie = rdc_interp_from(r.cw2.x, r.wd.y, r.cu, sc.weight_degree.u, &re);
-  const float wm = rdc_lerp_stop(__ldg(sc.weight.value + iw), __ldg(sc.weight.value + iw + 1), rw);
-  const float e = rdc_lerp_stop(__ldg(sc.weight_degree.value + ie), __ldg(sc.weight_degree.value + ie + 1), re);
-  const float f = rdc_weight_falloff(r.h.t, e);
-  out.w = wm * f;
-  rdc_f2 v[4];
-  load_control_points(sc, r.seg, v);
-  const bool right = rdc_is_ray_right(r.u, r.dx, r.dy, v[0], v[1], v[2], v[3], aa.r.orzan != 0);
-  float cr, cg, cb;
-  if (right) colour_stop(r.cw.y, r.wc.w, sc.color_right.u, sc.color_right.rgb, r.cu, cr, cg, cb);
-  else colour_stop(r.cw.x, r.wc.y, sc.color_left.u, sc.color_left.rgb, r.cu, cr, cg, cb);
-  const float blur = scalar_stop(sc.blur, r.cw.z, r.ws.y, r.cu);
-  // a zero gradient component adds nothing, whatever the stop value
-  out.s = (g.x != 0.0f ? (double)g.x * cr : 0.0) + (g.y != 0.0f ? (double)g.y * cg : 0.0) +
-          (g.z != 0.0f ? (double)g.z * cb : 0.0) + (g.w != 0.0f ? (double)g.w * blur : 0.0);
-  if (KEY) {
-    out.f = f, out.t = r.h.t, out.rw = rw, out.re = re;
-    out.iw = (uint32_t)iw, out.ie = (uint32_t)ie;
+  const HitWalks& hw = r.w;
+  const ScalarStop wm = stop_walk(sc.weight, hw.cw.w, hw.ws.w, hw.cu);
+  const ScalarStop e = stop_walk(sc.weight_degree, hw.cw2.x, hw.wd.y, hw.cu);
+  const float f = rdc_weight_falloff(r.h.t, e.value);
+  out.w = wm.value * f;
+  if constexpr (FAMILY == kWeightStops || (KEY && FAMILY == kColourStops)) {
+    rdc_f2 v[4];
+    load_control_points(sc, hw.seg, v);
+    const bool right = rdc_is_ray_right(hw.u, r.dx, r.dy, v[0], v[1], v[2], v[3], aa.r.orzan != 0);
+    float ratio, cr, cg, cb;
+    const int ind = terminal_colour(sc, hw, right, ratio, cr, cg, cb);
+    if constexpr (FAMILY == kColourStops) {
+      out.key = ((uint32_t)ind << 1) | (right ? 1u : 0u);
+      out.ratio = ratio;
+    } else {
+      const float blur = scalar_stop(sc.blur, hw.cw.z, hw.ws.y, hw.cu);
+      // a zero gradient component adds nothing, whatever the stop value
+      out.s = (g.x != 0.0f ? (double)g.x * cr : 0.0) + (g.y != 0.0f ? (double)g.y * cg : 0.0) +
+              (g.z != 0.0f ? (double)g.z * cb : 0.0) + (g.w != 0.0f ? (double)g.w * blur : 0.0);
+      if (KEY) {
+        out.f = f, out.t = r.h.t, out.rw = wm.ratio, out.re = e.ratio;
+        out.iw = (uint32_t)wm.ind, out.ie = (uint32_t)e.ind;
+      }
+    }
+  }
+  if constexpr (KEY && FAMILY == kBlurStops) {
+    const ScalarStop b = stop_walk(sc.blur, hw.cw.z, hw.ws.y, hw.cu);
+    out.key = (uint32_t)b.ind;
+    out.ratio = b.ratio;
   }
   return out;
 }
@@ -1946,9 +1955,9 @@ __global__ void __launch_bounds__(kBlock) k_stop_adjoint(const AdjointArgs aa) {
   const Pixel px = tile_pixel(a, tile, aa.tiles_x, lane);
   float4 g = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
   if (px.valid) {
-    if (kColour) {
+    if constexpr (kColour) {
       g = __ldg(aa.grad + px.local);
-    } else if (kWeight) {  // g.w = dL/dsigma; a null gradient is zero
+    } else if constexpr (kWeight) {  // g.w = dL/dsigma; a null gradient is zero
       if (aa.grad) g = __ldg(aa.grad + px.local);
       g.w = aa.sigma_grad ? __ldg(aa.sigma_grad + px.local) : 0.0f;
     } else {
@@ -1968,8 +1977,6 @@ __global__ void __launch_bounds__(kBlock) k_stop_adjoint(const AdjointArgs aa) {
     if (rel < 0) rel += n;
     return rel <= cull_span;
   };
-  uint32_t key = kNoStop;
-  float ratio = 0.0f;
   // pass 1: W = sum of the weights, in fp32 and in ray order like PixelSums::add
   float W = 0.0f;
   double W64 = 0.0, WS = 0.0;  // weights: W and sum_i w_i s_i in fp64
@@ -1977,27 +1984,26 @@ __global__ void __launch_bounds__(kBlock) k_stop_adjoint(const AdjointArgs aa) {
 #pragma unroll 1
     for (int i = 0; i < n; ++i) {
       if (!reaches(i)) continue;
+      const AdjointRay r = adjoint_ray<FAMILY, false>(aa, ac, px, i, small_angle, g);
+      W += r.w;
       if constexpr (kWeight) {
-        const WeightRay r = weight_ray<false>(aa, ac, px, i, small_angle, g);
-        W += r.w;
         W64 += (double)r.w;
         WS += (double)r.w * r.s;
-      } else {
-        W += adjoint_ray<FAMILY, false>(aa, ac, px, i, small_angle, key, ratio);
       }
     }
   }
   live = live && W != 0.0f;  // W == 0: the render writes NaN, the pixel is outside the image's linear map
-  if constexpr (kWeight) {
-    // K and 1/W from the fp64 sums: sum_i w_i (s_i - K) then vanishes to fp64 rounding, so the weights' gradient keeps the
-    // frame's invariance to scaling every weight
-    const double inv_w = live ? 1.0 / W64 : 0.0, K = WS * inv_w;
+  // weights: K and 1/W from the fp64 sums: sum_i w_i (s_i - K) then vanishes to fp64 rounding, so the weights' gradient
+  // keeps the frame's invariance to scaling every weight
+  const double inv_w = live ? (kWeight ? 1.0 / W64 : 1.0 / (double)W) : 0.0, K = WS * inv_w;
+  // pass 2
 #pragma unroll 1
-    for (int i = 0; i < n; ++i) {
-      const bool on = live && reaches(i);
-      if (!__any_sync(0xFFFFFFFFu, on)) continue;
-      WeightRay r{0.0f, 0.0f, 0.0f, 0.0f, 0.0f, 0.0, kNoStop, kNoStop};
-      if (on) r = weight_ray<true>(aa, ac, px, i, small_angle, g);
+  for (int i = 0; i < n; ++i) {
+    const bool on = live && reaches(i);
+    if (!__any_sync(0xFFFFFFFFu, on)) continue;
+    AdjointRay r;
+    if (on) r = adjoint_ray<FAMILY, true>(aa, ac, px, i, small_angle, g);
+    if constexpr (kWeight) {
       const double q = r.iw == kNoStop ? 0.0 : (r.s - K) * inv_w;
       const double fw = (double)r.f * q, de = r.iw == kNoStop ? 0.0 : -(double)r.w * log((double)r.t) * q;
       scatter_groups<2>(
@@ -2008,18 +2014,8 @@ __global__ void __launch_bounds__(kBlock) k_stop_adjoint(const AdjointArgs aa) {
           lane, r.ie,
           [&](double* v, bool mine) { v[0] = mine ? de * (double)(1.0f - r.re) : 0.0, v[1] = mine ? de * (double)r.re : 0.0; },
           [&](uint32_t k) { return aa.degree + k; });
-    }
-  } else {
-    const double inv_w = live ? 1.0 / (double)W : 0.0;
-    // pass 2
-#pragma unroll 1
-    for (int i = 0; i < n; ++i) {
-      const bool on = live && reaches(i);
-      if (!__any_sync(0xFFFFFFFFu, on)) continue;
-      key = kNoStop;
-      float w = 0.0f;
-      if (on) w = adjoint_ray<FAMILY, true>(aa, ac, px, i, small_angle, key, ratio);
-      const double f = (double)w * inv_w, f1 = f * (double)ratio, f0 = f * (double)(1.0f - ratio);
+    } else {
+      const double f = (double)r.w * inv_w, f1 = f * (double)r.ratio, f0 = f * (double)(1.0f - r.ratio);
       const double gx = g.x, gy = g.y, gz = g.z;
       auto terms = [&](double* v, bool mine) {
         if constexpr (kColour) {
@@ -2029,20 +2025,41 @@ __global__ void __launch_bounds__(kBlock) k_stop_adjoint(const AdjointArgs aa) {
           v[0] = mine ? gx * f0 : 0.0, v[1] = mine ? gx * f1 : 0.0;
         }
       };
-      scatter_groups<kTerms>(lane, key, terms, [&](uint32_t k) {
+      scatter_groups<kTerms>(lane, r.key, terms, [&](uint32_t k) {
         return kColour ? ((k & 1u) ? aa.right : aa.left) + 3 * (size_t)(k >> 1) : aa.blur + k;
       });
     }
   }
 }
 
-// The table of base directions for the launch's rays per pixel, after ensure_capacity and the wait for the previous launch
-int ensure_base_dirs(rdc_scene* s, const LaunchPlan& L, const rdc_frame_params& p, cudaStream_t stream) {
+// The fields of RenderArgs that describe the view, which the render and the adjoints share: the table of base directions
+// for the launch's rays per pixel (made after ensure_capacity and the wait for the previous launch), the scene with the
+// launch's widened boxes, the frame's size and band, the rays, the camera and the traversal.
+int view_args(rdc_scene* s, const rdc_frame_params& p, int n_iter, cudaStream_t stream, RenderArgs& a) {
   if (s->base_dirs_n != p.number_of_rays_per_pixel) {
-    k_base_dirs<<<1, 32, 0, stream>>>(s->base_dirs, L.n_iter, 2 / p.number_of_rays_per_pixel);
+    k_base_dirs<<<1, 32, 0, stream>>>(s->base_dirs, n_iter, 2 / p.number_of_rays_per_pixel);
     RDC_CUDA(cudaGetLastError());
     s->base_dirs_n = p.number_of_rays_per_pixel;
   }
+  if (int rc = widened_boxes(s, slab_widening(s, p), stream, &a.sc)) return rc;
+  a.base_dirs = s->base_dirs;
+  a.width = p.image_width;
+  a.height = p.image_height;
+  a.row_begin = p.row_begin;
+  a.row_end = p.row_end;
+  a.n_iter = n_iter;
+  a.n_rays = p.number_of_rays_per_pixel;
+  a.two_over_n = 2 / p.number_of_rays_per_pixel;
+  a.zoom = p.zoom_factor;
+  a.off_x = p.offset_x;
+  a.off_y = p.offset_y;
+  a.frame = p.frame;
+  a.seed = p.seed;
+  a.orzan = p.use_diffusion_curve_save;
+  a.use_aa = p.use_aa;
+  a.max_depth = p.max_trace_depth;
+  a.brute = p.traversal == RDC_TRAVERSAL_BRUTE_FORCE;
+  a.cull = p.traversal == RDC_TRAVERSAL_LBVH;  // the brute-force kernel really tests every ray against every chord
   return 0;
 }
 
@@ -2114,13 +2131,11 @@ int render(rdc_scene* s, const rdc_frame_params& p, float4* image, float* blur_m
   const LaunchPlan L = plan_launch(s, p);
   if (L.local_rows == 0) return 0;
   if (int rc = ensure_capacity(s, L, stream)) return rc;
-  // One launch at a time per handle (shared work counters, partial sums, base directions): a launch on another
-  // stream waits — on the device — for the handle's previous one.
-  if (s->launched_any && s->launched_on != stream) RDC_CUDA(cudaStreamWaitEvent(stream, s->launched, 0));
-  if (int rc = ensure_base_dirs(s, L, p, stream)) return rc;
+  // One launch at a time per handle (shared work counters, partial sums, base directions)
+  if (int rc = wait_previous_launch(s, stream)) return rc;
 
   RenderArgs a{};
-  if (int rc = widened_boxes(s, slab_widening(s, p), stream, &a.sc)) return rc;
+  if (int rc = view_args(s, p, L.n_iter, stream, a)) return rc;
   a.image = image;
   a.blur_map = blur_map;
   a.n_targets = n_targets;
@@ -2132,25 +2147,8 @@ int render(rdc_scene* s, const rdc_frame_params& p, float4* image, float* blur_m
   a.hit_ids = p.hit_ids;
   a.max_sigma = p.max_sigma;
   a.stats = p.stats;
-  a.width = p.image_width;
-  a.height = p.image_height;
-  a.row_begin = p.row_begin;
-  a.row_end = p.row_end;
   a.strip_stride = L.strip_stride;
   a.strip_offset = L.strip_offset;
-  a.n_iter = L.n_iter;
-  a.n_rays = p.number_of_rays_per_pixel;
-  a.two_over_n = 2 / p.number_of_rays_per_pixel;
-  a.zoom = p.zoom_factor;
-  a.off_x = p.offset_x;
-  a.off_y = p.offset_y;
-  a.frame = p.frame;
-  a.seed = p.seed;
-  a.orzan = p.use_diffusion_curve_save;
-  a.use_aa = p.use_aa;
-  a.max_depth = p.max_trace_depth;
-  a.brute = p.traversal == RDC_TRAVERSAL_BRUTE_FORCE;
-  a.cull = p.traversal == RDC_TRAVERSAL_LBVH;  // the brute-force kernel really tests every ray against every chord
   a.local_rows = L.local_rows;
   a.row_skew = L.row_skew;
   a.local_r0 = L.local_r0;
@@ -2183,10 +2181,7 @@ int render(rdc_scene* s, const rdc_frame_params& p, float4* image, float* blur_m
   RDC_CUDA(cudaMemsetAsync(s->work_counters, 0, 2 * sizeof(unsigned int), stream));
   kernel<<<grid, kBlock, L.dyn, stream>>>(a);
   RDC_CUDA(cudaGetLastError());
-  RDC_CUDA(cudaEventRecord(s->launched, stream));
-  s->launched_on = stream;
-  s->launched_any = true;
-  return 0;
+  return record_launch(s, stream);
 }
 
 namespace {
@@ -2216,7 +2211,7 @@ int stop_adjoint(rdc_scene* s, const rdc_frame_params& p, AdjointArgs aa, const 
   LaunchPlan L;  // one unit per tile: only the table of base directions is needed
   L.n_iter = (int)ceilf(p.number_of_rays_per_pixel);
   if (int rc = ensure_capacity(s, L, stream)) return rc;
-  if (s->launched_any && s->launched_on != stream) RDC_CUDA(cudaStreamWaitEvent(stream, s->launched, 0));
+  if (int rc = wait_previous_launch(s, stream)) return rc;
   if (FAMILY == kColourStops) {
     const size_t bytes = 3 * (size_t)s->colour_stops * sizeof(double);
     RDC_CUDA(cudaMemsetAsync(aa.left, 0, bytes, stream));
@@ -2227,42 +2222,20 @@ int stop_adjoint(rdc_scene* s, const rdc_frame_params& p, AdjointArgs aa, const 
     RDC_CUDA(cudaMemsetAsync(aa.weight, 0, (size_t)s->weight_stops * sizeof(double), stream));
     RDC_CUDA(cudaMemsetAsync(aa.degree, 0, (size_t)s->degree_stops * sizeof(double), stream));
   }
-  if (int rc = ensure_base_dirs(s, L, p, stream)) return rc;
   RenderArgs& a = aa.r;
-  if (int rc = widened_boxes(s, slab_widening(s, p), stream, &a.sc)) return rc;
-  a.base_dirs = s->base_dirs;
-  a.width = p.image_width;
-  a.height = p.image_height;
-  a.row_begin = p.row_begin;
-  a.row_end = p.row_end;
+  if (int rc = view_args(s, p, L.n_iter, stream, a)) return rc;
   a.strip_stride = 1;
   a.strip_offset = 0;
   a.local_rows = p.row_end - p.row_begin;
   a.row_skew = p.row_begin % kWarpTileH;  // tiles on the full frame's grid, as in the render
   a.split = 1;
-  a.n_iter = L.n_iter;
-  a.n_rays = p.number_of_rays_per_pixel;
-  a.two_over_n = 2 / p.number_of_rays_per_pixel;
-  a.zoom = p.zoom_factor;
-  a.off_x = p.offset_x;
-  a.off_y = p.offset_y;
-  a.frame = p.frame;
-  a.seed = p.seed;
-  a.orzan = p.use_diffusion_curve_save;
-  a.use_aa = p.use_aa;
-  a.max_depth = p.max_trace_depth;
-  a.brute = p.traversal == RDC_TRAVERSAL_BRUTE_FORCE;
-  a.cull = p.traversal == RDC_TRAVERSAL_LBVH;
   aa.tiles_x = (p.image_width + kWarpTileW - 1) / kWarpTileW;
   aa.n_tiles = aa.tiles_x * ((a.local_rows + a.row_skew + kWarpTileH - 1) / kWarpTileH);
   aa.portals = s->info.has_portals;
   const uint32_t warps_per_block = kBlock / 32;
   k_stop_adjoint<FAMILY><<<(aa.n_tiles + warps_per_block - 1) / warps_per_block, kBlock, 0, stream>>>(aa);
   RDC_CUDA(cudaGetLastError());
-  RDC_CUDA(cudaEventRecord(s->launched, stream));
-  s->launched_on = stream;
-  s->launched_any = true;
-  return 0;
+  return record_launch(s, stream);
 }
 
 }  // namespace
